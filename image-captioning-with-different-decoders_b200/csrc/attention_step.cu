@@ -853,7 +853,7 @@ __global__ void __launch_bounds__(256) att_step_bwd_kernel(
 // ------------------------------------------------------------------------------------------------
 constexpr int PROJ_PB = 28;
 
-__global__ void att_proj_bwd_kernel(int B, int T, int P, int A,
+__device__ __forceinline__ void att_proj_bwd_body(int B, int T, int P, int A,
                                     const int* __restrict__ row_len,   // [B] number of active steps of row b
                                     const float* __restrict__ att_enc, const float* __restrict__ att_dec_all,
                                     long long ld_dec, const float* __restrict__ w_full,
@@ -927,6 +927,24 @@ __global__ void att_proj_bwd_kernel(int B, int T, int P, int A,
     if (a < A) { *reinterpret_cast<float4*>(mine + a) = wacc; *reinterpret_cast<float4*>(mine + A + a) = bacc; }
     const float tot = block_sum(de_sum, s_red);
     if (threadIdx.x == 0) { mine[2 * A] = tot; mine[2 * A + 1] = 0.f; mine[2 * A + 2] = 0.f; mine[2 * A + 3] = 0.f; }
+}
+__global__ void att_proj_bwd_kernel(int B, int T, int P, int A,
+                                    const int* __restrict__ row_len,   // [B] number of active steps of row b
+                                    const float* __restrict__ att_enc, const float* __restrict__ att_dec_all,
+                                    long long ld_dec, const float* __restrict__ w_full,
+                                    const float* __restrict__ d_e, float* __restrict__ d_att_enc,
+                                    float* __restrict__ partial) {
+    att_proj_bwd_body(B, T, P, A, row_len, att_enc, att_dec_all, ld_dec, w_full, d_e, d_att_enc, partial);
+}
+// blocks of more than 512 threads (A > 2048): the kernel above uses more than 64 registers, so 1024 threads would not fit the 64K
+// registers of an SM; this instantiation caps them at 64
+__global__ void __launch_bounds__(1024) att_proj_bwd_kernel_wide(int B, int T, int P, int A,
+                                    const int* __restrict__ row_len,   // [B] number of active steps of row b
+                                    const float* __restrict__ att_enc, const float* __restrict__ att_dec_all,
+                                    long long ld_dec, const float* __restrict__ w_full,
+                                    const float* __restrict__ d_e, float* __restrict__ d_att_enc,
+                                    float* __restrict__ partial) {
+    att_proj_bwd_body(B, T, P, A, row_len, att_enc, att_dec_all, ld_dec, w_full, d_e, d_att_enc, partial);
 }
 
 struct BtPack { int v[ICD_MAX_STEPS]; };
@@ -1046,13 +1064,18 @@ extern "C" int icd_attention_proj_bwd(int B, int T, int P, int A, const int32_t*
         static size_t configured = 48 * 1024;
         if (smem > configured) {
             ICD_CUDA(cudaFuncSetAttribute(att_proj_bwd_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+            ICD_CUDA(cudaFuncSetAttribute(att_proj_bwd_kernel_wide, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
             configured = smem;
         }
     }
     int threads = ((A / 4 + 31) / 32) * 32;
     dim3 grid(chunks, B);
-    att_proj_bwd_kernel<<<grid, threads, smem, s>>>(B, T, P, A, row_len, att_enc, att_dec_all, ld_dec, w_full,
-                                                     d_e, d_att_enc, partial);
+    if (threads > 512)
+        att_proj_bwd_kernel_wide<<<grid, threads, smem, s>>>(B, T, P, A, row_len, att_enc, att_dec_all, ld_dec, w_full,
+                                                               d_e, d_att_enc, partial);
+    else
+        att_proj_bwd_kernel<<<grid, threads, smem, s>>>(B, T, P, A, row_len, att_enc, att_dec_all, ld_dec, w_full,
+                                                              d_e, d_att_enc, partial);
     ICD_LAUNCH_CHECK();
     // reduce the per-CTA partials: [0,A) -> d_w_full, [A,2A) -> d enc_att.bias, column 2A -> d_b_full
     ICD_TRY(icd_colsum(partial, W, (int64_t)B * chunks, A, nullptr, d_w_full, s));

@@ -689,7 +689,7 @@ __device__ __forceinline__ float gt_mask(float a, float b) {
     return m;
 }
 
-__global__ void att_proj_bwd_bf16_kernel(int B, int T, int P, int A, const int* __restrict__ row_len,
+__device__ __forceinline__ void att_proj_bwd_bf16_body(int B, int T, int P, int A, const int* __restrict__ row_len,
                                          const __nv_bfloat16* __restrict__ att_enc,
                                          const float* __restrict__ att_dec_all, long long ld_dec,
                                          const float* __restrict__ w_full, const float* __restrict__ d_e,
@@ -810,6 +810,24 @@ __global__ void att_proj_bwd_bf16_kernel(int B, int T, int P, int A, const int* 
     }
     const float tot = block_sum(de_sum, s_red);
     if (threadIdx.x == 0) { mine[2 * A] = tot; mine[2 * A + 1] = 0.f; mine[2 * A + 2] = 0.f; mine[2 * A + 3] = 0.f; }
+}
+__global__ void att_proj_bwd_bf16_kernel(int B, int T, int P, int A, const int* __restrict__ row_len,
+                                         const __nv_bfloat16* __restrict__ att_enc,
+                                         const float* __restrict__ att_dec_all, long long ld_dec,
+                                         const float* __restrict__ w_full, const float* __restrict__ d_e,
+                                         float* __restrict__ d_att_enc, __nv_bfloat16* __restrict__ d_att_enc16,
+                                         float* __restrict__ partial, int split_wfull) {
+    att_proj_bwd_bf16_body(B, T, P, A, row_len, att_enc, att_dec_all, ld_dec, w_full, d_e, d_att_enc, d_att_enc16, partial, split_wfull);
+}
+// blocks of more than 512 threads (two halves of A/4 > 256 threads, up to A = 2048): the kernel above uses more than 64 registers, so
+// 1024 threads would not fit the 64K registers of an SM; this instantiation caps them at 64
+__global__ void __launch_bounds__(1024) att_proj_bwd_bf16_kernel_wide(int B, int T, int P, int A, const int* __restrict__ row_len,
+                                         const __nv_bfloat16* __restrict__ att_enc,
+                                         const float* __restrict__ att_dec_all, long long ld_dec,
+                                         const float* __restrict__ w_full, const float* __restrict__ d_e,
+                                         float* __restrict__ d_att_enc, __nv_bfloat16* __restrict__ d_att_enc16,
+                                         float* __restrict__ partial, int split_wfull) {
+    att_proj_bwd_bf16_body(B, T, P, A, row_len, att_enc, att_dec_all, ld_dec, w_full, d_e, d_att_enc, d_att_enc16, partial, split_wfull);
 }
 
 // ------------------------------------------------------------------------------------------------
@@ -1129,11 +1147,13 @@ extern "C" int icd_attention_proj_bwd_bf16_ex(int B, int T, int P, int A, const 
     static size_t configured = 48 * 1024;
     if (smem > configured) {
         ICD_CUDA(cudaFuncSetAttribute(att_proj_bwd_bf16_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+        ICD_CUDA(cudaFuncSetAttribute(att_proj_bwd_bf16_kernel_wide, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
         configured = smem;
     }
     const int threads = 2 * (((A / 4 + 31) / 32) * 32);              // two halves, see the kernel
     dim3 grid(chunks, B);
-    ICD_CUDA(icd_launch_pdl(ICD_PDL_POINTWISE, att_proj_bwd_bf16_kernel, grid, dim3((unsigned)threads), smem, s, B, T, P, A, (const int*)row_len,
+    ICD_CUDA(icd_launch_pdl(ICD_PDL_POINTWISE, threads > 512 ? att_proj_bwd_bf16_kernel_wide : att_proj_bwd_bf16_kernel, grid,
+                            dim3((unsigned)threads), smem, s, B, T, P, A, (const int*)row_len,
                             reinterpret_cast<const __nv_bfloat16*>(att_enc16), att_dec_all, ld_dec, w_full, d_e, d_att_enc,
                             reinterpret_cast<__nv_bfloat16*>(d_att_enc16), partial, d_att_dec_all ? 1 : 0));
     ICD_LAUNCH_CHECK();

@@ -18,6 +18,7 @@ void icd_set_error(const char* fmt, ...);
 #define ICD_CUDA(call)                                                                 \
     do { cudaError_t e_ = (call); if (e_ != cudaSuccess) {                             \
         icd_set_error("%s:%d %s -> %s", __FILE__, __LINE__, #call, cudaGetErrorString(e_)); \
+        (void)cudaGetLastError();   /* consumed: a refused launch is not reported again by a later call */ \
         return (int)e_; } } while (0)
 
 extern long long g_icd_launches;      // api.cu: kernels launched by this library (bench.py reports it)

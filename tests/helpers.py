@@ -173,13 +173,19 @@ def assert_digest_close(name, t, dg, tol, atol=0.0):
 # the timed configuration (B = 512, V = 9490, full dimensions) can be checked tensor by tensor in about a minute.
 # --------------------------------------------------------------------------------------------
 def oracle_fp64_chunked(sd, enc, caps, lens, keep_mask=None, p=0.0, frozen=(), chunk=64, cuda_preds=None,
-                        cuda_alphas=None, alpha_c=1.0):
+                        cuda_alphas=None, alpha_c=1.0, per_step=False, cuda_d_enc=None):
     """Full-batch loss and parameter gradients of the reference train step (models/attention.py:396-420) from the fp64
     oracle, accumulated over row chunks:  loss = sum_rows CE / n_packed + sum_{b,p} (alpha_c - sum_t alpha)^2 / (B*P).
     Lengths must be equal or sorted descending (then "first batch_size_t rows" == "rows with l > t" in every chunk).
     keep_mask: (T, B, D) uint8 dropout keep-mask (train mode) or None.
     cuda_preds / cuda_alphas: optional CPU fp32 copies of the CUDA outputs (or dicts name -> tensor for several candidates);
-    their squared errors against the oracle are accumulated chunk by chunk.  -> dict(loss, grads{name: fp64}, err{predictions, alphas} norm-wise relative)"""
+    their squared errors against the oracle are accumulated chunk by chunk.  -> dict(loss, grads{name: fp64}, err{predictions, alphas} norm-wise relative)
+    Opt-in outputs (same candidate keying as ``err``):
+      per_step=True -> step_sums{predictions, alphas}: (T, 2) fp64 [sum_b (got - ref)^2, sum_b ref^2] of every step t
+        (all rows of the step; see step_rel_err);
+      cuda_d_enc: candidate gradient(s) w.r.t. encoder_out, (B, ..., C) on any device (pulled to the host one row chunk at
+        a time) -> row_sums: (B, 2) fp64 [|got_b - ref_b|^2, |ref_b|^2] per row (see row_rel_err).  The chunk's features
+        are an fp64 leaf; the full fp64 reference gradient is never held."""
     from oracle import decoders as O
     import torch.nn.functional as F
     B = enc.shape[0]
@@ -187,7 +193,8 @@ def oracle_fp64_chunked(sd, enc, caps, lens, keep_mask=None, p=0.0, frozen=(), c
     assert all(dl[i] >= dl[i + 1] for i in range(B - 1)), "chunked oracle needs equal or descending lengths"
     T = max(dl)
     n_packed = sum(dl)
-    P = enc.reshape(B, -1, enc.shape[-1]).shape[1]
+    C = enc.shape[-1]
+    P = enc.reshape(B, -1, C).shape[1]
     w64 = {k: v.detach().cpu().double().clone().requires_grad_(k not in frozen) for k, v in sd.items()}
     loss_total = 0.0
     outputs = {}                      # candidate name -> (predictions, alphas) CPU tensors to be compared with the oracle
@@ -195,7 +202,15 @@ def oracle_fp64_chunked(sd, enc, caps, lens, keep_mask=None, p=0.0, frozen=(), c
         outputs = {k: (cuda_preds[k], cuda_alphas[k]) for k in cuda_preds}
     elif cuda_preds is not None:
         outputs = {"": (cuda_preds, cuda_alphas)}
+    denc = {}                         # candidate name -> gradient w.r.t. encoder_out
+    if isinstance(cuda_d_enc, dict):
+        denc = dict(cuda_d_enc)
+    elif cuda_d_enc is not None:
+        denc = {"": cuda_d_enc}
     acc = {k: {"predictions": [0.0, 0.0], "alphas": [0.0, 0.0]} for k in outputs}
+    steps = {k: {"predictions": torch.zeros(T, 2, dtype=torch.float64), "alphas": torch.zeros(T, 2, dtype=torch.float64)}
+             for k in outputs} if per_step else None
+    rows = {k: torch.zeros(B, 2, dtype=torch.float64) for k in denc}
     margins, ids = [], []
     for r0 in range(0, B, chunk):
         r1 = min(B, r0 + chunk)
@@ -205,7 +220,8 @@ def oracle_fp64_chunked(sd, enc, caps, lens, keep_mask=None, p=0.0, frozen=(), c
         masks = None
         if keep_mask is not None:
             masks = [keep_mask[t, r0:r0 + sum(1 for l in dl[r0:r1] if l > t)].double() for t in range(max(dl[r0:r1]))]
-        pr, _, dls, al = O.attention_decoder_forward(w64, enc[r0:r1].double(), caps[r0:r1], ls, dropout_p=p,
+        e64 = enc[r0:r1].double().reshape(r1 - r0, P, C).requires_grad_(bool(denc))
+        pr, _, dls, al = O.attention_decoder_forward(w64, e64, caps[r0:r1], ls, dropout_p=p,
                                                      dropout_masks=masks, hoist=True)
         Tc = max(dls)
         active = torch.tensor([[t < d for t in range(Tc)] for d in dls])
@@ -220,6 +236,15 @@ def oracle_fp64_chunked(sd, enc, caps, lens, keep_mask=None, p=0.0, frozen=(), c
                     gsl = got[r0:r1, :Tc].double()
                     acc[cand][name][0] += float(((gsl - ref) ** 2).sum())
                     acc[cand][name][1] += float((ref ** 2).sum())
+                    if per_step:
+                        steps[cand][name][:Tc, 0] += ((gsl - ref) ** 2).sum(dim=(0, 2))
+                        steps[cand][name][:Tc, 1] += (ref ** 2).sum(dim=(0, 2))
+            for cand, got in denc.items():
+                g = got[r0:r1].detach().to("cpu", torch.float64).reshape(r1 - r0, P, C)
+                rows[cand][r0:r1, 0] = ((g - e64.grad) ** 2).sum(dim=(1, 2))
+                rows[cand][r0:r1, 1] = (e64.grad ** 2).sum(dim=(1, 2))
+                del g
+            e64 = None
             top2 = pr.detach().topk(2, dim=2)
             mg = torch.zeros(r1 - r0, T)
             ii = torch.zeros(r1 - r0, T, dtype=torch.int64)
@@ -230,11 +255,50 @@ def oracle_fp64_chunked(sd, enc, caps, lens, keep_mask=None, p=0.0, frozen=(), c
     # rows of all-padding chunks contribute alpha_c^2 each to the regulariser (alphas stay 0)
     done_rows = min(B, ((max(i for i in range(B) if dl[i] > 0) // chunk) + 1) * chunk)
     loss_total += (B - done_rows) * P * alpha_c ** 2 / (B * P)
+    # (their reference gradient w.r.t. the features is 0: the rows never attend and h0 / c0 are never used)
+    for cand, got in denc.items():
+        for r0 in range(done_rows, B, chunk):
+            r1 = min(B, r0 + chunk)
+            rows[cand][r0:r1, 0] = (got[r0:r1].detach().to("cpu", torch.float64).reshape(r1 - r0, -1) ** 2).sum(dim=1)
     err = {c: {k: ((v[0] ** 0.5) / (v[1] ** 0.5) if v[1] > 0 else None) for k, v in a.items()} for c, a in acc.items()}
     if list(err) == [""]:
         err = err[""]
-    return dict(loss=loss_total, grads={k: v.grad for k, v in w64.items() if v.grad is not None}, err=err,
-                margin=torch.cat(margins, 0), ids=torch.cat(ids, 0), decode_lengths=dl)
+    out = dict(loss=loss_total, grads={k: v.grad for k, v in w64.items() if v.grad is not None}, err=err,
+               margin=torch.cat(margins, 0), ids=torch.cat(ids, 0), decode_lengths=dl)
+    if per_step:
+        out["step_sums"] = steps[""] if list(steps) == [""] else steps
+    if denc:
+        out["row_sums"] = rows[""] if list(rows) == [""] else rows
+    return out
+
+
+def step_rel_err(sums):
+    """(T, 2) [squared error, squared reference] per step -> (T,) norm-wise relative error of each step (absolute where
+    the reference is 0)."""
+    return (sums[:, 0].sqrt() / torch.where(sums[:, 1] > 0, sums[:, 1], torch.ones_like(sums[:, 1])).sqrt())
+
+
+row_rel_err = step_rel_err        # (B, 2) per-row sums -> (B,) relative error of each row
+
+
+def aggregate_rel_err(sums):
+    """Norm-wise relative error of the whole tensor from its per-step or per-row sums."""
+    return float(sums[:, 0].sum().sqrt() / sums[:, 1].sum().sqrt())
+
+
+def row_spread_failures(err_rows, bound, k):
+    """Per-row criterion of the regime-B parity test: every row within ``bound`` and none more than ``k`` times the median
+    row.  Rows are independent chains, so a row (or a group of rows) that some launch form computes wrongly stands out
+    against the median even where the norm-wise error of the whole tensor hides it.  -> list of failure messages."""
+    med = float(err_rows.median())
+    bad = []
+    worst = int(err_rows.argmax())
+    if float(err_rows[worst]) > bound:
+        over = (err_rows > bound).nonzero().flatten().tolist()
+        bad.append("rows %s over the bound %.1e (worst row %d: %.2e)" % (over[:16], bound, worst, float(err_rows[worst])))
+    if float(err_rows[worst]) > k * med:
+        bad.append("row %d: %.2e > %g x the median row %.2e" % (worst, float(err_rows[worst]), k, med))
+    return bad
 
 
 def seeded_keep_mask(T, B, D, p, seed):

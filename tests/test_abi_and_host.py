@@ -246,6 +246,47 @@ def test_attention_step_launch_forms_host_logic(monkeypatch):
     assert plan(1, 32) == (2, 32, 64, 0)
 
 
+def test_regime_b_schedule_visits_every_attention_step_launch_form(monkeypatch):
+    """tests/test_gpu_ragged_regime_b.py checks the launch forms of the bf16 attention-step kernels against the oracle by running
+    the regime-B schedule (batch_size_t 512 x 7, 488, ..., 46, 24).  If the plan rules change so that the schedule no longer
+    reaches one of them, that test silently stops covering it: this fails instead."""
+    from icd_b200 import synthetic
+    from icd_b200._lib import lib, check
+    for v in ("ICD_ATT_FWD_SPLIT", "ICD_ATT_BWD_SPLIT", "ICD_ATT_BWD_SPLIT_ROWS", "ICD_ATT_BWD_DEEP"):
+        monkeypatch.delenv(v, raising=False)
+    L = lib()
+    _, lens = synthetic.captions(512, 9490, max_len=25, lengths="ragged")
+    dl = [l - 1 for l in lens]
+    bt = [sum(l > t for l in dl) for t in range(max(dl))]
+    assert bt == [512] * 7 + [488, 467, 434, 410, 388, 362, 338, 298, 274, 244, 216, 186, 160, 126, 88, 46, 24]
+
+    def plan(direction, rows):
+        out = (ctypes.c_int32 * 4)()
+        check(L.icd_attention_step_launch_plan_bf16(direction, rows, 196, 2048, 512, out), "launch_plan")
+        return tuple(out)
+
+    def fwd_form(rows):
+        per, shared, grid, deep = plan(0, rows)
+        return "%d per row%s" % (per, " deep" if deep else "")
+
+    def bwd_form(rows):
+        per, shared, grid, deep = plan(1, rows)
+        if shared == 0:
+            return "whole rows"
+        if shared == rows:
+            return "all halves" + (" deep" if deep else "")
+        return "full balance" if grid % 148 == 0 else "minimal balance"    # full: rows + halves fill every SM equally
+    fwd, bwd = {}, {}
+    for r in bt:
+        fwd.setdefault(fwd_form(r), []).append(r)
+        bwd.setdefault(bwd_form(r), []).append(r)
+    assert fwd == {"1 per row": [512] * 7 + [488, 467, 434, 410, 388, 362, 338, 298, 274, 244], "2 per row": [216, 186, 160],
+                   "2 per row deep": [126, 88], "4 per row deep": [46, 24]}
+    assert set(bwd) == {"full balance", "minimal balance", "all halves", "all halves deep"}
+    assert bwd["minimal balance"] == [467, 338, 298] and 512 in bwd["full balance"] and 488 in bwd["full balance"]
+    assert bwd["all halves"] == [216, 186, 160] and bwd["all halves deep"] == [126, 88, 46, 24]
+
+
 def test_version_counter_guard_of_the_autograd_functions():
     """The decoders' backward reads weights through raw pointers; `_lib.remember_versions` / `check_versions` stand in for
     autograd's saved-tensor check (pure host logic: CPU tensors suffice)."""

@@ -243,13 +243,22 @@ def test_gemm_bf16_transposed_forms_and_beta(cuda):
     H.assert_close_norm(c, ref, 2e-5, "tc gemm TN beta")
 
 
-@pytest.mark.parametrize("R,A,Cdim,use_index", [(3, 48, 2048, False), (6, 512, 2048, True), (2, 64, 512, False)])
-def test_attention_step_bf16_features_matches_oracle_on_rounded_features(cuda, R, A, Cdim, use_index):
+def _bf16_features_case(R, A, Cdim, use_index, P):
+    """P = 196 keeps the test id it had before P was a parameter."""
+    ids = [R, A, Cdim, use_index] + ([] if P == 196 else ["P%d" % P])
+    return pytest.param(R, A, Cdim, use_index, P, id="-".join(str(x) for x in ids))
+
+
+@pytest.mark.parametrize("R,A,Cdim,use_index,P", [_bf16_features_case(*c) for c in [
+    (3, 48, 2048, False, 196), (6, 512, 2048, True, 196), (2, 64, 512, False, 196), (3, 48, 264, False, 196), (2, 64, 520, False, 61),
+    (3, 48, 2048, False, 1), (4, 64, 512, False, 16), (5, 48, 264, False, 31)]])
+def test_attention_step_bf16_features_matches_oracle_on_rounded_features(cuda, R, A, Cdim, use_index, P):
     """bf16-STORED features, fp32 arithmetic: feeding the oracle the same bf16-rounded features must agree to fp32
-    accuracy (1e-5) — the only approximation of this variant is the storage rounding of enc / att_enc."""
+    accuracy (1e-5) — the only approximation of this variant is the storage rounding of enc / att_enc.
+    C = 264 / 520 (C % 256 != 0): the backward's scalar d_alpha path instead of the tensor-core one; P = 1 / 16 / 31 (< 32): the
+    launcher never shares a row between two CTAs, not even under ICD_ATT_BWD_SPLIT=2."""
     ops = _ops()
     g = torch.Generator().manual_seed(R * 13 + A)
-    P = 196
     n_img = 3 if use_index else R
     enc16 = torch.randn(n_img, P, Cdim, generator=g).clamp_min_(0).bfloat16()
     att_enc16 = (torch.randn(n_img, P, A, generator=g) * 0.5).bfloat16()
@@ -281,9 +290,11 @@ def test_attention_step_bf16_features_matches_oracle_on_rounded_features(cuda, R
     d_att_dec, d_fb, d_e, dz16 = ops.attention_step_bwd_bf16(enc16.to(cuda), att_enc16.to(cuda), att_dec.to(cuda),
                                                             wf.to(cuda), alpha, gate, awe, d_gated.to(cuda),
                                                             d_alpha.to(cuda))
-    H.assert_close_norm(d_att_dec, ad64.grad, 2e-5, "d_att_dec")
+    # (P = 1: alpha is 1 and d_att_dec is 0 exactly; its rounding residue is held to an absolute 1e-6)
+    tiny = 1e-6 if P == 1 else 0.0
+    H.assert_close_norm(d_att_dec, ad64.grad, 2e-5, "d_att_dec", atol=tiny)
     H.assert_close_norm(d_fb, fb64.grad, 2e-5, "d_fbeta_pre")
-    H.assert_close_norm(dz16[:, :A].float(), ad64.grad, 4e-3, "dz16[:, :A]")
+    H.assert_close_norm(dz16[:, :A].float(), ad64.grad, 4e-3, "dz16[:, :A]", atol=tiny)
     H.assert_close_norm(dz16[:, A:].float(), fb64.grad, 4e-3, "dz16[:, A:]")
     # row-balance mode of the backward kernel: rows run as two half-row CTAs (2-CTA cluster, halves meet through distributed
     # shared memory); forced here for every row, the balance rule itself splits only the tail of a launch
@@ -294,20 +305,20 @@ def test_attention_step_bf16_features_matches_oracle_on_rounded_features(cuda, R
     finally:
         del os.environ["ICD_ATT_BWD_SPLIT"]
     assert torch.equal(s_fb, d_fb) and torch.equal(s_dz16[:, A:], dz16[:, A:])
-    H.assert_close_norm(s_att_dec, ad64.grad, 2e-5, "d_att_dec (split rows)")
+    H.assert_close_norm(s_att_dec, ad64.grad, 2e-5, "d_att_dec (split rows)", atol=tiny)
     H.assert_close_norm(s_e, d_e, 1e-5, "d_e (split rows)")
-    H.assert_close_norm(s_dz16[:, :A].float(), ad64.grad, 4e-3, "dz16[:, :A] (split rows)")
+    H.assert_close_norm(s_dz16[:, :A].float(), ad64.grad, 4e-3, "dz16[:, :A] (split rows)", atol=tiny)
     d_att_enc, d_att_enc16, d_wf, d_bf, d_be = ops.attention_proj_bwd_bf16(att_enc16.to(cuda), att_dec.to(cuda).view(1, R, A),
                                                         wf.to(cuda), d_e.view(R, 1, P), [R])
-    H.assert_close_norm(d_att_enc, ae64.grad, 2e-5, "d_att_enc")
-    H.assert_close_norm(d_att_enc16.float(), ae64.grad, 4e-3, "d_att_enc16")
-    H.assert_close_norm(d_be, ae64.grad.sum(dim=(0, 1)), 2e-5, "d_b_enc")
-    H.assert_close_norm(d_wf, wf64.grad, 2e-5, "d_w_full")
+    H.assert_close_norm(d_att_enc, ae64.grad, 2e-5, "d_att_enc", atol=tiny)
+    H.assert_close_norm(d_att_enc16.float(), ae64.grad, 4e-3, "d_att_enc16", atol=tiny)
+    H.assert_close_norm(d_be, ae64.grad.sum(dim=(0, 1)), 2e-5, "d_b_enc", atol=tiny)
+    H.assert_close_norm(d_wf, wf64.grad, 2e-5, "d_w_full", atol=tiny)
     # split form of d_w_full (masked sums in the kernel + (sum att_dec * d_att_dec) / w afterwards): same results
     s_att_enc, s_att_enc16, s_wf, s_bf, s_be = ops.attention_proj_bwd_bf16(att_enc16.to(cuda), att_dec.to(cuda).view(1, R, A),
                                                         wf.to(cuda), d_e.view(R, 1, P), [R], d_att_dec_all=d_att_dec.view(1, R, A))
     assert torch.equal(s_att_enc, d_att_enc) and torch.equal(s_att_enc16, d_att_enc16) and torch.equal(s_be, d_be)
-    H.assert_close_norm(s_wf, wf64.grad, 2e-5, "d_w_full (split form)")
+    H.assert_close_norm(s_wf, wf64.grad, 2e-5, "d_w_full (split form)", atol=tiny)
     # ... and a w_full with a zero entry falls back to the direct form inside the kernel
     wf0 = wf.clone(); wf0[3] = 0.0
     z_ref = ops.attention_proj_bwd_bf16(att_enc16.to(cuda), att_dec.to(cuda).view(1, R, A), wf0.to(cuda), d_e.view(R, 1, P), [R])
@@ -601,3 +612,159 @@ def test_persistent_lstm_recurrence_matches_torch(cuda, B, L, H):
     # run-to-run determinism (fixed summation order inside one tcgen05 accumulator)
     out2 = ops.lstm_seq_fwd(w_hh.to(cuda), xg.to(cuda))
     assert torch.equal(out["hout"], out2["hout"]) and torch.equal(out["c_all"], out2["c_all"])
+
+
+def _ragged_bt(B, T, g, n_empty):
+    """Descending decode lengths with dl[0] = T and the last n_empty rows at 0 (Tb = 0) -> (dl, bt)."""
+    dl = sorted((int(x) for x in torch.randint(1, T + 1, (B - n_empty,), generator=g)), reverse=True) + [0] * n_empty
+    dl[0] = T
+    return dl, [sum(1 for l in dl if l > t) for t in range(T)]
+
+
+PROJ_CASES = {        # B, T, P, A, att_dec row stride, w_full kind, rows with no active step
+    "regime_b_like": dict(B=64, T=24, P=196, A=512, ld=512 + 2048 + 2048, w="normal", empty=3),
+    "p1": dict(B=7, T=5, P=1, A=64, ld=72, w="normal", empty=2),
+    "p28": dict(B=6, T=9, P=28, A=128, ld=128, w="normal", empty=1),
+    "p29": dict(B=6, T=9, P=29, A=96, ld=100, w="tiny", empty=1),
+    "p57": dict(B=5, T=6, P=57, A=64, ld=68, w="fallback", empty=1),
+    "t1_a2048": dict(B=3, T=1, P=29, A=2048, ld=2056, w="normal", empty=0),
+    "t104_a512": dict(B=3, T=104, P=29, A=512, ld=512, w="normal", empty=1),
+    "t3_a4096_fp32": dict(B=4, T=3, P=30, A=4096, ld=4096, w="normal", empty=1),     # (the bf16 kernels stop at A = 2048)
+}
+
+
+@pytest.mark.parametrize("case", list(PROJ_CASES))
+def test_attention_proj_bwd_multi_step_ragged_matches_fp64(cuda, case):
+    """The reductions after the time loop over many steps of a ragged batch (one step is covered above):
+        d_att_enc, d_w_full, d_b_full, d_b_enc  of  sum_{b, t < Tb, p} d_e[b,t,p] (sum_a relu(att_enc[b,p,a] + att_dec[t,b,a]) w[a] + b_full)
+    for icd_attention_proj_bwd (fp32), icd_attention_proj_bwd_bf16 (direct form) and its split form (d_att_dec_all given).
+    Edges: pixel tails (P = 1, 29, 57: P % 28 != 0, the clamped loads and the early break), rows with no active step (their
+    d_att_enc rows are exactly 0), att_dec_all with a row stride > A (a slice of the decoders' z), exact ties
+    att_enc + att_dec == 0 (split form x > -att_dec == direct form x + att_dec > 0), w_full entries from 1e-17 to 1 and one
+    below the split form's floor (fallback to the direct form), T = 1 at A = 2048 (1024-thread blocks, two staged rows; these
+    failed to launch before the kernels got an instantiation capped at 64 registers), A = 4096 in the fp32 kernel (1024 threads),
+    T = 104 at A = 512 (the shared-memory limit; 105 is an argument error).  d_e at inactive (t, b) — and att_dec_all there,
+    for the kernels that do not read it in the split form's column dot — is NaN: it must never be read."""
+    from icd_b200 import _lib
+    ops = _ops()
+    c = PROJ_CASES[case]
+    B, T, P, A, ld = c["B"], c["T"], c["P"], c["A"], c["ld"]
+    g = torch.Generator().manual_seed(B * 1000 + T * 10 + P)
+    if case == "regime_b_like":              # bench.py's regime-B lengths, one row in eight, and three rows with no step
+        from icd_b200 import synthetic
+        _, lens = synthetic.captions(8 * (B - 3), 9490, max_len=25, lengths="ragged")
+        dl = [l - 1 for l in lens[::8]] + [0] * 3
+        bt = [sum(1 for l in dl if l > t) for t in range(T)]
+        assert bt[0] == B - 3 and bt[-1] < bt[12] < bt[0]
+    else:
+        dl, bt = _ragged_bt(B, T, g, c["empty"])
+    active = torch.tensor([[t < dl[b] for t in range(T)] for b in range(B)])           # (B, T)
+    att_enc = (torch.randn(B, P, A, generator=g) * 0.5).bfloat16().float()              # exact in both kernels
+    dec_buf = torch.randn(T, B, ld, generator=g) * 0.5
+    for t in range(T):                       # exact ties: att_dec[t, b, :A/4] = -att_enc[b, p0, :A/4]
+        p0 = int(torch.randint(0, P, (1,), generator=g))
+        dec_buf[t, :, :A // 4] = -att_enc[:, p0, :A // 4]
+    if c["w"] == "normal":
+        w = torch.randn(A, generator=g) * 0.2
+    else:                                    # magnitudes 1e-17 .. 1, both signs
+        w = 10.0 ** (-17 * torch.rand(A, generator=g)) * torch.sign(torch.randn(A, generator=g))
+        if c["w"] == "fallback":
+            w[A // 3] = 1e-19
+    d_e = torch.randn(B, T, P, generator=g)
+    # fp64 reference (autograd), one step at a time
+    ae64 = att_enc.double().requires_grad_(True)
+    w64 = w.double().requires_grad_(True)
+    b64 = torch.zeros(1, dtype=torch.float64, requires_grad=True)
+    for t in range(T):
+        n = bt[t]
+        if n == 0:
+            continue
+        s = torch.relu(ae64[:n] + dec_buf[t, :n, None, :A].double()) @ w64 + b64          # (n, P)
+        (s * d_e[:n, t].double()).sum().backward()
+    # split-form input: d_att_dec_all[t, b] = w * sum_p [att_enc + att_dec > 0] d_e, 0 at inactive (t, b)
+    ddec_buf = torch.zeros(T, B, ld)
+    with torch.no_grad():
+        for t in range(T):
+            n = bt[t]
+            m = ((ae64[:n] + dec_buf[t, :n, None, :A].double()) > 0).double()               # (n, P, A)
+            ddec_buf[t, :n, :A] = (w64 * (m * d_e[:n, t, :, None].double()).sum(1)).float()
+    # never-read entries
+    d_e_nan = d_e.clone()
+    d_e_nan[~active] = float("nan")
+    dec_nan = dec_buf.clone()
+    dec_nan[~active.t()] = float("nan")
+    dev = lambda x: x.to(cuda)
+    dec_nan_d, dec_d, ddec_d = dev(dec_nan)[:, :, :A], dev(dec_buf)[:, :, :A], dev(ddec_buf)[:, :, :A]
+    assert dec_nan_d.stride(1) == ld
+    want = dict(d_att_enc=ae64.grad, d_w_full=w64.grad, d_b_full=b64.grad, d_b_enc=ae64.grad.sum(dim=(0, 1)))
+    empty_rows = [b for b in range(B) if dl[b] == 0]
+
+    def check(res, what):
+        d_att_enc, d_wf, d_bf, d_be = res[0], res[-3], res[-2], res[-1]
+        H.assert_close_norm(d_att_enc, want["d_att_enc"], 2e-5, what + " d_att_enc")
+        H.assert_close_norm(d_wf, want["d_w_full"], 2e-5, what + " d_w_full")
+        H.assert_close_norm(d_bf, want["d_b_full"], 1e-4, what + " d_b_full", atol=1e-5)
+        H.assert_close_norm(d_be, want["d_b_enc"], 2e-5, what + " d_b_enc")
+        if len(res) == 5:
+            H.assert_close_norm(res[1].float(), want["d_att_enc"], 4e-3, what + " d_att_enc16")
+            assert torch.all(res[1][empty_rows] == 0)
+        assert torch.all(d_att_enc[empty_rows] == 0), what + ": rows with no active step"
+        assert all(torch.isfinite(x).all() for x in res), what + ": non-finite output (a never-read entry was read)"
+
+    att_enc_d, att_enc16_d, w_d, d_e_d = dev(att_enc), dev(att_enc.bfloat16()), dev(w), dev(d_e_nan)
+    check(ops.attention_proj_bwd(att_enc_d, dec_nan_d, w_d, d_e_d, bt), "fp32")
+    if case.endswith("_fp32"):
+        return
+    direct = ops.attention_proj_bwd_bf16(att_enc16_d, dec_nan_d, w_d, d_e_d, bt)
+    check(direct, "bf16 direct")
+    split = ops.attention_proj_bwd_bf16(att_enc16_d, dec_d, w_d, d_e_d, bt, d_att_dec_all=ddec_d)
+    check(split, "bf16 split")
+    # the split form's masked sums equal the direct form's bit for bit (exact ties included)
+    assert torch.equal(split[0], direct[0]) and torch.equal(split[1], direct[1]) and torch.equal(split[4], direct[4])
+    if c["w"] == "fallback":                 # a |w_full| entry below the floor: the direct form, bit for bit
+        assert torch.equal(split[2], direct[2])
+    if case == "t104_a512":                  # one more step no longer fits the shared memory: an argument error, no launch
+        bt1 = bt + [0]
+        dec1 = torch.zeros(T + 1, B, A, device=cuda)
+        de1 = torch.zeros(B, T + 1, P, device=cuda)
+        with pytest.raises(_lib.IcdError):
+            ops.attention_proj_bwd(att_enc_d, dec1, w_d, de1, bt1)
+        with pytest.raises(_lib.IcdError):
+            ops.attention_proj_bwd_bf16(att_enc16_d, dec1, w_d, de1, bt1)
+
+
+@pytest.mark.parametrize("C,P", [(4, 1), (1028, 50), (2048, 196)])
+@pytest.mark.parametrize("T", [1, 31, 32, 33, 65])
+@pytest.mark.parametrize("with_mean", [True, False])
+def test_attention_enc_grad_multi_step_matches_fp64(cuda, T, C, P, with_mean):
+    """icd_attention_enc_grad on its own: d_enc[b,p,c] = sum_{t < Tb} alpha[b,t,p] d_awe[t,b,c] + d_mean[b,c] / P.  The kernel keeps
+    d_awe of at most 32 steps in registers and accumulates d_enc in place over the chunks of 32 steps (T = 33, 65); rows with
+    Tb = 0 get d_mean / P only (0 without d_mean); C = 4 / 1028: one thread / a partly filled second block of channels.
+    alphas and d_awe at inactive (t, b) are NaN: they must never be read."""
+    ops = _ops()
+    g = torch.Generator().manual_seed(T * 100 + C + P)
+    B = 6
+    dl, bt = _ragged_bt(B, T, g, 2 if T > 1 else 1)
+    alphas = torch.rand(B, T, P, generator=g) / P
+    d_awe = torch.randn(T, B, C, generator=g)
+    d_mean = torch.randn(B, C, generator=g) if with_mean else None
+    ref = torch.zeros(B, P, C, dtype=torch.float64)
+    for b in range(B):
+        n = dl[b]
+        ref[b] = torch.einsum("tp,tc->pc", alphas[b, :n].double(), d_awe[:n, b].double())
+        if with_mean:
+            ref[b] += d_mean[b].double() / P
+    for b in range(B):
+        alphas[b, dl[b]:] = float("nan")
+        d_awe[dl[b]:, b] = float("nan")
+    got = ops.attention_enc_grad(alphas.to(cuda), d_awe.to(cuda), d_mean.to(cuda) if with_mean else None, bt)
+    assert torch.isfinite(got).all()
+    H.assert_close_norm(got, ref, 1e-5, "d_enc")
+    for b in range(B):
+        if dl[b] == 0:
+            if with_mean:
+                H.assert_close_norm(got[b], ref[b], 1e-6, "d_enc of a row with no active step")
+            else:
+                assert torch.all(got[b] == 0)
+        else:
+            H.assert_close_norm(got[b], ref[b], 1e-5, "d_enc row %d (%d steps)" % (b, dl[b]))
