@@ -69,6 +69,7 @@ GemmDesc = _make_struct("icd_gemm_desc_t")
 AttDesc = _make_struct("icd_att_desc_t")
 BaseDesc = _make_struct("icd_base_desc_t")
 BeamDesc = _make_struct("icd_beam_desc_t")
+BaseBeamDesc = _make_struct("icd_base_beam_desc_t")
 
 PREC_FP32 = DEFINES["ICD_PREC_FP32"]
 PREC_BF16 = DEFINES["ICD_PREC_BF16"]
@@ -94,6 +95,7 @@ def lib():
     L = ctypes.CDLL(LIB_PATH)
     L.icd_last_error_string.restype = ctypes.c_char_p
     L.icd_beam_search_ws_bytes.restype = ctypes.c_int64
+    L.icd_baseline_beam_search_ws_bytes.restype = ctypes.c_int64
     L.icd_attention_proj_bwd_ws_floats.restype = ctypes.c_int64
     L.icd_launch_count.restype = ctypes.c_int64
     L.icd_gemm_ws_bytes.restype = ctypes.c_int64
@@ -104,7 +106,7 @@ def lib():
         raise IcdError("libicd_b200.so ABI %d != header ABI %d — rebuild" %
                        (L.icd_version(), DEFINES["ICD_B200_ABI_VERSION"]))
     for fn, st in (("icd_sizeof_att_desc", AttDesc), ("icd_sizeof_base_desc", BaseDesc),
-                   ("icd_sizeof_beam_desc", BeamDesc)):
+                   ("icd_sizeof_beam_desc", BeamDesc), ("icd_sizeof_base_beam_desc", BaseBeamDesc)):
         if getattr(L, fn)() != ctypes.sizeof(st):
             raise IcdError("%s: C says %d bytes, ctypes says %d" % (fn, getattr(L, fn)(), ctypes.sizeof(st)))
     _lib = L

@@ -112,4 +112,5 @@ const char* icd_last_error_string(void) { return g_err; }
 int icd_sizeof_att_desc(void) { return (int)sizeof(icd_att_desc_t); }
 int icd_sizeof_base_desc(void) { return (int)sizeof(icd_base_desc_t); }
 int icd_sizeof_beam_desc(void) { return (int)sizeof(icd_beam_desc_t); }
+int icd_sizeof_base_beam_desc(void) { return (int)sizeof(icd_base_beam_desc_t); }
 }

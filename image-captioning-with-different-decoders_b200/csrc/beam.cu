@@ -17,6 +17,10 @@
 // k_live (= remaining beams) of the flattened (k_live * V) scores, sorted descending (:82); scores are raw
 // summed log-probs (:74-76); beams that emit <end> leave the beam and are never replaced (:93-104); the winner is
 // the first completed beam with the maximal score (:127); the loop body runs for step = 1..max_steps+1 (:119).
+//
+// icd_baseline_beam_search runs the same state machine (the same top-k, compaction, reorder and finalize kernels) over the
+// BaselineDecoder's step: the image feature as LSTM step 0 from the zero state, then per step h W_hh^T on the live rows, one fused
+// kernel for the embg gather + LSTMCell (+ the split of h for the fp32-grade vocabulary contraction), and the vocabulary layer.
 #include "common.cuh"
 #include "gemm_tc.cuh"
 #include <cuda_bf16.h>
@@ -40,6 +44,9 @@ struct BeamWs {
     // ICD_PREC_FP32X3: 3-term bf16 splits (gemm_tc.cu) of the weights (once per call) and of the step activations
     void *x3_We, *x3_Wcat, *x3_WihE, *x3_WihC, *x3_Wh, *x3_Wc, *x3_Wfc, *x3_act;
     float* x3_splitk; long long x3_splitk_floats;
+    // baseline decoder only (carve_base): fp32 copy of an fp64 embedding table, split of W_hh
+    float* emb32;
+    void* x3_Whh;
 };
 
 inline long long up8ll(long long x) { return (x + 7) / 8 * 8; }
@@ -557,17 +564,140 @@ __global__ void __launch_bounds__(256) split3_mean_kernel(int P, int C, const fl
     }
 }
 
+// ---------------------------------------------------------------------------------------------- BaselineDecoder beam search
+// Workspace of icd_baseline_beam_search: the fields of BeamWs the baseline step uses (state rows of H, z = h W_hh^T of 4H, logits, the
+// whole-vocabulary embg, the bookkeeping of the shared top-k / compaction / reorder / finalize kernels) and the fp32x3 splits of
+// W_ih (x3_WihE), W_hh (x3_Whh) and the vocabulary layer (x3_Wfc).
+constexpr int BASE_EMBG_ROWS = 4096;      // vocabulary rows per embg pass (bounds the split activation scratch)
+
+size_t carve_base(const icd_base_beam_desc_t* d, BeamWs* w, char* base) {
+    const size_t R = (size_t)d->n_img * d->k, S = (size_t)d->max_steps + 1;
+    const int E = d->E, H = d->H, V = d->V, G = 4 * H;
+    size_t off = 0;
+    auto take = [&](size_t bytes) { size_t o = off; off += (bytes + 255) & ~(size_t)255; return base ? base + o : (char*)nullptr; };
+    float* f;
+#define TAKE_F(name, n) f = (float*)take(sizeof(float) * (n)); if (w) w->name = f;
+    TAKE_F(h0, (size_t)d->n_img * H) TAKE_F(c0, (size_t)d->n_img * H)
+    TAKE_F(h, R * H) TAKE_F(c, R * H) TAKE_F(h_tmp, R * H) TAKE_F(c_tmp, R * H)
+    TAKE_F(z, R * G)                                          // also the gates of the image step (n_img rows)
+    TAKE_F(logits, R * V)
+    TAKE_F(embg, (size_t)V * G)                               // embedding row x W_ih^T + b_ih + b_hh for EVERY token, once per call
+    TAKE_F(emb32, d->emb_is_f64 ? (size_t)V * E : 0)
+    TAKE_F(score, R) TAKE_F(score_tmp, R) TAKE_F(best_score, (size_t)d->n_img)
+#undef TAKE_F
+    int* ip;
+#define TAKE_I(name, n) ip = (int*)take(sizeof(int) * (n)); if (w) w->name = ip;
+    TAKE_I(img_index, R) TAKE_I(prev_word, R) TAKE_I(k_live, (size_t)d->n_img) TAKE_I(src, R)
+    TAKE_I(parent, S * R) TAKE_I(word, S * R) TAKE_I(best_step, (size_t)d->n_img) TAKE_I(best_parent, (size_t)d->n_img)
+    TAKE_I(slot_img, (size_t)d->n_img) TAKE_I(slot_img_tmp, (size_t)d->n_img) TAKE_I(k_live_tmp, (size_t)d->n_img)
+    TAKE_I(new_slot, (size_t)d->n_img) TAKE_I(n_live, 4) TAKE_I(word_tmp, R)
+    ip = (int*)take(sizeof(int) * (size_t)d->n_img); if (w) w->row_off[0] = ip;
+    ip = (int*)take(sizeof(int) * (size_t)d->n_img); if (w) w->row_off[1] = ip;
+#undef TAKE_I
+    long long* lp = (long long*)take(sizeof(long long) * R); if (w) w->tok64 = lp;
+    if (d->precision == ICD_PREC_FP32X3) {
+        void* v;
+#define TAKE_X3(name, rows, K) v = (void*)take((size_t)(rows) * 6 * up8ll(K) * 2); if (w) w->name = v;
+        TAKE_X3(x3_WihE, G, E) TAKE_X3(x3_Whh, G, H) TAKE_X3(x3_Wfc, V, H)
+#undef TAKE_X3
+        const size_t ve = (size_t)(V < BASE_EMBG_ROWS ? V : BASE_EMBG_ROWS);
+        size_t act_rows = R > ve ? R : ve;
+        const long long kmax = E > H ? E : H;
+        v = (void*)take(act_rows * 6 * up8ll(kmax) * 2); if (w) w->x3_act = v;
+        long long nf = 0;
+        const long long shapes[][3] = {{(long long)ve, G, 6 * up8ll(E)}, {(long long)d->n_img, G, 6 * up8ll(E)},
+                                       {(long long)R, G, 6 * up8ll(H)}, {(long long)R, V, 6 * up8ll(H)}};
+        for (const auto& sh : shapes) { const long long n = icd_gemm_bf16_splitk_floats((int)sh[0], (int)sh[1], (int)sh[2]); if (n > nf) nf = n; }
+        float* fp = (float*)take(sizeof(float) * (size_t)nf);
+        if (w) { w->x3_splitk = fp; w->x3_splitk_floats = nf; }
+    }
+    return off;
+}
+
+// The baseline decoder's step after the W_hh contraction, one CTA per live row r:
+//   gates = embg[tok[r]] + z[r]   (embg = emb W_ih^T + b_ih + b_hh for the whole vocabulary, z = h W_hh^T of this step)
+// then the LSTMCell with the activation code of lstm_pointwise_fwd_kernel (pointwise.cu) -> h_new, c_new.  In the fp32-grade tier
+// it also writes the 3-term bf16 split of h_new (rounding of icd_split3_bf16) into x3 — rows of nseg * up8(H): 3 stored planes
+// [t1 | t2 | t3] or the 6-segment A pattern [a1 | a1 | a2 | a1 | a3 | a2] (gemm_tc.cu), pad columns zero — which the vocabulary
+// contraction then consumes with pre_split.  embg == NULL: gates = z[r] (the image step); c_prev == NULL: the zero state.
+__global__ void __launch_bounds__(128) baseline_beam_cell_kernel(int H, const float* __restrict__ embg,
+                                                                  const long long* __restrict__ tok, const float* __restrict__ z,
+                                                                  const float* __restrict__ c_prev, float* __restrict__ c_new,
+                                                                  float* __restrict__ h_new, unsigned short* __restrict__ x3,
+                                                                  int nseg, const int* __restrict__ n_live) {
+    const long long r = blockIdx.x;
+    if (n_live && r >= n_live[1]) return;
+    const int G = 4 * H, seg = (H + 7) / 8 * 8;
+    const float* e = embg ? embg + tok[r] * G : nullptr;
+    const float* zr = z + r * G;
+    for (int col = 4 * threadIdx.x; col < seg; col += 4 * blockDim.x) {
+        float hv[4] = {0.f, 0.f, 0.f, 0.f};
+        if (col < H) {                                        // H % 4 == 0: a group of four is all data or all padding
+            float4 g[4];
+#pragma unroll
+            for (int q = 0; q < 4; ++q) {
+                g[q] = *reinterpret_cast<const float4*>(zr + q * H + col);
+                if (e) {
+                    const float4 a = *reinterpret_cast<const float4*>(e + q * H + col);
+                    g[q] = make_float4(a.x + g[q].x, a.y + g[q].y, a.z + g[q].z, a.w + g[q].w);
+                }
+            }
+            const float4 cp = c_prev ? *reinterpret_cast<const float4*>(c_prev + r * H + col) : make_float4(0.f, 0.f, 0.f, 0.f);
+            const float gi[4] = {g[0].x, g[0].y, g[0].z, g[0].w}, gf[4] = {g[1].x, g[1].y, g[1].z, g[1].w};
+            const float gg[4] = {g[2].x, g[2].y, g[2].z, g[2].w}, go[4] = {g[3].x, g[3].y, g[3].z, g[3].w};
+            const float cpv[4] = {cp.x, cp.y, cp.z, cp.w};
+            float cv[4];
+#pragma unroll
+            for (int u = 0; u < 4; ++u) {
+                const float i = sigmoidf_(gi[u]);
+                const float f = sigmoidf_(gf[u]);
+                const float gt = tanhf(gg[u]);
+                const float o = sigmoidf_(go[u]);
+                cv[u] = f * cpv[u] + i * gt;
+                hv[u] = o * tanhf(cv[u]);
+            }
+            *reinterpret_cast<float4*>(c_new + r * H + col) = make_float4(cv[0], cv[1], cv[2], cv[3]);
+            *reinterpret_cast<float4*>(h_new + r * H + col) = make_float4(hv[0], hv[1], hv[2], hv[3]);
+        }
+        if (x3) {
+            unsigned short t[3][4];
+#pragma unroll
+            for (int u = 0; u < 4; ++u) {
+                const __nv_bfloat16 b1 = __float2bfloat16_rn(hv[u]);
+                const float r1 = hv[u] - __bfloat162float(b1);
+                const __nv_bfloat16 b2 = __float2bfloat16_rn(r1);
+                const __nv_bfloat16 b3 = __float2bfloat16_rn(r1 - __bfloat162float(b2));
+                t[0][u] = __bfloat16_as_ushort(b1); t[1][u] = __bfloat16_as_ushort(b2); t[2][u] = __bfloat16_as_ushort(b3);
+            }
+            const int pat[6] = {0, 0, 1, 0, 2, 1};
+            unsigned short* dst = x3 + r * nseg * seg + col;
+#pragma unroll
+            for (int sg = 0; sg < 6; ++sg) {
+                if (sg >= nseg) break;
+                const unsigned short* tt = t[nseg == 3 ? sg : pat[sg]];
+                *reinterpret_cast<uint2*>(dst + (long long)sg * seg) =
+                    make_uint2((unsigned)tt[0] | ((unsigned)tt[1] << 16), (unsigned)tt[2] | ((unsigned)tt[3] << 16));
+            }
+        }
+    }
+}
+
+__global__ void f64_to_f32_kernel(const double* __restrict__ src, long long n, float* __restrict__ dst) {
+    for (long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += (long long)gridDim.x * blockDim.x)
+        dst[i] = (float)src[i];
+}
+
 }  // namespace
 
 // y[rows, N] = x[rows, K] * W[N, K]^T (+ bias + add + beta*y): fp32 FMA kernel, or the fp32-grade tensor-core tier with the
 // activation split on the fly and the weight split `w16x3` prepared once per call.
 int beam_mm(int prec, const BeamWs& w, const float* x, long long ldx, int rows, int K, const float* W, long long ldw,
             const void* w16x3, float* y, long long ldy, int N, const float* bias, const float* add, long long ldadd,
-            float beta, cudaStream_t s, const int* m_live = nullptr, bool pre_split = false) {
+            float beta, cudaStream_t s, const int* m_live = nullptr, bool pre_split = false, const float* bias2 = nullptr) {
     // m_live: device-side count of live rows (compacted to the front).  The tensor-core tier computes only those; the fp32
     // FMA tier computes all `rows` (rows beyond the live count hold stale, finite state and are never read back).
     if (prec != ICD_PREC_FP32X3)
-        return icd_gemm_simple(ICD_PREC_FP32, x, ldx, 1, W, ldw, 1, y, ldy, rows, N, K, bias, nullptr, add, ldadd, nullptr, 0,
+        return icd_gemm_simple(ICD_PREC_FP32, x, ldx, 1, W, ldw, 1, y, ldy, rows, N, K, bias, bias2, add, ldadd, nullptr, 0,
                                nullptr, beta, s);
     // three stored planes per operand where a segment is a whole number of k-blocks (gemm_tc.cuh), else the six-segment layout;
     // the weight splits of the call (w16x3) and the fused producers of w.x3_act follow the same rule
@@ -576,7 +706,7 @@ int beam_mm(int prec, const BeamWs& w, const float* x, long long ldx, int rows, 
     const long long ld3 = (p3 ? 3 : 6) * seg;
     if (!pre_split) ICD_TRY(icd_split3_bf16(x, ldx, rows, K, w.x3_act, p3 ? 2 : 0, s, m_live));   // (pre_split: the producer wrote w.x3_act)
     if (p3) icd_gemm_x3_planes((int)(seg / 64), (int)(seg / 64));
-    const int rc = icd_gemm_bf16_ex(w.x3_act, ld3, 0, w16x3, ld3, 0, y, ldy, rows, N, (int)(6 * seg), bias, nullptr, add, ldadd,
+    const int rc = icd_gemm_bf16_ex(w.x3_act, ld3, 0, w16x3, ld3, 0, y, ldy, rows, N, (int)(6 * seg), bias, bias2, add, ldadd,
                                     nullptr, 0, nullptr, beta, s, nullptr, 0, w.x3_splitk, w.x3_splitk_floats, nullptr, m_live);
     icd_gemm_x3_planes(0, 0);
     return rc;
@@ -720,6 +850,120 @@ extern "C" int icd_beam_search(const icd_beam_desc_t* d, void* stream) {
     beam_finalize_kernel<<<n_img, 128, 0, s>>>(k, P, S1, R, d->start_id, d->end_id, w.best_score, w.best_step,
                                                w.best_parent, w.parent, w.word, w.alpha_steps, d->out_len, d->out_seq,
                                                d->out_score, d->out_alpha);
+    ICD_LAUNCH_CHECK();
+    return 0;
+}
+
+static int base_beam_shape_check(const icd_base_beam_desc_t* d) {
+    ICD_CHECK_ARG(d != nullptr, "baseline_beam_search: null descriptor");
+    ICD_CHECK_ARG(d->n_img > 0 && d->k >= 1 && d->k <= KMAX, "baseline_beam_search: n_img=%d k=%d (k in 1..%d)", d->n_img, d->k, KMAX);
+    ICD_CHECK_ARG(d->max_steps >= 1 && d->max_steps + 1 <= ICD_MAX_STEPS, "baseline_beam_search: max_steps=%d out of range", d->max_steps);
+    ICD_CHECK_ARG(d->V >= d->k, "baseline_beam_search: vocabulary (%d) smaller than the beam (%d)", d->V, d->k);
+    ICD_CHECK_ARG(d->E > 0 && d->H > 0 && d->E % 4 == 0 && d->H % 4 == 0, "baseline_beam_search: E=%d H=%d must be positive multiples of 4",
+                  d->E, d->H);
+    ICD_CHECK_ARG((long long)d->n_img * d->k <= 65535, "baseline_beam_search: n_img*k=%lld exceeds 65535 rows per call (chunk the images)",
+                  (long long)d->n_img * d->k);
+    ICD_CHECK_ARG(d->precision == ICD_PREC_FP32 || d->precision == ICD_PREC_FP32X3,
+                  "baseline_beam_search: precision must be ICD_PREC_FP32 or ICD_PREC_FP32X3 (identical captions need fp32-grade logits)");
+    return 0;
+}
+
+static int base_beam_check(const icd_base_beam_desc_t* d) {
+    ICD_TRY(base_beam_shape_check(d));
+    ICD_CHECK_ARG(d->start_id >= 0 && d->start_id < d->V && d->end_id >= 0 && d->end_id < d->V,
+                  "baseline_beam_search: start_id / end_id outside the vocabulary");
+    ICD_CHECK_ARG(d->img_features && d->emb_w && d->w_ih && d->w_hh && d->b_ih && d->b_hh && d->lin_w && d->lin_b,
+                  "baseline_beam_search: null input or weight");
+    ICD_CHECK_ARG(d->out_len && d->out_seq && d->out_score, "baseline_beam_search: null result pointer");
+    ICD_CHECK_ARG(d->ws && d->ws_bytes >= (int64_t)carve_base(d, nullptr, nullptr), "baseline_beam_search: workspace too small");
+    return 0;
+}
+
+extern "C" int64_t icd_baseline_beam_search_ws_bytes(const icd_base_beam_desc_t* d) {
+    if (base_beam_shape_check(d) != 0) return -1;         // (the reason is in icd_last_error_string)
+    return (int64_t)carve_base(d, nullptr, nullptr);
+}
+
+extern "C" int icd_baseline_beam_search(const icd_base_beam_desc_t* d, void* stream) {
+    ICD_TRY(base_beam_check(d));                          // every argument before the first CUDA call
+    cudaStream_t s = icd_stream(stream);
+    BeamWs w;
+    carve_base(d, &w, (char*)d->ws);
+    const int n_img = d->n_img, k = d->k, E = d->E, H = d->H, V = d->V, G = 4 * H, prec = d->precision;
+    const long long R = (long long)n_img * k;
+    const int S1 = d->max_steps + 1;
+    const bool x3 = prec == ICD_PREC_FP32X3;
+    const int nseg = icd_x3_three_planes(H) ? 3 : 6;     // layout of the split of h_tmp the cell kernel writes (= beam_mm's)
+
+    if (x3) {                                             // weights are constant over the whole search: split them once
+        ICD_TRY(icd_split3_bf16(d->w_ih, E, G, E, w.x3_WihE, icd_x3_three_planes(E) ? 2 : 1, s));
+        ICD_TRY(icd_split3_bf16(d->w_hh, H, G, H, w.x3_Whh, icd_x3_three_planes(H) ? 2 : 1, s));
+        ICD_TRY(icd_split3_bf16(d->lin_w, H, V, H, w.x3_Wfc, icd_x3_three_planes(H) ? 2 : 1, s));
+    }
+    // an fp64 table is cast to fp32 once (the forward casts the rows it reads, models/baseline.py:101), so it takes the embg path too
+    const float* emb = (const float*)d->emb_w;
+    if (d->emb_is_f64) {
+        const long long n = (long long)V * E;
+        const long long blocks = (n + 255) / 256 < 4 * ICD_NUM_SMS ? (n + 255) / 256 : 4 * ICD_NUM_SMS;
+        f64_to_f32_kernel<<<(unsigned)blocks, 256, 0, s>>>((const double*)d->emb_w, n, w.emb32);
+        ICD_LAUNCH_CHECK();
+        emb = w.emb32;
+    }
+    // embg = emb W_ih^T + b_ih + b_hh for the whole vocabulary, once per call: the per-step input contraction becomes a row gather
+    for (int v0 = 0; v0 < V; v0 += BASE_EMBG_ROWS) {
+        const int nv = V - v0 < BASE_EMBG_ROWS ? V - v0 : BASE_EMBG_ROWS;
+        ICD_TRY(beam_mm(prec, w, emb + (size_t)v0 * E, E, nv, E, d->w_ih, E, w.x3_WihE, w.embg + (size_t)v0 * G, G, G, d->b_ih,
+                        nullptr, 0, 0.f, s, nullptr, false, d->b_hh));
+    }
+    // step 0 (models/baseline.py:101,106): the image feature through one LSTM step from the zero state; its logits are not scored
+    ICD_TRY(beam_mm(prec, w, d->img_features, E, n_img, E, d->w_ih, E, w.x3_WihE, w.z, G, G, d->b_ih, nullptr, 0, 0.f, s, nullptr,
+                    false, d->b_hh));
+    baseline_beam_cell_kernel<<<(unsigned)n_img, 128, 0, s>>>(H, nullptr, nullptr, w.z, nullptr, w.c0, w.h0, nullptr, 0, nullptr);
+    ICD_LAUNCH_CHECK();
+    {
+        const long long n = R * H;
+        beam_init_kernel<<<(unsigned)((n + 255) / 256), 256, 0, s>>>(n_img, k, H, d->start_id, w.h0, w.c0, w.h, w.c,
+                                                                      w.img_index, w.prev_word, w.tok64, w.score, w.k_live,
+                                                                      w.best_score, w.best_step, w.best_parent,
+                                                                      w.slot_img, w.n_live, w.row_off[0]);
+        ICD_LAUNCH_CHECK();
+    }
+    if (d->trace_words) ICD_CUDA(cudaMemsetAsync(d->trace_words, 0xff, sizeof(int32_t) * (size_t)S1 * R, s));
+    const int* live_rows = w.n_live + 1;
+    for (int step = 1; step <= S1; ++step) {               // steps 1 .. max_steps+1: the state machine of icd_beam_search
+        const int* row_off = w.row_off[(step - 1) & 1];
+        int* row_off_next = w.row_off[step & 1];
+        ICD_TRY(beam_mm(prec, w, w.h, H, (int)R, H, d->w_hh, H, w.x3_Whh, w.z, G, G, nullptr, nullptr, 0, 0.f, s, live_rows));
+        baseline_beam_cell_kernel<<<(unsigned)R, 128, 0, s>>>(H, w.embg, w.tok64, w.z, w.c, w.c_tmp, w.h_tmp,
+                                                              x3 ? reinterpret_cast<unsigned short*>(w.x3_act) : nullptr, nseg, w.n_live);
+        ICD_LAUNCH_CHECK();
+        ICD_TRY(beam_mm(prec, w, w.h_tmp, H, (int)R, H, d->lin_w, H, w.x3_Wfc, w.logits, V, V, d->lin_b, nullptr, 0, 0.f, s, live_rows,
+                        x3));
+#define ICD_BASE_TOPK(KT) beam_topk_kernel<KT><<<n_img, 256, 0, s>>>(k, V, step, d->end_id, w.logits, w.score, w.k_live, w.slot_img,     \
+                                               w.n_live, row_off, w.score_tmp, w.word_tmp, w.k_live_tmp, w.slot_img_tmp, w.src,      \
+                                               w.parent + (size_t)(step - 1) * R, w.word + (size_t)(step - 1) * R,                   \
+                                               d->trace_words ? d->trace_words + (size_t)(step - 1) * R : nullptr,                   \
+                                               w.best_score, w.best_step, w.best_parent, 0)
+        switch (k) {
+            case 1: ICD_BASE_TOPK(1); break;
+            case 2: ICD_BASE_TOPK(2); break;
+            case 3: ICD_BASE_TOPK(3); break;
+            case 4: ICD_BASE_TOPK(4); break;
+            case 5: ICD_BASE_TOPK(5); break;
+            case 6: ICD_BASE_TOPK(6); break;
+            default: ICD_BASE_TOPK(8); break;
+        }
+#undef ICD_BASE_TOPK
+        ICD_LAUNCH_CHECK();
+        beam_compact_kernel<<<1, 1024, 0, s>>>(n_img, k, w.k_live_tmp, w.new_slot, w.n_live, row_off_next);
+        ICD_LAUNCH_CHECK();
+        beam_reorder_kernel<<<(unsigned)R, 128, 0, s>>>(k, H, w.new_slot, w.k_live_tmp, w.slot_img_tmp, w.src, w.score_tmp,
+                                                        w.word_tmp, w.h_tmp, w.c_tmp, w.h, w.c, w.score, w.prev_word, w.tok64,
+                                                        w.k_live, w.slot_img, row_off, row_off_next);
+        ICD_LAUNCH_CHECK();
+    }
+    beam_finalize_kernel<<<n_img, 128, 0, s>>>(k, 0, S1, R, d->start_id, d->end_id, w.best_score, w.best_step, w.best_parent,
+                                               w.parent, w.word, nullptr, d->out_len, d->out_seq, d->out_score, nullptr);
     ICD_LAUNCH_CHECK();
     return 0;
 }

@@ -4,6 +4,13 @@
 and return tuple ``(seq, alphas, Caption_End)``; ``beam_search_batched`` decodes many images at once with the
 device-side engine of ``icd_beam_search`` (csrc/beam.cu): no per-step host synchronisation, features indexed per
 image, ``enc_att`` computed once per image.
+
+The reference has no generation function for the ``BaselineDecoder``.  ``baseline_beam_search_batched`` and
+``baseline_caption_image_beam_search`` give it one (``icd_baseline_beam_search``): the same beam state machine over the
+baseline's step.  The image feature is LSTM step 0 from the zero state and its logits are not scored: teacher forcing
+trains ``outputs[:, 0]`` against ``captions[:, 0] = <start>`` (models/baseline.py:93-109), so position 0 of every
+caption is ``<start>`` and the first scored prediction is conditioned on ``emb(<start>)``.  ``beam_size = 1`` is
+greedy decoding.
 """
 import ctypes
 
@@ -11,6 +18,7 @@ import torch
 
 from . import _lib, ops
 from ._lib import check, fill, lib, stream_ptr
+from .models.baseline import BaselineDecoder
 from .vocabulary import END_TOKEN, START_TOKEN
 
 
@@ -78,16 +86,77 @@ def beam_search_batched(decoder, features, beam_size, start_id, end_id, max_step
     return out
 
 
+def baseline_beam_search_batched(decoder, img_features, beam_size, start_id, end_id, max_steps=50, want_trace=False,
+                                 chunk=None, precision="fp32x3"):
+    """Beam search over a ``BaselineDecoder``.  img_features (n_img, E) CUDA — what the baseline encoder returns; cast to
+    fp32 like the forward does (models/baseline.py:101) -> dict with
+         len    (n_img,) int32  caption length incl. <start>/<end>; 0 = no beam completed (failure)
+         seq    (n_img, max_steps+2) int32, seq[:, 0] = <start>
+         score  (n_img,) float32 raw summed log-prob of the winner over steps 1 .. len-1
+         trace  (max_steps+1, n_img, k) int32 next-word ids per step, -1 = empty slot        [want_trace]
+    Step 0 feeds the image feature from the zero LSTM state and is not scored; steps 1 .. max_steps+1 feed emb(previous
+    word), <start> at step 1, with the state machine of ``beam_search_batched`` (gen_captions.py:16-131).  ``beam_size``
+    1 is greedy decoding.  ``precision`` is "fp32x3" (default) or "fp32"; never "bf16": identical captions need
+    fp32-grade logits.  An fp64 (GloVe) embedding table is cast to fp32 once per call."""
+    if precision not in ("fp32", "fp32x3"):
+        raise ValueError("beam search runs in fp32-grade arithmetic only: precision must be 'fp32' or 'fp32x3'")
+    if not img_features.is_cuda:
+        raise _lib.IcdError("baseline_beam_search_batched needs CUDA tensors; there is no CPU fallback")
+    img = img_features.contiguous().float()
+    n_img, E = img.shape
+    k = int(beam_size)
+    dev = img.device
+    lstm, lin = decoder.lstm, decoder.linear
+    ws = [t.detach().contiguous() for t in (lstm.weight_ih_l0, lstm.weight_hh_l0, lstm.bias_ih_l0, lstm.bias_hh_l0,
+                                             lin.weight, lin.bias)]
+    emb_w = decoder.embedding.weight.detach().contiguous()
+    H, V = ws[1].shape[1], ws[4].shape[0]
+    assert emb_w.shape[1] == E, "img_features must have the embedding width %d" % emb_w.shape[1]
+    if chunk is None:
+        chunk = max(1, min(n_img, 65535 // k))
+    S2 = max_steps + 2
+    out = dict(len=torch.empty(n_img, device=dev, dtype=torch.int32),
+               seq=torch.zeros(n_img, S2, device=dev, dtype=torch.int32),
+               score=torch.empty(n_img, device=dev, dtype=torch.float32))
+    traces = []
+    ws_cache = None
+    for i0 in range(0, n_img, chunk):
+        n = min(chunk, n_img - i0)
+        d = _lib.BaseBeamDesc()
+        trace = torch.empty(max_steps + 1, n, k, device=dev, dtype=torch.int32) if want_trace else None
+        fill(d, n_img=n, k=k, max_steps=max_steps, E=E, H=H, V=V, precision=ops.precision_id(precision),
+             emb_is_f64=int(emb_w.dtype == torch.float64), start_id=start_id, end_id=end_id, img_features=img[i0:i0 + n],
+             emb_w=emb_w, w_ih=ws[0], w_hh=ws[1], b_ih=ws[2], b_hh=ws[3], lin_w=ws[4], lin_b=ws[5],
+             out_len=out["len"][i0:i0 + n], out_seq=out["seq"][i0:i0 + n], out_score=out["score"][i0:i0 + n],
+             trace_words=trace)
+        need = int(lib().icd_baseline_beam_search_ws_bytes(ctypes.byref(d)))
+        if ws_cache is None or ws_cache.numel() < need:
+            ws_cache = torch.empty(need, device=dev, dtype=torch.uint8)
+        d.ws = ws_cache.data_ptr()
+        d.ws_bytes = need
+        check(lib().icd_baseline_beam_search(ctypes.byref(d), stream_ptr()), "icd_baseline_beam_search")
+        if want_trace:
+            traces.append(trace)
+    if want_trace:
+        out["trace"] = torch.cat(traces, dim=1)
+    return out
+
+
 def beam_search_sharded(decoder, features_local, beam_size, start_id, end_id, max_steps=50, group=None, dst=0,
                         precision="fp32x3"):
     """BASELINE.json configs[4] / SURVEY.md 8e row 3: images are independent units, so every rank decodes its own shard
     with ``beam_search_batched`` (no collective during the decode) and ONE final gather brings caption lengths, token ids
     and scores to rank ``dst``.  All ranks must hold the same number of images.  Works unchanged in a single process.
+    A ``BaselineDecoder`` takes (n, E) image features per rank and decodes with ``baseline_beam_search_batched``.
     -> on ``dst``: dict(len (world*n,), seq (world*n, max_steps+2), score (world*n,)) in rank order (CUDA tensors);
        elsewhere: None."""
     import torch.distributed as dist
-    res = beam_search_batched(decoder, features_local, beam_size, start_id, end_id, max_steps=max_steps,
-                              want_alphas=False, want_trace=False, precision=precision)
+    if isinstance(decoder, BaselineDecoder):
+        res = baseline_beam_search_batched(decoder, features_local, beam_size, start_id, end_id, max_steps=max_steps,
+                                           want_trace=False, precision=precision)
+    else:
+        res = beam_search_batched(decoder, features_local, beam_size, start_id, end_id, max_steps=max_steps,
+                                  want_alphas=False, want_trace=False, precision=precision)
     if not (dist.is_available() and dist.is_initialized()) or dist.get_world_size(group) == 1:
         return {k: res[k] for k in ("len", "seq", "score")}
     world, rank = dist.get_world_size(group), dist.get_rank(group)
@@ -129,3 +198,28 @@ def attention_caption_image_beam_search(device, args, img, encoder, decoder, voc
     alphas = res["alpha"][0, :n].view(n, enc_image_size, enc_image_size).tolist()
     assert vocab_size == decoder.fc.weight.shape[0]
     return seq, alphas, True
+
+
+def baseline_caption_image_beam_search(device, args, img, encoder, decoder, vocab):
+    """Captions an image with a ``BaselineDecoder`` — the counterpart of ``attention_caption_image_beam_search`` (same
+    arguments, same per-step print of the candidate words) for the decoder the reference cannot generate with.
+
+    ``encoder(img)`` returns the (1, E) image feature.  Returns ``(seq, Caption_End)``: ``seq`` a python list of token ids
+    including <start> and <end>, or ``([start, end], False)`` when no beam emitted <end> within 51 steps.  Step 0 (the
+    image feature) is not scored; position 0 is <start> (see the module docstring).  ``args.beam_size = 1`` is greedy."""
+    k = args.beam_size
+    features = encoder(img)
+    start_id, end_id = vocab(START_TOKEN), vocab(END_TOKEN)
+    with torch.no_grad():
+        res = baseline_beam_search_batched(decoder, features.reshape(1, -1), k, start_id, end_id, max_steps=50,
+                                           want_trace=True)
+    n = int(res["len"][0].item())
+    for words in res["trace"][:, 0, :].tolist():                                   # per-step print of the candidates
+        live = [w for w in words if w >= 0]
+        if not live:
+            break
+        print([vocab.i2w[w] for w in live])
+    if n == 0:
+        return [start_id, end_id], False
+    assert len(vocab) == decoder.linear.weight.shape[0]
+    return res["seq"][0, :n].tolist(), True

@@ -7,7 +7,7 @@
  *   models/attention.py:151-164 AttentionDecoder.init_hidden_state
  *   models/attention.py:218-284 AttentionDecoder.forward (+ its autograd backward)
  *   models/baseline.py:81-111   BaselineDecoder.forward  (+ its autograd backward)
- *   gen_captions.py:16-131      attention_caption_image_beam_search
+ *   gen_captions.py:16-131      attention_caption_image_beam_search (+ the same search over BaselineDecoder steps)
  *   train_utils.py:2-12 + models/attention.py:417-430   clamp(+-grad_clip) + Adam step
  * Each entry point below names the reference lines it replaces.  A reference maintainer binds
  * them with ctypes (see INTEGRATION.md); no torch types cross this boundary.
@@ -36,7 +36,7 @@
 extern "C" {
 #endif
 
-#define ICD_B200_ABI_VERSION 15
+#define ICD_B200_ABI_VERSION 16
 #define ICD_MAX_STEPS 256
 
 ICD_API int icd_version(void);                       /* ICD_B200_ABI_VERSION the library was built with */
@@ -44,6 +44,7 @@ ICD_API const char* icd_last_error_string(void);     /* per-thread, valid until 
 ICD_API int icd_sizeof_att_desc(void);               /* sizeof(icd_att_desc_t)  — struct-layout self check */
 ICD_API int icd_sizeof_base_desc(void);
 ICD_API int icd_sizeof_beam_desc(void);
+ICD_API int icd_sizeof_base_beam_desc(void);
 ICD_API int icd_has_tensor_core_gemm(void);          /* 1 if the tcgen05/TMA GEMM path was compiled in     */
 /* Tile pairing of the tensor-core contraction (also env ICD_GEMM_PAIR): 0 single-CTA tiles, 1 CTA pairs sharing the B tile
  * by TMA multicast, 2 CTA pairs on one 256-row tile with tcgen05.mma.cta_group::2; any other value restores the built-in
@@ -411,6 +412,37 @@ typedef struct {
 
 ICD_API int64_t icd_beam_search_ws_bytes(const icd_beam_desc_t* d);
 ICD_API int icd_beam_search(const icd_beam_desc_t* d, void* stream);
+
+/* ------------------------------------------------------------------------------------------------
+ * Batched beam search for the BaselineDecoder (models/baseline.py:81-111 run autoregressively; the reference has no
+ * generation function for this decoder).  The state machine is that of icd_beam_search; the decoder step is the
+ * baseline's: the image feature is LSTM step 0 from the zero state (its logits are not scored, position 0 of every
+ * caption is <start>), then steps 1 .. max_steps+1 feed emb(previous word), with <start> at step 1, through one LSTM step
+ * (gate order i,f,g,o, b_ih + b_hh) and the vocabulary layer.  k = 1 is greedy decoding.  An fp64 embedding table is
+ * cast to fp32 once per call (what the forward does with its rows, models/baseline.py:101).
+ * precision: ICD_PREC_FP32 or ICD_PREC_FP32X3 (identical captions need fp32-grade logits).
+ * Every argument is validated before the first CUDA call.
+ * ---------------------------------------------------------------------------------------------- */
+typedef struct {
+    int32_t n_img, k, max_steps;  /* k in 1..8, n_img*k <= 65535; loop body runs for step = 1 .. max_steps+1 */
+    int32_t E, H, V;              /* E, H multiples of 4; V >= k */
+    int32_t precision, emb_is_f64;
+    int32_t start_id, end_id;
+    const float* img_features;    /* (n_img,E) fp32 */
+    const void* emb_w;            /* (V,E) fp32 or fp64 */
+    const float *w_ih, *w_hh, *b_ih, *b_hh;   /* (4H,E) (4H,H) (4H) (4H) */
+    const float *lin_w, *lin_b;   /* (V,H) (V) */
+    /* results (device), as in icd_beam_desc_t */
+    int32_t* out_len;             /* (n_img)   length of best completed caption incl. <start>/<end>; 0 => none completed */
+    int32_t* out_seq;             /* (n_img, max_steps+2) */
+    float* out_score;             /* (n_img)   raw summed log-prob of the winner (steps >= 1) */
+    int32_t* trace_words;         /* (max_steps+1, n_img, k) next-word ids per step, -1 = empty slot; may be NULL */
+    /* workspace (device) */
+    void* ws; int64_t ws_bytes;   /* >= icd_baseline_beam_search_ws_bytes(desc) */
+} icd_base_beam_desc_t;
+
+ICD_API int64_t icd_baseline_beam_search_ws_bytes(const icd_base_beam_desc_t* d);   /* -1: shape refused (see the error string) */
+ICD_API int icd_baseline_beam_search(const icd_base_beam_desc_t* d, void* stream);
 
 /* ------------------------------------------------------------------------------------------------
  * Optimiser glue: element-wise gradient clamp to +-grad_clip (train_utils.py:2-12) fused with the
