@@ -404,21 +404,82 @@ bool persistent_enabled() {
     return on;
 }
 
+// dynamic shared memory of one CTA for B rows and hidden size H (the backward adds the DSMEM exchange buffer); 0 if fewer
+// than 2 A stages fit beside the resident weight slice
+int seq_smem(int BWD, int B, int H, int* stages) {
+    const int MT = (B + LP_BM - 1) / LP_BM;
+    const int smem = plan_smem((H + TC_BK - 1) / TC_BK, BWD ? MT * 4 * LP_BM * 16 : 0, stages);
+    return *stages >= 2 ? smem : 0;
+}
+
+// raise the kernel's dynamic-shared-memory limit to at least smem (never lowers it: other shapes may be in flight)
+template <int BWD>
+cudaError_t ensure_smem_attr(int smem) {
+    static int smem_set = 0;
+    if (smem_set >= smem) return cudaSuccess;
+    const cudaError_t e = cudaFuncSetAttribute(lstm_seq_kernel<BWD>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem);
+    if (e == cudaSuccess) smem_set = smem;
+    return e;
+}
+
+// the pure shape rules: whole 16-unit groups, one forward CTA per SM at most, every row tile's accumulator in the TMEM
+// allocation, at least 2 A stages beside the resident weight slice
+bool shape_ok(int B, int L, int H) {
+    if (B < 1 || L < 1 || H < 16 || H % 16 != 0) return false;
+    if (H / 4 > ICD_NUM_SMS) return false;
+    if ((B + LP_BM - 1) / LP_BM > LP_MAX_MT) return false;
+    int st;
+    return seq_smem(1, B, H, &st) > 0;
+}
+
+// Co-residency, read from the occupancy calculator at the shared memory each direction launches with: the forward grid
+// (H/4 CTAs) needs blocks-per-SM x SMs >= H/4, the backward (H/16 clusters of 4) needs as many co-resident 4-CTA clusters.
+// Clusters cannot span GPCs, so the second answer is not implied by the first.  Launches nothing.
+// -> 0 and the two capacities, or -1 if a query failed (its error is consumed).
+int query_residency(int B, int H, int* fwd_ctas, int* bwd_clusters) {
+    *fwd_ctas = 0; *bwd_clusters = 0;
+    int st, dev = 0, sms = 0, per_sm = 0;
+    const int smem_f = seq_smem(0, B, H, &st), smem_b = seq_smem(1, B, H, &st);
+    if (!smem_f || !smem_b) return 0;
+    bool ok = cudaGetDevice(&dev) == cudaSuccess && cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev) == cudaSuccess &&
+              ensure_smem_attr<0>(smem_f) == cudaSuccess && ensure_smem_attr<1>(smem_b) == cudaSuccess &&
+              cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, lstm_seq_kernel<0>, LP_THREADS, (size_t)smem_f) == cudaSuccess;
+    if (ok) {
+        cudaLaunchConfig_t cfg = {};
+        cfg.gridDim = dim3(H / 4); cfg.blockDim = dim3(LP_THREADS); cfg.dynamicSmemBytes = (size_t)smem_b;
+        cudaLaunchAttribute at[1];
+        at[0].id = cudaLaunchAttributeClusterDimension;
+        at[0].val.clusterDim.x = 4; at[0].val.clusterDim.y = 1; at[0].val.clusterDim.z = 1;
+        cfg.attrs = at; cfg.numAttrs = 1;
+        ok = cudaOccupancyMaxActiveClusters(bwd_clusters, lstm_seq_kernel<1>, &cfg) == cudaSuccess;
+    }
+    if (!ok) { (void)cudaGetLastError(); *bwd_clusters = 0; return -1; }
+    *fwd_ctas = per_sm * sms;
+    return 0;
+}
+
+// 1 if both grids of (B, H) are co-resident; cached per shape class (row tiles, H): the answer depends on nothing else.
+// A failed query refuses the shape.
+bool resident(int B, int H) {
+    static signed char cache[LP_MAX_MT + 1][ICD_NUM_SMS / 4 + 1] = {};     // 0 unknown, 1 fits, -1 refused
+    signed char& c = cache[(B + LP_BM - 1) / LP_BM][H / 16];
+    if (c == 0) {
+        int f, b;
+        c = (query_residency(B, H, &f, &b) == 0 && f >= H / 4 && b >= H / 16) ? 1 : -1;
+    }
+    return c == 1;
+}
+
 // A16: the bf16 activation stack [a_rows][a_cols] the per-step A operands are cut from (a.K = this CTA's contraction length)
 template <int BWD>
 int launch_seq(const LstmSeqArgs& a0, const __nv_bfloat16* A16, int a_rows, int a_cols, cudaStream_t s) {
     LstmSeqArgs a = a0;
     a.nkb = (a.K + TC_BK - 1) / TC_BK;
-    const int MT = (a.B + LP_BM - 1) / LP_BM;
-    const int smem = plan_smem(a.nkb, BWD ? MT * 4 * LP_BM * 16 : 0, &a.stages);
-    ICD_CHECK_ARG(a.stages >= 2, "lstm_seq: hidden size %d too large for the resident weight slice", a.H);
+    const int smem = seq_smem(BWD, a.B, a.H, &a.stages);
+    ICD_CHECK_ARG(smem > 0, "lstm_seq: hidden size %d too large for the resident weight slice", a.H);
     CUtensorMap tmA;
     ICD_TRY(make_tmap(&tmA, A16, a_cols, a_rows, a_cols, LP_BM, 0));
-    static int smem_set = 0;
-    if (smem_set < smem) {
-        ICD_CUDA(cudaFuncSetAttribute(lstm_seq_kernel<BWD>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem));
-        smem_set = smem;
-    }
+    ICD_CUDA(ensure_smem_attr<BWD>(smem));
     ICD_CUDA(cudaMemsetAsync(a.bar, 0, sizeof(unsigned int), s));
     const int grid = a.H / 4;                              // forward: 4 units per CTA; backward: 16 units per 4-CTA cluster
     cudaLaunchConfig_t cfg = {};
@@ -431,9 +492,10 @@ int launch_seq(const LstmSeqArgs& a0, const __nv_bfloat16* A16, int a_rows, int 
     cfg.attrs = attr; cfg.numAttrs = BWD ? 2 : 1;
     cudaError_t e = cudaLaunchKernelEx(&cfg, lstm_seq_kernel<BWD>, tmA, a);
     if (BWD && e == cudaSuccess) g_bwd_launch_mode = 1;
-    if (e != cudaSuccess && BWD) {
-        // a driver that refuses cooperative + cluster launches: the grid (<= 148 CTAs, one per SM, launched on an otherwise
-        // ordered stream) is co-resident in practice; the barrier's spin limit turns a violation into a fault, not a hang
+    if (e != cudaSuccess && BWD && resident(a.B, a.H)) {
+        // a driver that refuses cooperative + cluster launches: the occupancy query said every cluster of this grid is
+        // co-resident on an idle device, so the grid barrier completes once the stream's earlier work has drained; the
+        // barrier's spin limit turns a violation into a fault, not a hang
         (void)cudaGetLastError();
         cfg.attrs = attr + 1; cfg.numAttrs = 1;
         e = cudaLaunchKernelEx(&cfg, lstm_seq_kernel<BWD>, tmA, a);
@@ -446,16 +508,12 @@ int launch_seq(const LstmSeqArgs& a0, const __nv_bfloat16* A16, int a_rows, int 
 
 }  // namespace
 
-// 1 if the persistent kernels cover this shape (else the caller keeps its launch chain): every CTA must be co-resident
-// (grid <= #SMs), the accumulator of all row tiles must fit the TMEM allocation, H must split into whole unit groups.
+// 1 if the persistent kernels cover this shape (else the caller keeps its launch chain): the pure shape rules first, then
+// co-residency of both directions' grids as the occupancy calculator reports it for this device (the grid barrier needs
+// every CTA resident at once).
 int icd_lstm_seq_persistent_ok(int B, int L, int H) {
     if (!persistent_enabled()) return 0;
-    if (B < 1 || L < 1 || H < 16 || H % 16 != 0) return 0;
-    if (H / 4 > ICD_NUM_SMS) return 0;
-    if ((B + LP_BM - 1) / LP_BM > LP_MAX_MT) return 0;
-    int st;
-    plan_smem((H + TC_BK - 1) / TC_BK, ((B + LP_BM - 1) / LP_BM) * 4 * LP_BM * 16, &st);
-    return st >= 2 ? 1 : 0;
+    return shape_ok(B, L, H) && resident(B, H) ? 1 : 0;
 }
 
 int icd_lstm_seq_fwd_persistent(int B, int L, int H, const float* w_hh, const float* xg, float* gates_act, float* c_all,
@@ -479,6 +537,13 @@ int icd_lstm_seq_bwd_persistent(int B, int L, int H, const float* w_hh, const fl
 
 // ---- C ABI (include/icd_b200.h): the LSTM recurrence on its own, for callers that hoist the input contraction themselves ----
 extern "C" int icd_lstm_seq_supported(int B, int L, int H) { return icd_lstm_seq_persistent_ok(B, L, H); }
+extern "C" int icd_lstm_seq_shape_ok(int B, int L, int H) { return shape_ok(B, L, H) ? 1 : 0; }
+extern "C" int icd_lstm_seq_residency(int B, int H, int* fwd_ctas, int* bwd_clusters) {
+    ICD_CHECK_ARG(fwd_ctas && bwd_clusters, "lstm_seq_residency: null output");
+    ICD_CHECK_ARG(shape_ok(B, 1, H), "lstm_seq_residency: shape B=%d H=%d fails the shape rules", B, H);
+    ICD_CHECK_ARG(query_residency(B, H, fwd_ctas, bwd_clusters) == 0, "lstm_seq_residency: occupancy query failed");
+    return 0;
+}
 extern "C" int icd_lstm_seq_bwd_launch_mode(void) { return g_bwd_launch_mode; }
 
 extern "C" int icd_lstm_seq_fwd(int B, int L, int H, const float* w_hh, const float* xg, float* gates_act, float* c_all,

@@ -36,7 +36,7 @@
 extern "C" {
 #endif
 
-#define ICD_B200_ABI_VERSION 16
+#define ICD_B200_ABI_VERSION 17
 #define ICD_MAX_STEPS 256
 
 ICD_API int icd_version(void);                       /* ICD_B200_ABI_VERSION the library was built with */
@@ -373,12 +373,20 @@ ICD_API int icd_baseline_decoder_bwd(const icd_base_desc_t* d, void* stream);
  *   backward: d_hout (B,L,H) in; gates_act, c_all from the forward; dc_ws (B,H) scratch; dg (L,B,4H) fp32 and
  *             dg16 (L*B, 4H) bf16 out — d(loss)/d(gates_pre), the operand of every weight / input gradient contraction
  *   barrier_ws: >= 4 bytes of device memory (the grid-barrier counter).
- * icd_lstm_seq_supported: 1 if (B, L, H) is covered: H a multiple of 16, H/4 <= #SMs (every CTA co-resident), B <= 512;
- * otherwise callers keep a per-step launch chain (icd_baseline_decoder_fwd does that by itself).
+ * icd_lstm_seq_shape_ok: the pure shape rules, no device needed: L >= 1, H a multiple of 16, H/4 <= 148 (one forward CTA per
+ * SM), B <= 512 (4 row tiles of 128), and room for the resident weight slice.
+ * icd_lstm_seq_supported: 1 if (B, L, H) passes the shape rules AND both grids are co-resident on the current device at the
+ * shared memory they launch with (forward: H/4 CTAs; backward: H/16 clusters of 4 CTAs), as the occupancy calculator says;
+ * cached per (row tiles, H).  Otherwise callers keep a per-step launch chain (icd_baseline_decoder_fwd does that by itself).
+ * icd_lstm_seq_residency: diagnostic, launches nothing — how many forward CTAs (blocks per SM x SMs) and how many
+ * backward 4-CTA clusters the device can hold at once at the shared memory (B, H) launches with.
  * ---------------------------------------------------------------------------------------------- */
+ICD_API int icd_lstm_seq_shape_ok(int B, int L, int H);
 ICD_API int icd_lstm_seq_supported(int B, int L, int H);
+ICD_API int icd_lstm_seq_residency(int B, int H, int* fwd_ctas, int* bwd_clusters);
 /* diagnostic: how the last backward recurrence was launched — 0 not yet, 1 cooperative + 4-CTA clusters (co-residency
- * guaranteed by the driver), 2 plain cluster launch (a driver that refuses the combination; co-resident in practice) */
+ * guaranteed by the driver), 2 plain cluster launch (a driver that refuses the combination; only for a grid the occupancy
+ * query found co-resident) */
 ICD_API int icd_lstm_seq_bwd_launch_mode(void);
 ICD_API int icd_lstm_seq_fwd(int B, int L, int H, const float* w_hh, const float* xg, float* gates_act, float* c_all,
                      float* h_all, float* hout, void* h16, void* hout16, void* barrier_ws, void* stream);
