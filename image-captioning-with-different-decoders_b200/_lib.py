@@ -70,6 +70,8 @@ AttDesc = _make_struct("icd_att_desc_t")
 BaseDesc = _make_struct("icd_base_desc_t")
 BeamDesc = _make_struct("icd_beam_desc_t")
 BaseBeamDesc = _make_struct("icd_base_beam_desc_t")
+SampleDesc = _make_struct("icd_sample_desc_t")
+BaseSampleDesc = _make_struct("icd_base_sample_desc_t")
 
 PREC_FP32 = DEFINES["ICD_PREC_FP32"]
 PREC_BF16 = DEFINES["ICD_PREC_BF16"]
@@ -96,6 +98,8 @@ def lib():
     L.icd_last_error_string.restype = ctypes.c_char_p
     L.icd_beam_search_ws_bytes.restype = ctypes.c_int64
     L.icd_baseline_beam_search_ws_bytes.restype = ctypes.c_int64
+    L.icd_sample_captions_ws_bytes.restype = ctypes.c_int64
+    L.icd_baseline_sample_captions_ws_bytes.restype = ctypes.c_int64
     L.icd_attention_proj_bwd_ws_floats.restype = ctypes.c_int64
     L.icd_launch_count.restype = ctypes.c_int64
     L.icd_gemm_ws_bytes.restype = ctypes.c_int64
@@ -106,7 +110,8 @@ def lib():
         raise IcdError("libicd_b200.so ABI %d != header ABI %d — rebuild" %
                        (L.icd_version(), DEFINES["ICD_B200_ABI_VERSION"]))
     for fn, st in (("icd_sizeof_att_desc", AttDesc), ("icd_sizeof_base_desc", BaseDesc),
-                   ("icd_sizeof_beam_desc", BeamDesc), ("icd_sizeof_base_beam_desc", BaseBeamDesc)):
+                   ("icd_sizeof_beam_desc", BeamDesc), ("icd_sizeof_base_beam_desc", BaseBeamDesc),
+                   ("icd_sizeof_sample_desc", SampleDesc), ("icd_sizeof_base_sample_desc", BaseSampleDesc)):
         if getattr(L, fn)() != ctypes.sizeof(st):
             raise IcdError("%s: C says %d bytes, ctypes says %d" % (fn, getattr(L, fn)(), ctypes.sizeof(st)))
     _lib = L

@@ -113,4 +113,6 @@ int icd_sizeof_att_desc(void) { return (int)sizeof(icd_att_desc_t); }
 int icd_sizeof_base_desc(void) { return (int)sizeof(icd_base_desc_t); }
 int icd_sizeof_beam_desc(void) { return (int)sizeof(icd_beam_desc_t); }
 int icd_sizeof_base_beam_desc(void) { return (int)sizeof(icd_base_beam_desc_t); }
+int icd_sizeof_sample_desc(void) { return (int)sizeof(icd_sample_desc_t); }
+int icd_sizeof_base_sample_desc(void) { return (int)sizeof(icd_base_sample_desc_t); }
 }

@@ -21,7 +21,7 @@
 // icd_baseline_beam_search runs the same state machine (the same top-k, compaction, reorder and finalize kernels) over the
 // BaselineDecoder's step: the image feature as LSTM step 0 from the zero state, then per step h W_hh^T on the live rows, one fused
 // kernel for the embg gather + LSTMCell (+ the split of h for the fp32-grade vocabulary contraction), and the vocabulary layer.
-#include "common.cuh"
+#include "beam.cuh"
 #include "gemm_tc.cuh"
 #include <cuda_bf16.h>
 #include <stdlib.h>
@@ -31,23 +31,6 @@ namespace {
 constexpr int TOPK_NL = 19;     // 64-bit loads per thread of the register-resident top-k pass: rows of up to 2 * 256 * 19 = 9728 logits
 constexpr int TOPK_CAP = 512;   // shared candidate list of that pass (logits >= tau of one row); more (massive ties): the streaming pass
 constexpr int KMAX = 8;          // beam slots per image supported by the top-k kernel
-
-struct BeamWs {
-    float *att_enc, *mean, *h0, *c0, *h, *c, *h_tmp, *c_tmp, *w_cat, *b_cat, *emb_x, *z, *gated, *gates_pre,
-          *gates_act_unused, *logits, *alpha_steps, *score, *best_score, *embg;
-    int *img_index, *prev_word, *k_live, *src, *parent, *word, *best_step, *best_parent;
-    int *slot_img, *slot_img_tmp, *k_live_tmp, *new_slot, *n_live, *word_tmp;   // n_live[0] = live slots, [1] = live rows
-    int* ring_ticket;                                                           // one slot-ticket counter per step (attention ring kernel)
-    int *row_off[2];                                                            // slot -> first state row (ping-pong per step)
-    float* score_tmp;
-    long long* tok64;
-    // ICD_PREC_FP32X3: 3-term bf16 splits (gemm_tc.cu) of the weights (once per call) and of the step activations
-    void *x3_We, *x3_Wcat, *x3_WihE, *x3_WihC, *x3_Wh, *x3_Wc, *x3_Wfc, *x3_act;
-    float* x3_splitk; long long x3_splitk_floats;
-    // baseline decoder only (carve_base): fp32 copy of an fp64 embedding table, split of W_hh
-    float* emb32;
-    void* x3_Whh;
-};
 
 inline long long up8ll(long long x) { return (x + 7) / 8 * 8; }
 constexpr int X3_IMG_CHUNK = 64;          // most images per enc_att projection pass (bounds the split activation scratch)
@@ -66,7 +49,9 @@ inline int x3_img_chunk(int P, int A) {
     return best;
 }
 
-size_t carve(const icd_beam_desc_t* d, BeamWs* w, char* base) {
+}  // namespace
+
+size_t carve(const icd_beam_desc_t* d, BeamWs* w, char* base, bool history) {
     const size_t R = (size_t)d->n_img * d->k, S = (size_t)d->max_steps + 1;
     const int P = d->P, C = d->C, A = d->A, D = d->D, E = d->E, V = d->V, NZ = A + C + 4 * D;
     size_t off = 0;
@@ -82,17 +67,20 @@ size_t carve(const icd_beam_desc_t* d, BeamWs* w, char* base) {
     TAKE_F(emb_x, R * E) TAKE_F(z, R * NZ) TAKE_F(gated, R * C) TAKE_F(gates_pre, R * 4 * D)
     TAKE_F(logits, R * V)
     TAKE_F(embg, d->emb_is_f64 ? 0 : (size_t)V * 4 * D)       // embedding row x W_ih[:, :E]^T + b_ih for EVERY token, once per call
-    TAKE_F(alpha_steps, S * R * P)
+    TAKE_F(alpha_steps, (history ? S : 1) * R * P)
     TAKE_F(score, R) TAKE_F(score_tmp, R) TAKE_F(best_score, (size_t)d->n_img)
 #undef TAKE_F
     int* ip;
 #define TAKE_I(name, n) ip = (int*)take(sizeof(int) * (n)); if (w) w->name = ip;
     TAKE_I(img_index, R) TAKE_I(prev_word, R) TAKE_I(k_live, (size_t)d->n_img) TAKE_I(src, R)
-    TAKE_I(parent, S * R) TAKE_I(word, S * R) TAKE_I(best_step, (size_t)d->n_img) TAKE_I(best_parent, (size_t)d->n_img)
+    TAKE_I(parent, history ? S * R : 0) TAKE_I(word, history ? S * R : 0) TAKE_I(best_step, (size_t)d->n_img)
+    TAKE_I(best_parent, (size_t)d->n_img)
     TAKE_I(slot_img, (size_t)d->n_img) TAKE_I(slot_img_tmp, (size_t)d->n_img) TAKE_I(k_live_tmp, (size_t)d->n_img)
     TAKE_I(new_slot, (size_t)d->n_img) TAKE_I(n_live, 4) TAKE_I(word_tmp, R) TAKE_I(ring_ticket, S + 2)
     ip = (int*)take(sizeof(int) * (size_t)d->n_img); if (w) w->row_off[0] = ip;
     ip = (int*)take(sizeof(int) * (size_t)d->n_img); if (w) w->row_off[1] = ip;
+    if (w) w->tag = w->tag_tmp = nullptr;
+    if (!history) { TAKE_I(tag, R) TAKE_I(tag_tmp, R) }
 #undef TAKE_I
     long long* lp = (long long*)take(sizeof(long long) * R); if (w) w->tok64 = lp;
     if (d->precision == ICD_PREC_FP32X3) {
@@ -114,6 +102,8 @@ size_t carve(const icd_beam_desc_t* d, BeamWs* w, char* base) {
     }
     return off;
 }
+
+namespace {
 
 __global__ void beam_init_kernel(int n_img, int k, int D, int start_id, const float* __restrict__ h0,
                                  const float* __restrict__ c0, float* __restrict__ h, float* __restrict__ c,
@@ -423,7 +413,8 @@ __global__ void beam_reorder_kernel(int k, int D, const int* __restrict__ new_sl
                                     float* __restrict__ h, float* __restrict__ c, float* __restrict__ score,
                                     int* __restrict__ prev_word, long long* __restrict__ tok64,
                                     int* __restrict__ k_live, int* __restrict__ slot_img,
-                                    const int* __restrict__ row_off_old, const int* __restrict__ row_off_new) {
+                                    const int* __restrict__ row_off_old, const int* __restrict__ row_off_new,
+                                    const int* __restrict__ tag_tmp, int* __restrict__ tag) {   // tag: optional (sampler)
     const int r = blockIdx.x;                       // (old slot, surviving beam j): index into the *_tmp arrays
     const int s = r / k, j = r % k;
     const int dslot = new_slot[s];
@@ -436,6 +427,7 @@ __global__ void beam_reorder_kernel(int k, int D, const int* __restrict__ new_sl
     if (threadIdx.x == 0) {
         score[dr] = score_tmp[r];
         prev_word[dr] = word_tmp[r]; tok64[dr] = word_tmp[r];
+        if (tag) tag[dr] = tag_tmp[r];
         if (j == 0) { k_live[dslot] = kl; slot_img[dslot] = slot_img_tmp[s]; }
     }
 }
@@ -570,7 +562,9 @@ __global__ void __launch_bounds__(256) split3_mean_kernel(int P, int C, const fl
 // W_ih (x3_WihE), W_hh (x3_Whh) and the vocabulary layer (x3_Wfc).
 constexpr int BASE_EMBG_ROWS = 4096;      // vocabulary rows per embg pass (bounds the split activation scratch)
 
-size_t carve_base(const icd_base_beam_desc_t* d, BeamWs* w, char* base) {
+}  // namespace
+
+size_t carve_base(const icd_base_beam_desc_t* d, BeamWs* w, char* base, bool history) {
     const size_t R = (size_t)d->n_img * d->k, S = (size_t)d->max_steps + 1;
     const int E = d->E, H = d->H, V = d->V, G = 4 * H;
     size_t off = 0;
@@ -588,11 +582,14 @@ size_t carve_base(const icd_base_beam_desc_t* d, BeamWs* w, char* base) {
     int* ip;
 #define TAKE_I(name, n) ip = (int*)take(sizeof(int) * (n)); if (w) w->name = ip;
     TAKE_I(img_index, R) TAKE_I(prev_word, R) TAKE_I(k_live, (size_t)d->n_img) TAKE_I(src, R)
-    TAKE_I(parent, S * R) TAKE_I(word, S * R) TAKE_I(best_step, (size_t)d->n_img) TAKE_I(best_parent, (size_t)d->n_img)
+    TAKE_I(parent, history ? S * R : 0) TAKE_I(word, history ? S * R : 0) TAKE_I(best_step, (size_t)d->n_img)
+    TAKE_I(best_parent, (size_t)d->n_img)
     TAKE_I(slot_img, (size_t)d->n_img) TAKE_I(slot_img_tmp, (size_t)d->n_img) TAKE_I(k_live_tmp, (size_t)d->n_img)
     TAKE_I(new_slot, (size_t)d->n_img) TAKE_I(n_live, 4) TAKE_I(word_tmp, R)
     ip = (int*)take(sizeof(int) * (size_t)d->n_img); if (w) w->row_off[0] = ip;
     ip = (int*)take(sizeof(int) * (size_t)d->n_img); if (w) w->row_off[1] = ip;
+    if (w) w->tag = w->tag_tmp = nullptr;
+    if (!history) { TAKE_I(tag, R) TAKE_I(tag_tmp, R) }
 #undef TAKE_I
     long long* lp = (long long*)take(sizeof(long long) * R); if (w) w->tok64 = lp;
     if (d->precision == ICD_PREC_FP32X3) {
@@ -613,6 +610,8 @@ size_t carve_base(const icd_base_beam_desc_t* d, BeamWs* w, char* base) {
     }
     return off;
 }
+
+namespace {
 
 // The baseline decoder's step after the W_hh contraction, one CTA per live row r:
 //   gates = embg[tok[r]] + z[r]   (embg = emb W_ih^T + b_ih + b_hh for the whole vocabulary, z = h W_hh^T of this step)
@@ -712,27 +711,9 @@ int beam_mm(int prec, const BeamWs& w, const float* x, long long ldx, int rows, 
     return rc;
 }
 
-extern "C" int64_t icd_beam_search_ws_bytes(const icd_beam_desc_t* d) {
-    if (!d) return -1;
-    return (int64_t)carve(d, nullptr, nullptr);
-}
-
-extern "C" int icd_beam_search(const icd_beam_desc_t* d, void* stream) {
-    ICD_CHECK_ARG(d != nullptr, "beam_search: null descriptor");
-    ICD_CHECK_ARG(d->n_img > 0 && d->k >= 1 && d->k <= KMAX, "beam_search: n_img=%d k=%d (k <= %d)", d->n_img, d->k, KMAX);
-    ICD_CHECK_ARG(d->max_steps >= 1 && d->max_steps + 1 <= ICD_MAX_STEPS, "beam_search: max_steps=%d out of range", d->max_steps);
-    ICD_CHECK_ARG(d->V >= d->k, "beam_search: vocabulary smaller than the beam");
-    ICD_CHECK_ARG(d->A % 4 == 0 && d->C % 4 == 0 && d->D % 4 == 0 && d->E % 4 == 0, "beam_search: dims must be multiples of 4");
-    ICD_CHECK_ARG(d->ws && d->ws_bytes >= icd_beam_search_ws_bytes(d), "beam_search: workspace too small");
-    cudaStream_t s = icd_stream(stream);
-    BeamWs w;
-    carve(d, &w, (char*)d->ws);
-    const int n_img = d->n_img, k = d->k, P = d->P, C = d->C, A = d->A, D = d->D, E = d->E, V = d->V;
+int beam_att_prologue(const icd_beam_desc_t* d, BeamWs& w, bool* use_embg_out, cudaStream_t s) {
+    const int n_img = d->n_img, P = d->P, C = d->C, A = d->A, D = d->D, E = d->E, V = d->V;
     const int NZ = A + C + 4 * D, prec = d->precision;
-    const long long R = (long long)n_img * k;
-    ICD_CHECK_ARG(R <= 65535, "beam_search: n_img*k=%lld exceeds 65535 rows per call (chunk the images)", R);
-    const int S1 = d->max_steps + 1;
-
     ICD_CUDA(cudaMemcpyAsync(w.w_cat, d->dec_att_w, sizeof(float) * (size_t)A * D, cudaMemcpyDeviceToDevice, s));
     ICD_CUDA(cudaMemcpyAsync(w.w_cat + (size_t)A * D, d->f_beta_w, sizeof(float) * (size_t)C * D, cudaMemcpyDeviceToDevice, s));
     ICD_CUDA(cudaMemcpyAsync(w.w_cat + (size_t)(A + C) * D, d->w_hh, sizeof(float) * (size_t)4 * D * D, cudaMemcpyDeviceToDevice, s));
@@ -754,6 +735,7 @@ extern "C" int icd_beam_search(const icd_beam_desc_t* d, void* stream) {
     // embedding -> gate contribution for the whole vocabulary, once per call: V rows instead of (live rows) x (steps) rows, and
     // no per-step activation split of the embedding rows (fp32 tables; an fp64 GloVe table keeps the per-step contraction)
     const bool use_embg = !d->emb_is_f64 && (NZ % 4 == 0) && ((A + C) % 4 == 0);
+    *use_embg_out = use_embg;
     if (use_embg) {
         const int VC = 4096;                                 // rows per pass: bounds the split scratch (x3_act holds >= 64*P rows of C)
         for (int v0 = 0; v0 < V; v0 += VC) {
@@ -781,48 +763,95 @@ extern "C" int icd_beam_search(const icd_beam_desc_t* d, void* stream) {
         ICD_TRY(icd_weighted_pixel_sum(n_img, P, C, nullptr, d->enc, nullptr, 0, nullptr, 0, w.mean, nullptr, nullptr, s));
     ICD_TRY(beam_mm(prec, w, w.mean, C, n_img, C, d->h_lin_w, C, w.x3_Wh, w.h0, D, D, d->h_lin_b, nullptr, 0, 0.f, s));
     ICD_TRY(beam_mm(prec, w, w.mean, C, n_img, C, d->c_lin_w, C, w.x3_Wc, w.c0, D, D, d->c_lin_b, nullptr, 0, 0.f, s));
-    {
-        const long long n = R * D;
-        beam_init_kernel<<<(unsigned)((n + 255) / 256), 256, 0, s>>>(n_img, k, D, d->start_id, w.h0, w.c0, w.h, w.c,
-                                                                      w.img_index, w.prev_word, w.tok64, w.score, w.k_live,
-                                                                      w.best_score, w.best_step, w.best_parent,
-                                                                      w.slot_img, w.n_live, w.row_off[0]);
+    return 0;
+}
+
+int beam_att_step(const icd_beam_desc_t* d, BeamWs& w, int step, bool use_embg, const int* row_off, float* alpha_s, cudaStream_t s) {
+    const int n_img = d->n_img, k = d->k, P = d->P, C = d->C, A = d->A, D = d->D, E = d->E, V = d->V;
+    const int NZ = A + C + 4 * D, prec = d->precision;
+    const long long R = (long long)n_img * k;
+    const int* live_rows = w.n_live + 1;
+    if (!use_embg) {
+        gather_rows_kernel<<<(unsigned)R, 128, 0, s>>>(d->emb_is_f64 ? nullptr : (const float*)d->emb_w,
+                                                       d->emb_is_f64 ? (const double*)d->emb_w : nullptr,
+                                                       w.tok64, E, w.emb_x, w.n_live);       // :65
         ICD_LAUNCH_CHECK();
     }
+    ICD_TRY(beam_mm(prec, w, w.h, D, (int)R, D, w.w_cat, D, w.x3_Wcat, w.z, NZ, NZ, w.b_cat, nullptr, 0, 0.f, s, live_rows));
+    // :66-69 — one CTA per live slot serves all of its live beams (features read once per image and step)
+    // fp32-grade tensor-core tier: the attention kernel emits the 3-term bf16 split of `gated` itself (the A operand of the
+    // gate contraction below), so neither the fp32 copy nor a split pass over (rows, C) is needed
+    const bool fused_split = prec == ICD_PREC_FP32X3 && use_embg && (C % 8 == 0);
+    ICD_TRY(icd_attention_step_fwd_grouped(n_img, k, P, C, A, w.k_live, d->enc, w.att_enc, w.z, NZ, d->full_att_w,
+                                           d->full_att_b, w.z + A, NZ, alpha_s, P, fused_split ? nullptr : w.gated, w.slot_img,
+                                           w.n_live, row_off, s, fused_split ? w.x3_act : nullptr, w.ring_ticket + step,
+                                           icd_x3_three_planes(C) ? 3 : 6));
+    if (use_embg) {
+        beam_gates_init_kernel<<<(unsigned)R, 128, 0, s>>>(w.embg, w.tok64, 4 * D, w.z + A + C, NZ, w.gates_pre, w.n_live);
+        ICD_LAUNCH_CHECK();
+    } else
+        ICD_TRY(beam_mm(prec, w, w.emb_x, E, (int)R, E, d->w_ih, E + C, w.x3_WihE, w.gates_pre, 4 * D, 4 * D,
+                        d->b_ih, w.z + A + C, NZ, 0.f, s, live_rows));
+    ICD_TRY(beam_mm(prec, w, w.gated, C, (int)R, C, d->w_ih + E, E + C, w.x3_WihC, w.gates_pre, 4 * D, 4 * D,
+                    nullptr, nullptr, 0, 1.f, s, live_rows, fused_split));               // :70-71
+    ICD_TRY(icd_lstm_pointwise_fwd((int)R, D, w.gates_pre, w.c, nullptr, w.c_tmp, w.h_tmp, nullptr, 0, nullptr, 1.f, s,
+                                   nullptr, nullptr, live_rows));
+    ICD_TRY(beam_mm(prec, w, w.h_tmp, D, (int)R, D, d->fc_w, D, w.x3_Wfc, w.logits, V, V, d->fc_b, nullptr, 0, 0.f, s, live_rows));   // :72
+    return 0;
+}
+
+int beam_launch_init(int n_img, int k, int D, int start_id, BeamWs& w, cudaStream_t s) {
+    const long long n = (long long)n_img * k * D;
+    beam_init_kernel<<<(unsigned)((n + 255) / 256), 256, 0, s>>>(n_img, k, D, start_id, w.h0, w.c0, w.h, w.c,
+                                                                  w.img_index, w.prev_word, w.tok64, w.score, w.k_live,
+                                                                  w.best_score, w.best_step, w.best_parent,
+                                                                  w.slot_img, w.n_live, w.row_off[0]);
+    ICD_LAUNCH_CHECK();
+    return 0;
+}
+
+int beam_launch_advance(int n_img, int k, int D, BeamWs& w, const int* row_off, int* row_off_next, cudaStream_t s) {
+    beam_compact_kernel<<<1, 1024, 0, s>>>(n_img, k, w.k_live_tmp, w.new_slot, w.n_live, row_off_next);
+    ICD_LAUNCH_CHECK();
+    beam_reorder_kernel<<<(unsigned)((long long)n_img * k), 128, 0, s>>>(k, D, w.new_slot, w.k_live_tmp, w.slot_img_tmp, w.src,
+                                                                         w.score_tmp, w.word_tmp, w.h_tmp, w.c_tmp, w.h, w.c,
+                                                                         w.score, w.prev_word, w.tok64, w.k_live, w.slot_img,
+                                                                         row_off, row_off_next, w.tag_tmp, w.tag);
+    ICD_LAUNCH_CHECK();
+    return 0;
+}
+
+extern "C" int64_t icd_beam_search_ws_bytes(const icd_beam_desc_t* d) {
+    if (!d) return -1;
+    return (int64_t)carve(d, nullptr, nullptr);
+}
+
+extern "C" int icd_beam_search(const icd_beam_desc_t* d, void* stream) {
+    ICD_CHECK_ARG(d != nullptr, "beam_search: null descriptor");
+    ICD_CHECK_ARG(d->n_img > 0 && d->k >= 1 && d->k <= KMAX, "beam_search: n_img=%d k=%d (k <= %d)", d->n_img, d->k, KMAX);
+    ICD_CHECK_ARG(d->max_steps >= 1 && d->max_steps + 1 <= ICD_MAX_STEPS, "beam_search: max_steps=%d out of range", d->max_steps);
+    ICD_CHECK_ARG(d->V >= d->k, "beam_search: vocabulary smaller than the beam");
+    ICD_CHECK_ARG(d->A % 4 == 0 && d->C % 4 == 0 && d->D % 4 == 0 && d->E % 4 == 0, "beam_search: dims must be multiples of 4");
+    ICD_CHECK_ARG(d->ws && d->ws_bytes >= icd_beam_search_ws_bytes(d), "beam_search: workspace too small");
+    cudaStream_t s = icd_stream(stream);
+    BeamWs w;
+    carve(d, &w, (char*)d->ws);
+    const int n_img = d->n_img, k = d->k, P = d->P, D = d->D, V = d->V;
+    const long long R = (long long)n_img * k;
+    ICD_CHECK_ARG(R <= 65535, "beam_search: n_img*k=%lld exceeds 65535 rows per call (chunk the images)", R);
+    const int S1 = d->max_steps + 1;
+
+    bool use_embg = false;
+    ICD_TRY(beam_att_prologue(d, w, &use_embg, s));
+    ICD_TRY(beam_launch_init(n_img, k, D, d->start_id, w, s));
     // candidate words of images that are already finished at a step stay -1 (:91 prints nothing for them)
     if (d->trace_words) ICD_CUDA(cudaMemsetAsync(d->trace_words, 0xff, sizeof(int32_t) * (size_t)S1 * R, s));
-    const int* live_rows = w.n_live + 1;
     ICD_CUDA(cudaMemsetAsync(w.ring_ticket, 0, sizeof(int) * (size_t)(S1 + 2), s));
     for (int step = 1; step <= S1; ++step) {
         float* alpha_s = w.alpha_steps + (size_t)(step - 1) * R * P;
         const int* row_off = w.row_off[(step - 1) & 1];
         int* row_off_next = w.row_off[step & 1];
-        if (!use_embg) {
-            gather_rows_kernel<<<(unsigned)R, 128, 0, s>>>(d->emb_is_f64 ? nullptr : (const float*)d->emb_w,
-                                                           d->emb_is_f64 ? (const double*)d->emb_w : nullptr,
-                                                           w.tok64, E, w.emb_x, w.n_live);       // :65
-            ICD_LAUNCH_CHECK();
-        }
-        ICD_TRY(beam_mm(prec, w, w.h, D, (int)R, D, w.w_cat, D, w.x3_Wcat, w.z, NZ, NZ, w.b_cat, nullptr, 0, 0.f, s, live_rows));
-        // :66-69 — one CTA per live slot serves all of its live beams (features read once per image and step)
-        // fp32-grade tensor-core tier: the attention kernel emits the 3-term bf16 split of `gated` itself (the A operand of the
-        // gate contraction below), so neither the fp32 copy nor a split pass over (rows, C) is needed
-        const bool fused_split = prec == ICD_PREC_FP32X3 && use_embg && (C % 8 == 0);
-        ICD_TRY(icd_attention_step_fwd_grouped(n_img, k, P, C, A, w.k_live, d->enc, w.att_enc, w.z, NZ, d->full_att_w,
-                                               d->full_att_b, w.z + A, NZ, alpha_s, P, fused_split ? nullptr : w.gated, w.slot_img,
-                                               w.n_live, row_off, s, fused_split ? w.x3_act : nullptr, w.ring_ticket + step,
-                                               icd_x3_three_planes(C) ? 3 : 6));
-        if (use_embg) {
-            beam_gates_init_kernel<<<(unsigned)R, 128, 0, s>>>(w.embg, w.tok64, 4 * D, w.z + A + C, NZ, w.gates_pre, w.n_live);
-            ICD_LAUNCH_CHECK();
-        } else
-            ICD_TRY(beam_mm(prec, w, w.emb_x, E, (int)R, E, d->w_ih, E + C, w.x3_WihE, w.gates_pre, 4 * D, 4 * D,
-                            d->b_ih, w.z + A + C, NZ, 0.f, s, live_rows));
-        ICD_TRY(beam_mm(prec, w, w.gated, C, (int)R, C, d->w_ih + E, E + C, w.x3_WihC, w.gates_pre, 4 * D, 4 * D,
-                        nullptr, nullptr, 0, 1.f, s, live_rows, fused_split));               // :70-71
-        ICD_TRY(icd_lstm_pointwise_fwd((int)R, D, w.gates_pre, w.c, nullptr, w.c_tmp, w.h_tmp, nullptr, 0, nullptr, 1.f, s,
-                                       nullptr, nullptr, live_rows));
-        ICD_TRY(beam_mm(prec, w, w.h_tmp, D, (int)R, D, d->fc_w, D, w.x3_Wfc, w.logits, V, V, d->fc_b, nullptr, 0, 0.f, s, live_rows));   // :72
+        ICD_TRY(beam_att_step(d, w, step, use_embg, row_off, alpha_s, s));
 #define ICD_TOPK(KT) beam_topk_kernel<KT><<<n_img, 256, 0, s>>>(k, V, step, d->end_id, w.logits, w.score, w.k_live, w.slot_img, w.n_live, \
                                                row_off, w.score_tmp, w.word_tmp, w.k_live_tmp, w.slot_img_tmp, w.src,                   \
                                                w.parent + (size_t)(step - 1) * R, w.word + (size_t)(step - 1) * R,                      \
@@ -840,12 +869,7 @@ extern "C" int icd_beam_search(const icd_beam_desc_t* d, void* stream) {
         }
 #undef ICD_TOPK
         ICD_LAUNCH_CHECK();
-        beam_compact_kernel<<<1, 1024, 0, s>>>(n_img, k, w.k_live_tmp, w.new_slot, w.n_live, row_off_next);
-        ICD_LAUNCH_CHECK();
-        beam_reorder_kernel<<<(unsigned)R, 128, 0, s>>>(k, D, w.new_slot, w.k_live_tmp, w.slot_img_tmp, w.src, w.score_tmp,
-                                                        w.word_tmp, w.h_tmp, w.c_tmp, w.h, w.c, w.score, w.prev_word, w.tok64,
-                                                        w.k_live, w.slot_img, row_off, row_off_next);
-        ICD_LAUNCH_CHECK();
+        ICD_TRY(beam_launch_advance(n_img, k, D, w, row_off, row_off_next, s));
     }
     beam_finalize_kernel<<<n_img, 128, 0, s>>>(k, P, S1, R, d->start_id, d->end_id, w.best_score, w.best_step,
                                                w.best_parent, w.parent, w.word, w.alpha_steps, d->out_len, d->out_seq,
@@ -884,18 +908,9 @@ extern "C" int64_t icd_baseline_beam_search_ws_bytes(const icd_base_beam_desc_t*
     return (int64_t)carve_base(d, nullptr, nullptr);
 }
 
-extern "C" int icd_baseline_beam_search(const icd_base_beam_desc_t* d, void* stream) {
-    ICD_TRY(base_beam_check(d));                          // every argument before the first CUDA call
-    cudaStream_t s = icd_stream(stream);
-    BeamWs w;
-    carve_base(d, &w, (char*)d->ws);
-    const int n_img = d->n_img, k = d->k, E = d->E, H = d->H, V = d->V, G = 4 * H, prec = d->precision;
-    const long long R = (long long)n_img * k;
-    const int S1 = d->max_steps + 1;
-    const bool x3 = prec == ICD_PREC_FP32X3;
-    const int nseg = icd_x3_three_planes(H) ? 3 : 6;     // layout of the split of h_tmp the cell kernel writes (= beam_mm's)
-
-    if (x3) {                                             // weights are constant over the whole search: split them once
+int beam_base_prologue(const icd_base_beam_desc_t* d, BeamWs& w, cudaStream_t s) {
+    const int n_img = d->n_img, E = d->E, H = d->H, V = d->V, G = 4 * H, prec = d->precision;
+    if (prec == ICD_PREC_FP32X3) {                        // weights are constant over the whole search: split them once
         ICD_TRY(icd_split3_bf16(d->w_ih, E, G, E, w.x3_WihE, icd_x3_three_planes(E) ? 2 : 1, s));
         ICD_TRY(icd_split3_bf16(d->w_hh, H, G, H, w.x3_Whh, icd_x3_three_planes(H) ? 2 : 1, s));
         ICD_TRY(icd_split3_bf16(d->lin_w, H, V, H, w.x3_Wfc, icd_x3_three_planes(H) ? 2 : 1, s));
@@ -920,25 +935,40 @@ extern "C" int icd_baseline_beam_search(const icd_base_beam_desc_t* d, void* str
                     false, d->b_hh));
     baseline_beam_cell_kernel<<<(unsigned)n_img, 128, 0, s>>>(H, nullptr, nullptr, w.z, nullptr, w.c0, w.h0, nullptr, 0, nullptr);
     ICD_LAUNCH_CHECK();
-    {
-        const long long n = R * H;
-        beam_init_kernel<<<(unsigned)((n + 255) / 256), 256, 0, s>>>(n_img, k, H, d->start_id, w.h0, w.c0, w.h, w.c,
-                                                                      w.img_index, w.prev_word, w.tok64, w.score, w.k_live,
-                                                                      w.best_score, w.best_step, w.best_parent,
-                                                                      w.slot_img, w.n_live, w.row_off[0]);
-        ICD_LAUNCH_CHECK();
-    }
-    if (d->trace_words) ICD_CUDA(cudaMemsetAsync(d->trace_words, 0xff, sizeof(int32_t) * (size_t)S1 * R, s));
+    return 0;
+}
+
+int beam_base_step(const icd_base_beam_desc_t* d, BeamWs& w, cudaStream_t s) {
+    const int H = d->H, V = d->V, G = 4 * H, prec = d->precision;
+    const long long R = (long long)d->n_img * d->k;
+    const bool x3 = prec == ICD_PREC_FP32X3;
+    const int nseg = icd_x3_three_planes(H) ? 3 : 6;     // layout of the split of h_tmp the cell kernel writes (= beam_mm's)
     const int* live_rows = w.n_live + 1;
+    ICD_TRY(beam_mm(prec, w, w.h, H, (int)R, H, d->w_hh, H, w.x3_Whh, w.z, G, G, nullptr, nullptr, 0, 0.f, s, live_rows));
+    baseline_beam_cell_kernel<<<(unsigned)R, 128, 0, s>>>(H, w.embg, w.tok64, w.z, w.c, w.c_tmp, w.h_tmp,
+                                                          x3 ? reinterpret_cast<unsigned short*>(w.x3_act) : nullptr, nseg, w.n_live);
+    ICD_LAUNCH_CHECK();
+    ICD_TRY(beam_mm(prec, w, w.h_tmp, H, (int)R, H, d->lin_w, H, w.x3_Wfc, w.logits, V, V, d->lin_b, nullptr, 0, 0.f, s, live_rows,
+                    x3));
+    return 0;
+}
+
+extern "C" int icd_baseline_beam_search(const icd_base_beam_desc_t* d, void* stream) {
+    ICD_TRY(base_beam_check(d));                          // every argument before the first CUDA call
+    cudaStream_t s = icd_stream(stream);
+    BeamWs w;
+    carve_base(d, &w, (char*)d->ws);
+    const int n_img = d->n_img, k = d->k, H = d->H, V = d->V;
+    const long long R = (long long)n_img * k;
+    const int S1 = d->max_steps + 1;
+
+    ICD_TRY(beam_base_prologue(d, w, s));
+    ICD_TRY(beam_launch_init(n_img, k, H, d->start_id, w, s));
+    if (d->trace_words) ICD_CUDA(cudaMemsetAsync(d->trace_words, 0xff, sizeof(int32_t) * (size_t)S1 * R, s));
     for (int step = 1; step <= S1; ++step) {               // steps 1 .. max_steps+1: the state machine of icd_beam_search
         const int* row_off = w.row_off[(step - 1) & 1];
         int* row_off_next = w.row_off[step & 1];
-        ICD_TRY(beam_mm(prec, w, w.h, H, (int)R, H, d->w_hh, H, w.x3_Whh, w.z, G, G, nullptr, nullptr, 0, 0.f, s, live_rows));
-        baseline_beam_cell_kernel<<<(unsigned)R, 128, 0, s>>>(H, w.embg, w.tok64, w.z, w.c, w.c_tmp, w.h_tmp,
-                                                              x3 ? reinterpret_cast<unsigned short*>(w.x3_act) : nullptr, nseg, w.n_live);
-        ICD_LAUNCH_CHECK();
-        ICD_TRY(beam_mm(prec, w, w.h_tmp, H, (int)R, H, d->lin_w, H, w.x3_Wfc, w.logits, V, V, d->lin_b, nullptr, 0, 0.f, s, live_rows,
-                        x3));
+        ICD_TRY(beam_base_step(d, w, s));
 #define ICD_BASE_TOPK(KT) beam_topk_kernel<KT><<<n_img, 256, 0, s>>>(k, V, step, d->end_id, w.logits, w.score, w.k_live, w.slot_img,     \
                                                w.n_live, row_off, w.score_tmp, w.word_tmp, w.k_live_tmp, w.slot_img_tmp, w.src,      \
                                                w.parent + (size_t)(step - 1) * R, w.word + (size_t)(step - 1) * R,                   \
@@ -955,12 +985,7 @@ extern "C" int icd_baseline_beam_search(const icd_base_beam_desc_t* d, void* str
         }
 #undef ICD_BASE_TOPK
         ICD_LAUNCH_CHECK();
-        beam_compact_kernel<<<1, 1024, 0, s>>>(n_img, k, w.k_live_tmp, w.new_slot, w.n_live, row_off_next);
-        ICD_LAUNCH_CHECK();
-        beam_reorder_kernel<<<(unsigned)R, 128, 0, s>>>(k, H, w.new_slot, w.k_live_tmp, w.slot_img_tmp, w.src, w.score_tmp,
-                                                        w.word_tmp, w.h_tmp, w.c_tmp, w.h, w.c, w.score, w.prev_word, w.tok64,
-                                                        w.k_live, w.slot_img, row_off, row_off_next);
-        ICD_LAUNCH_CHECK();
+        ICD_TRY(beam_launch_advance(n_img, k, H, w, row_off, row_off_next, s));
     }
     beam_finalize_kernel<<<n_img, 128, 0, s>>>(k, 0, S1, R, d->start_id, d->end_id, w.best_score, w.best_step, w.best_parent,
                                                w.parent, w.word, nullptr, d->out_len, d->out_seq, d->out_score, nullptr);

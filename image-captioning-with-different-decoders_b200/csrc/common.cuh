@@ -117,6 +117,18 @@ __device__ __forceinline__ float block_max(float v, float* scratch) {
 
 __device__ __forceinline__ float sigmoidf_(float x) { return 1.f / (1.f + expf(-x)); }
 
+// Philox4x32-10 counter-based generator (Salmon et al. 2011): ten rounds on the counter c under the key (k0, k1), in place.
+// Dropout's keep masks (pointwise.cu) and the caption sampler's Gumbel noise (sample.cu) draw from it.
+__device__ __forceinline__ void philox4x32_10(uint32_t (&c)[4], uint32_t k0, uint32_t k1) {
+#pragma unroll
+    for (int r = 0; r < 10; ++r) {
+        const uint32_t hi0 = __umulhi(0xD2511F53u, c[0]), lo0 = 0xD2511F53u * c[0];
+        const uint32_t hi1 = __umulhi(0xCD9E8D57u, c[2]), lo1 = 0xCD9E8D57u * c[2];
+        c[0] = hi1 ^ c[1] ^ k0; c[1] = lo1; c[2] = hi0 ^ c[3] ^ k1; c[3] = lo0;
+        k0 += 0x9E3779B9u; k1 += 0xBB67AE85u;
+    }
+}
+
 // ---- programmatic dependent launch (PDL) ----------------------------------------------------------------
 // The kernels of the per-time-step chain (contraction -> attention step -> contraction -> LSTM gate math) are short and
 // strictly dependent; launched with cudaLaunchAttributeProgrammaticStreamSerialization the next kernel's CTAs become

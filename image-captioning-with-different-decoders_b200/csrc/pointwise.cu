@@ -350,23 +350,13 @@ __global__ void __launch_bounds__(256) embed_segment_reduce_kernel(const unsigne
     }
 }
 
-// Philox4x32-10 counter-based generator (Salmon et al. 2011).
-__device__ __forceinline__ void philox_round(uint32_t (&c)[4], uint32_t k0, uint32_t k1) {
-    const uint32_t hi0 = __umulhi(0xD2511F53u, c[0]), lo0 = 0xD2511F53u * c[0];
-    const uint32_t hi1 = __umulhi(0xCD9E8D57u, c[2]), lo1 = 0xCD9E8D57u * c[2];
-    const uint32_t n0 = hi1 ^ c[1] ^ k0, n1 = lo1, n2 = hi0 ^ c[3] ^ k1, n3 = lo0;
-    c[0] = n0; c[1] = n1; c[2] = n2; c[3] = n3;
-}
-
 __global__ void dropout_mask_kernel(unsigned char* __restrict__ out, long long n, float p,
                                     unsigned long long seed, unsigned long long offset) {
     const long long q = (long long)blockIdx.x * blockDim.x + threadIdx.x;   // one thread -> 4 outputs
     if (q * 4 >= n) return;
     const unsigned long long ctr = offset + (unsigned long long)q;
     uint32_t c[4] = {(uint32_t)ctr, (uint32_t)(ctr >> 32), 0u, 0u};
-    uint32_t k0 = (uint32_t)seed, k1 = (uint32_t)(seed >> 32);
-#pragma unroll
-    for (int r = 0; r < 10; ++r) { philox_round(c, k0, k1); k0 += 0x9E3779B9u; k1 += 0xBB67AE85u; }
+    philox4x32_10(c, (uint32_t)seed, (uint32_t)(seed >> 32));          // common.cuh
 #pragma unroll
     for (int j = 0; j < 4; ++j) {
         const long long i = q * 4 + j;

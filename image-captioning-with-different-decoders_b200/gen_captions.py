@@ -11,6 +11,9 @@ baseline's step.  The image feature is LSTM step 0 from the zero state and its l
 trains ``outputs[:, 0]`` against ``captions[:, 0] = <start>`` (models/baseline.py:93-109), so position 0 of every
 caption is ``<start>`` and the first scored prediction is conditioned on ``emb(<start>)``.  ``beam_size = 1`` is
 greedy decoding.
+
+``sample_captions`` draws captions at random from either decoder instead (seeded temperature / top-k sampling,
+``icd_sample_captions`` / ``icd_baseline_sample_captions``), with the log-probability of every sampled token.
 """
 import ctypes
 
@@ -139,6 +142,105 @@ def baseline_beam_search_batched(decoder, img_features, beam_size, start_id, end
             traces.append(trace)
     if want_trace:
         out["trace"] = torch.cat(traces, dim=1)
+    return out
+
+
+def sample_captions(decoder, features, n_samples, start_id, end_id, temperature=1.0, top_k=0, seed=None, max_steps=50,
+                    want_logp=False, chunk=None, precision="fp32x3", sample_base=0):
+    """Draw ``n_samples`` captions per image from an ``AttentionDecoder`` (features as for ``beam_search_batched``) or a
+    ``BaselineDecoder`` (img_features as for ``baseline_beam_search_batched``) -> dict with
+         seq    (n_img, n_samples, max_steps+2) int32, seq[..., 0] = <start>, 0 beyond len
+         len    (n_img, n_samples) int32  length incl. <start> and <end>; max_steps+2 for a truncated sample
+         ended  (n_img, n_samples) uint8  1 = the sample drew <end>, 0 = truncated after step max_steps+1
+         score  (n_img, n_samples) float32 sum of the log-probabilities of the sampled tokens (steps 1 .. len-1)
+         logp   (n_img, n_samples, max_steps+1) float32 each step's term, 0 beyond len-1          [want_logp]
+         seed   the seed used
+    Every step draws from softmax(logits / temperature) restricted to the ``top_k`` largest logits (0: all) by Gumbel-max
+    with counter-based noise keyed by (seed, image index, sample index, step, token); ``temperature = 0`` is greedy.  The
+    log-probabilities are those of the model at temperature 1 over the whole vocabulary.  Sample j of an image is the same
+    whatever ``chunk`` is, whichever images share the call and however many samples are drawn; ``sample_base`` is the
+    global index of the first sample (more samples of the same images later: the next indices).  ``seed=None`` draws one
+    from torch's default CPU generator (``torch.manual_seed`` makes runs reproducible).  ``precision`` is "fp32x3" or "fp32";
+    never "bf16"."""
+    if precision not in ("fp32", "fp32x3"):
+        raise ValueError("caption sampling runs in fp32-grade arithmetic only: precision must be 'fp32' or 'fp32x3'")
+    if not features.is_cuda:
+        raise _lib.IcdError("sample_captions needs CUDA tensors; there is no CPU fallback")
+    n = int(n_samples)
+    if n < 1:
+        raise ValueError("n_samples must be >= 1")
+    if seed is None:
+        seed = int(torch.randint(0, 2 ** 63 - 1, (1,), dtype=torch.int64).item())
+    seed = int(seed) & (2 ** 64 - 1)
+    base = isinstance(decoder, BaselineDecoder)
+    n_img = features.shape[0]
+    dev = features.device
+    if base:
+        x = features.contiguous().float()
+        lstm, lin = decoder.lstm, decoder.linear
+        ws = [t.detach().contiguous() for t in (lstm.weight_ih_l0, lstm.weight_hh_l0, lstm.bias_ih_l0, lstm.bias_hh_l0,
+                                                 lin.weight, lin.bias)]
+        emb_w = decoder.embedding.weight.detach().contiguous()
+        E = x.shape[1]
+        H, V = ws[1].shape[1], ws[4].shape[0]
+        assert emb_w.shape[1] == E, "img_features must have the embedding width %d" % emb_w.shape[1]
+        dims = dict(E=E, H=H, V=V)
+        weights = dict(emb_w=emb_w, w_ih=ws[0], w_hh=ws[1], b_ih=ws[2], b_hh=ws[3], lin_w=ws[4], lin_b=ws[5])
+        Desc, size_fn, run_fn, name = (_lib.BaseSampleDesc, "icd_baseline_sample_captions_ws_bytes",
+                                       "icd_baseline_sample_captions", "icd_baseline_sample_captions")
+    else:
+        C = features.shape[-1]
+        x = features.reshape(n_img, -1, C).contiguous().float()
+        a = decoder.attention
+        A, D, E, V = a.enc_att.weight.shape[0], decoder.decode_step.weight_hh.shape[1], \
+            decoder.embedding.weight.shape[1], decoder.fc.weight.shape[0]
+        emb_w = decoder.embedding.weight
+        dims = dict(P=x.shape[1], C=C, A=A, D=D, E=E, V=V)
+        weights = dict(enc_att_w=a.enc_att.weight, enc_att_b=a.enc_att.bias, dec_att_w=a.dec_att.weight,
+                       dec_att_b=a.dec_att.bias, full_att_w=a.full_att.weight, full_att_b=a.full_att.bias,
+                       w_ih=decoder.decode_step.weight_ih, w_hh=decoder.decode_step.weight_hh,
+                       b_ih=decoder.decode_step.bias_ih, b_hh=decoder.decode_step.bias_hh,
+                       h_lin_w=decoder.h_lin.weight, h_lin_b=decoder.h_lin.bias, c_lin_w=decoder.c_lin.weight,
+                       c_lin_b=decoder.c_lin.bias, f_beta_w=decoder.f_beta.weight, f_beta_b=decoder.f_beta.bias,
+                       fc_w=decoder.fc.weight, fc_b=decoder.fc.bias, emb_w=emb_w)
+        Desc, size_fn, run_fn, name = _lib.SampleDesc, "icd_sample_captions_ws_bytes", "icd_sample_captions", \
+            "icd_sample_captions"
+    S1 = max_steps + 1
+    groups = []
+    ws_cache = None
+    for j0 in range(0, n, 8):                             # samples in groups of at most 8, keyed by their global index
+        m = min(8, n - j0)
+        step_imgs = max(1, min(n_img, 65535 // m)) if chunk is None else int(chunk)
+        g = dict(seq=torch.empty(n_img, m, S1 + 1, device=dev, dtype=torch.int32),
+                 len=torch.empty(n_img, m, device=dev, dtype=torch.int32),
+                 ended=torch.empty(n_img, m, device=dev, dtype=torch.uint8),
+                 score=torch.empty(n_img, m, device=dev, dtype=torch.float32))
+        if want_logp:
+            g["logp"] = torch.empty(n_img, m, S1, device=dev, dtype=torch.float32)
+        for i0 in range(0, n_img, step_imgs):
+            ni = min(step_imgs, n_img - i0)
+            d = Desc()
+            fill(d, n_img=ni, m=m, max_steps=max_steps, precision=ops.precision_id(precision),
+                 emb_is_f64=int(emb_w.dtype == torch.float64), start_id=start_id, end_id=end_id, top_k=int(top_k),
+                 img_base=i0, sample_base=int(sample_base) + j0, temperature=float(temperature), seed=seed,
+                 out_seq=g["seq"][i0:i0 + ni], out_len=g["len"][i0:i0 + ni], out_ended=g["ended"][i0:i0 + ni],
+                 out_score=g["score"][i0:i0 + ni], out_logp=(g["logp"][i0:i0 + ni] if want_logp else None), **dims,
+                 **weights)
+            if base:
+                fill(d, img_features=x[i0:i0 + ni])
+            else:
+                fill(d, enc=x[i0:i0 + ni])
+            need = int(getattr(lib(), size_fn)(ctypes.byref(d)))
+            if need < 0:
+                check(-1, name)
+            if ws_cache is None or ws_cache.numel() < need:
+                ws_cache = torch.empty(need, device=dev, dtype=torch.uint8)
+            d.ws = ws_cache.data_ptr()
+            d.ws_bytes = need
+            check(getattr(lib(), run_fn)(ctypes.byref(d), stream_ptr()), name)
+        groups.append(g)
+    out = {key: torch.cat([g[key] for g in groups], dim=1) for key in groups[0]}
+    out["seed"] = seed
     return out
 
 

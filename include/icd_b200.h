@@ -8,6 +8,7 @@
  *   models/attention.py:218-284 AttentionDecoder.forward (+ its autograd backward)
  *   models/baseline.py:81-111   BaselineDecoder.forward  (+ its autograd backward)
  *   gen_captions.py:16-131      attention_caption_image_beam_search (+ the same search over BaselineDecoder steps)
+ *                               and seeded caption sampling (temperature, top-k) over both decoders' steps
  *   train_utils.py:2-12 + models/attention.py:417-430   clamp(+-grad_clip) + Adam step
  * Each entry point below names the reference lines it replaces.  A reference maintainer binds
  * them with ctypes (see INTEGRATION.md); no torch types cross this boundary.
@@ -36,7 +37,7 @@
 extern "C" {
 #endif
 
-#define ICD_B200_ABI_VERSION 17
+#define ICD_B200_ABI_VERSION 18
 #define ICD_MAX_STEPS 256
 
 ICD_API int icd_version(void);                       /* ICD_B200_ABI_VERSION the library was built with */
@@ -45,6 +46,8 @@ ICD_API int icd_sizeof_att_desc(void);               /* sizeof(icd_att_desc_t)  
 ICD_API int icd_sizeof_base_desc(void);
 ICD_API int icd_sizeof_beam_desc(void);
 ICD_API int icd_sizeof_base_beam_desc(void);
+ICD_API int icd_sizeof_sample_desc(void);
+ICD_API int icd_sizeof_base_sample_desc(void);
 ICD_API int icd_has_tensor_core_gemm(void);          /* 1 if the tcgen05/TMA GEMM path was compiled in     */
 /* Tile pairing of the tensor-core contraction (also env ICD_GEMM_PAIR): 0 single-CTA tiles, 1 CTA pairs sharing the B tile
  * by TMA multicast, 2 CTA pairs on one 256-row tile with tcgen05.mma.cta_group::2; any other value restores the built-in
@@ -451,6 +454,82 @@ typedef struct {
 
 ICD_API int64_t icd_baseline_beam_search_ws_bytes(const icd_base_beam_desc_t* d);   /* -1: shape refused (see the error string) */
 ICD_API int icd_baseline_beam_search(const icd_base_beam_desc_t* d, void* stream);
+
+/* ------------------------------------------------------------------------------------------------
+ * Seeded, batched caption sampling (temperature, top-k) for the attention decoder (icd_sample_captions) and the
+ * BaselineDecoder (icd_baseline_sample_captions).  n_img images x m samples, fully device-side (no per-step host sync).
+ * Sample j of image i starts from the decoder's start state exactly as the beam searches above do, and runs steps
+ * s = 1 .. max_steps+1; step 1 runs one row per image and draws all m tokens from it.  At each step, with the fp32-grade
+ * logits l (V):
+ *   lp  = log_softmax(l) at temperature 1 over the full vocabulary (the quantity the beam score sums);
+ *   candidates: every token when top_k == 0 (or top_k == V), else the top_k largest l (ties: the lower token id first);
+ *   temperature == 0: the token is argmax l (lowest id on a tie);
+ *   else Gumbel-max: the candidate with the largest key_v = l_v / temperature + g_v (IEEE fp32 division; lower id on a tie),
+ *     g_v = -log(-log(u_v)), u_v = ((bits >> 8) + 0.5) * 2^-24 in (0, 1), bits = word v % 4 of
+ *     Philox4x32-10(counter = (v / 4, s, img_base + i, sample_base + j), key = (seed lo, seed hi)).  In fp32, -log(u) is
+ *     logf of the exact u below 1/2 and -log1pf(-(1 - u)) (exact 1 - u) above, so it never rounds to 0.
+ *   The noise depends on (seed, image, sample, step, token) only: not on chunking, compaction or which images share a call.
+ * A sample that draws end_id ends: len = its length incl. <start> and <end>, ended = 1.  One that has not ended after step
+ * max_steps+1 keeps its truncated caption: len = max_steps+2, ended = 0.  score = sum of lp[token] over steps 1 .. len-1,
+ * fp32 in step order; logp[i, j, s-1] holds each term.  seq beyond len and logp beyond len-1 are 0; every entry is written.
+ * m in 1..8, n_img*m <= 65535, temperature finite and >= 0, top_k in 0..V, precision ICD_PREC_FP32 or ICD_PREC_FP32X3.
+ * Every argument is validated before the first CUDA call; the size queries return -1 for a refused shape.  The workspace
+ * holds one step of state (no per-step history): it does not grow with max_steps.
+ * ---------------------------------------------------------------------------------------------- */
+typedef struct {
+    int32_t n_img, m, max_steps;  /* m samples per image; steps 1 .. max_steps+1 */
+    int32_t P, C, A, D, E, V;
+    int32_t precision, emb_is_f64;
+    int32_t start_id, end_id;
+    int32_t top_k;                /* 0 = the whole vocabulary */
+    int32_t img_base, sample_base;   /* global index of image 0 and of sample 0 of this call (noise counters) */
+    float temperature;            /* 0 = greedy */
+    uint64_t seed;
+    /* inputs and weights, as in icd_beam_desc_t */
+    const float* enc;             /* (n_img,P,C) */
+    const float *enc_att_w, *enc_att_b, *dec_att_w, *dec_att_b, *full_att_w, *full_att_b;
+    const float *w_ih, *w_hh, *b_ih, *b_hh;
+    const float *h_lin_w, *h_lin_b, *c_lin_w, *c_lin_b;
+    const float *f_beta_w, *f_beta_b, *fc_w, *fc_b;
+    const void* emb_w;
+    /* results (device) */
+    int32_t* out_seq;             /* (n_img, m, max_steps+2), [.., 0] = <start> */
+    int32_t* out_len;             /* (n_img, m) */
+    uint8_t* out_ended;           /* (n_img, m) 1 = drew <end> */
+    float* out_score;             /* (n_img, m) */
+    float* out_logp;              /* (n_img, m, max_steps+1); may be NULL */
+    /* workspace (device) */
+    void* ws; int64_t ws_bytes;   /* >= icd_sample_captions_ws_bytes(desc) */
+} icd_sample_desc_t;
+
+ICD_API int64_t icd_sample_captions_ws_bytes(const icd_sample_desc_t* d);     /* -1: shape refused (see the error string) */
+ICD_API int icd_sample_captions(const icd_sample_desc_t* d, void* stream);
+
+typedef struct {
+    int32_t n_img, m, max_steps;
+    int32_t E, H, V;
+    int32_t precision, emb_is_f64;
+    int32_t start_id, end_id;
+    int32_t top_k;
+    int32_t img_base, sample_base;
+    float temperature;
+    uint64_t seed;
+    /* inputs and weights, as in icd_base_beam_desc_t */
+    const float* img_features;    /* (n_img,E) fp32 */
+    const void* emb_w;            /* (V,E) fp32 or fp64 */
+    const float *w_ih, *w_hh, *b_ih, *b_hh;
+    const float *lin_w, *lin_b;
+    /* results (device), as in icd_sample_desc_t */
+    int32_t* out_seq;
+    int32_t* out_len;
+    uint8_t* out_ended;
+    float* out_score;
+    float* out_logp;
+    void* ws; int64_t ws_bytes;   /* >= icd_baseline_sample_captions_ws_bytes(desc) */
+} icd_base_sample_desc_t;
+
+ICD_API int64_t icd_baseline_sample_captions_ws_bytes(const icd_base_sample_desc_t* d);
+ICD_API int icd_baseline_sample_captions(const icd_base_sample_desc_t* d, void* stream);
 
 /* ------------------------------------------------------------------------------------------------
  * Optimiser glue: element-wise gradient clamp to +-grad_clip (train_utils.py:2-12) fused with the
