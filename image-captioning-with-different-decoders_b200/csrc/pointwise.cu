@@ -469,10 +469,13 @@ __global__ void __launch_bounds__(256, 8) cross_entropy_fwd_kernel(int V, const 
 // while its log-sum-exp is formed (exactly as cross_entropy_fwd_kernel does), then the bf16 gradient
 // (exp(x - lse) - onehot) * inv_count is written from the parked copy — every logit is read from HBM once instead of twice.
 // The upstream gradient of the loss is applied afterwards (scale_bf16_by_device_scalar_kernel: a no-op when it is 1).
+// WEIGHTED: the gradient of row r is also scaled by weights[r] (scale = inv_count * w_r; row_loss stays unweighted).
+template <bool WEIGHTED>
 __global__ void __launch_bounds__(256, 5) cross_entropy_fwd_grad16_kernel(int V, const float* __restrict__ logits,
                                                                        const long long* __restrict__ targets, float inv_count,
                                                                        float* __restrict__ row_loss, float* __restrict__ lse_out,
-                                                                       __nv_bfloat16* __restrict__ d16, long long ld16) {
+                                                                       __nv_bfloat16* __restrict__ d16, long long ld16,
+                                                                       const float* __restrict__ weights) {
     extern __shared__ __align__(16) float s_x[];     // V floats (+ reduction scratch behind them)
     float* s_m = s_x + ((V + 3) & ~3) + 4;           // behind the row and its alignment pad (see sx below)
     float* s_s = s_m + 8;
@@ -511,6 +514,8 @@ __global__ void __launch_bounds__(256, 5) cross_entropy_fwd_grad16_kernel(int V,
     // alignment phase allows (pad even: every row of an even-V matrix)
     const int V8 = V >> 3, itgt = (int)tgt;
     const bool pair_ok = (pad & 1) == 0;
+    float scale = inv_count;
+    if (WEIGHTED) scale *= weights[r];
     for (int q = threadIdx.x; q < (int)(ld16 >> 3); q += 256) {
         float xv[8];
         const int v0 = 8 * q;
@@ -523,7 +528,7 @@ __global__ void __launch_bounds__(256, 5) cross_entropy_fwd_grad16_kernel(int V,
         }
         float g[8];
 #pragma unroll
-        for (int h = 0; h < 8; ++h) g[h] = ce_grad(xv[h], v0 + h == itgt, lse, inv_count);
+        for (int h = 0; h < 8; ++h) g[h] = ce_grad(xv[h], v0 + h == itgt, lse, scale);
         if (q >= V8) {
 #pragma unroll
             for (int h = 0; h < 8; ++h) if (v0 + h >= V) g[h] = 0.f;                    // pad columns of the bf16 row
@@ -553,12 +558,16 @@ __global__ void __launch_bounds__(256) scale_bf16_by_device_scalar_kernel(__nv_b
     }
 }
 
+// WEIGHTED: the gradient of row r is also scaled by weights[r] (scale = (inv_count * upstream) * w_r, so w = 1 gives the
+// unweighted bits); a row of weight 0 is still written, as zeros.
+template <bool WEIGHTED>
 __global__ void __launch_bounds__(256) cross_entropy_bwd_kernel(int V, const float* __restrict__ logits,
                                                                 const long long* __restrict__ targets,
                                                                 const float* __restrict__ lse_in,
                                                                 const float* __restrict__ upstream, float inv_count,
                                                                 float* __restrict__ d_logits,
-                                                                __nv_bfloat16* __restrict__ d16, long long ld16) {
+                                                                __nv_bfloat16* __restrict__ d16, long long ld16,
+                                                                const float* __restrict__ weights) {
     const long long r = blockIdx.x;
     const float* x = logits + r * V;
     const long long tgt = targets[r];
@@ -575,7 +584,8 @@ __global__ void __launch_bounds__(256) cross_entropy_bwd_kernel(int V, const flo
         return;
     }
     const float lse = lse_in[r];
-    const float scale = inv_count * (upstream ? upstream[0] : 1.f);
+    float scale = inv_count * (upstream ? upstream[0] : 1.f);
+    if (WEIGHTED) scale *= weights[r];
     // scalar head up to the row's first 16-byte boundary, 128-bit body with four loads in flight per thread, scalar tail
     // (the fp32 gradient rows share the alignment of the logit rows when both buffers are 16-byte aligned)
     const int itgt = (int)tgt;
@@ -789,8 +799,11 @@ extern "C" int icd_cross_entropy_fwd(int64_t R, int V, const float* logits, cons
     return 0;
 }
 
-extern "C" int icd_cross_entropy_fwd_grad16(int64_t R, int V, const float* logits, const int64_t* targets, float inv_count,
-                                            float* row_loss, float* lse, void* d_logits16, int64_t ld16, void* stream) {
+template <bool WEIGHTED>
+static int cross_entropy_fwd_grad16(int64_t R, int V, const float* logits, const int64_t* targets, float inv_count,
+                                    const float* weights, float* row_loss, float* lse, void* d_logits16, int64_t ld16,
+                                    void* stream) {
+    ICD_CHECK_ARG(!WEIGHTED || weights, "weighted_cross_entropy_fwd_grad16: weights is null");
     if (R <= 0) return 0;
     ICD_CHECK_ARG(row_loss && lse && d_logits16, "cross_entropy_fwd_grad16: null output");
     ICD_CHECK_ARG(ld16 % 8 == 0 && ld16 >= V && (reinterpret_cast<uintptr_t>(d_logits16) & 15) == 0,
@@ -799,13 +812,24 @@ extern "C" int icd_cross_entropy_fwd_grad16(int64_t R, int V, const float* logit
     ICD_CHECK_ARG(smem <= 200 * 1024, "cross_entropy_fwd_grad16: V=%d does not fit in shared memory (use the two-kernel path)", V);
     static size_t configured = 48 * 1024;
     if (smem > configured) {
-        ICD_CUDA(cudaFuncSetAttribute(cross_entropy_fwd_grad16_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+        ICD_CUDA(cudaFuncSetAttribute(cross_entropy_fwd_grad16_kernel<WEIGHTED>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
         configured = smem;
     }
-    cross_entropy_fwd_grad16_kernel<<<(unsigned)R, 256, smem, icd_stream(stream)>>>(V, logits, (const long long*)targets, inv_count,
-                                                                                    row_loss, lse, (__nv_bfloat16*)d_logits16, ld16);
+    cross_entropy_fwd_grad16_kernel<WEIGHTED><<<(unsigned)R, 256, smem, icd_stream(stream)>>>(
+        V, logits, (const long long*)targets, inv_count, row_loss, lse, (__nv_bfloat16*)d_logits16, ld16, weights);
     ICD_LAUNCH_CHECK();
     return 0;
+}
+
+extern "C" int icd_cross_entropy_fwd_grad16(int64_t R, int V, const float* logits, const int64_t* targets, float inv_count,
+                                            float* row_loss, float* lse, void* d_logits16, int64_t ld16, void* stream) {
+    return cross_entropy_fwd_grad16<false>(R, V, logits, targets, inv_count, nullptr, row_loss, lse, d_logits16, ld16, stream);
+}
+
+extern "C" int icd_weighted_cross_entropy_fwd_grad16(int64_t R, int V, const float* logits, const int64_t* targets,
+                                                     float inv_count, const float* weights, float* row_loss, float* lse,
+                                                     void* d_logits16, int64_t ld16, void* stream) {
+    return cross_entropy_fwd_grad16<true>(R, V, logits, targets, inv_count, weights, row_loss, lse, d_logits16, ld16, stream);
 }
 
 extern "C" int icd_scale_bf16_by_device_scalar(void* x16, int64_t n, const float* scale, void* stream) {
@@ -818,15 +842,29 @@ extern "C" int icd_scale_bf16_by_device_scalar(void* x16, int64_t n, const float
     return 0;
 }
 
+template <bool WEIGHTED>
+static int cross_entropy_bwd(int64_t R, int V, const float* logits, const int64_t* targets, const float* lse,
+                             const float* upstream, float inv_count, const float* weights, float* d_logits, void* d_logits16,
+                             int64_t ld16, void* stream) {
+    ICD_CHECK_ARG(!WEIGHTED || weights, "weighted_cross_entropy_bwd: weights is null");
+    if (R <= 0) return 0;
+    ICD_CHECK_ARG(!d_logits16 || (ld16 % 8 == 0 && ld16 >= V), "cross_entropy_bwd: ld16=%lld must be a multiple of 8 and >= V", (long long)ld16);
+    cross_entropy_bwd_kernel<WEIGHTED><<<(unsigned)R, 256, 0, icd_stream(stream)>>>(
+        V, logits, (const long long*)targets, lse, upstream, inv_count, d_logits, (__nv_bfloat16*)d_logits16, ld16, weights);
+    ICD_LAUNCH_CHECK();
+    return 0;
+}
+
 extern "C" int icd_cross_entropy_bwd(int64_t R, int V, const float* logits, const int64_t* targets, const float* lse,
                                      const float* upstream, float inv_count, float* d_logits, void* d_logits16,
                                      int64_t ld16, void* stream) {
-    if (R <= 0) return 0;
-    ICD_CHECK_ARG(!d_logits16 || (ld16 % 8 == 0 && ld16 >= V), "cross_entropy_bwd: ld16=%lld must be a multiple of 8 and >= V", (long long)ld16);
-    cross_entropy_bwd_kernel<<<(unsigned)R, 256, 0, icd_stream(stream)>>>(V, logits, (const long long*)targets, lse, upstream,
-                                                                          inv_count, d_logits, (__nv_bfloat16*)d_logits16, ld16);
-    ICD_LAUNCH_CHECK();
-    return 0;
+    return cross_entropy_bwd<false>(R, V, logits, targets, lse, upstream, inv_count, nullptr, d_logits, d_logits16, ld16, stream);
+}
+
+extern "C" int icd_weighted_cross_entropy_bwd(int64_t R, int V, const float* logits, const int64_t* targets, const float* lse,
+                                              const float* upstream, float inv_count, const float* weights, float* d_logits,
+                                              void* d_logits16, int64_t ld16, void* stream) {
+    return cross_entropy_bwd<true>(R, V, logits, targets, lse, upstream, inv_count, weights, d_logits, d_logits16, ld16, stream);
 }
 
 // ---- doubly stochastic attention regulariser (models/attention.py:413-414) -------------------------------------------

@@ -61,8 +61,10 @@ _FUSED_CE_MAX_V = 49000          # rows up to this many classes fit the one-pass
 
 
 class _FusedCE(torch.autograd.Function):
+    """sum_r weights[r] * CE_r / n_valid over the rows with target >= 0; ``weights`` None is the plain mean (every weight 1)."""
+
     @staticmethod
-    def forward(ctx, logits2d, targets, n_valid, want_bf16, bf16_only=False, box=None):
+    def forward(ctx, logits2d, targets, n_valid, want_bf16, bf16_only=False, box=None, weights=None):
         ctx.n_valid, ctx.want_bf16 = n_valid, bool(want_bf16 and box is not None)
         ctx.bf16_only = bool(bf16_only and ctx.want_bf16)
         ctx.box = box
@@ -70,28 +72,32 @@ class _FusedCE(torch.autograd.Function):
         if ctx.bf16_only and ctx.needs_input_grad[0] and logits2d.shape[1] <= _FUSED_CE_MAX_V:
             # training fast path: the only gradient anyone will ask for is the bf16 one, so it is formed in the SAME pass over
             # the logits as the loss (each row parked in shared memory); the backward only applies the upstream scalar
-            row_loss, lse, ctx.d16 = ops.cross_entropy_fwd_grad16(logits2d, targets, 1.0 / n_valid)
+            row_loss, lse, ctx.d16 = ops.cross_entropy_fwd_grad16(logits2d, targets, 1.0 / n_valid, weights=weights)
         else:
             row_loss, lse = ops.cross_entropy_fwd(logits2d, targets)
-        ctx.save_for_backward(logits2d, targets, lse)
+        ctx.save_for_backward(logits2d, targets, lse, weights)
         if ctx.bf16_only:
             box.hollow_expected = True
-        return row_loss.sum() / n_valid
+        if weights is None:
+            return row_loss.sum() / n_valid
+        out = (row_loss * weights).sum() / n_valid
+        out.row_loss = row_loss                      # per-row unweighted cross-entropy (weighted_token_loss documents it)
+        return out
 
     @staticmethod
     def backward(ctx, g):
-        logits2d, targets, lse = ctx.saved_tensors
+        logits2d, targets, lse, weights = ctx.saved_tensors
         g = g.reshape(1).float().contiguous()
         if ctx.d16 is not None:
             d16, ctx.d16 = ops.scale_bf16_by_device_scalar(ctx.d16, g), None
             d_logits = torch.empty_like(logits2d)            # hollow: never written, never read (GradBox refuses anything else)
             ctx.box.put(d16, d_logits, True)
-            return d_logits, None, None, None, None, None
+            return d_logits, None, None, None, None, None, None
         d_logits, d16 = ops.cross_entropy_bwd(logits2d, targets, lse, 1.0 / ctx.n_valid, upstream=g,
-                                              want_bf16=ctx.want_bf16, want_fp32=not ctx.bf16_only)
+                                              want_bf16=ctx.want_bf16, want_fp32=not ctx.bf16_only, weights=weights)
         if d16 is not None:
             ctx.box.put(d16, d_logits, ctx.bf16_only)
-        return d_logits, None, None, None, None, None
+        return d_logits, None, None, None, None, None, None
 
 
 class _AlphaReg(torch.autograd.Function):
@@ -161,6 +167,23 @@ def attention_caption_loss(predictions, encoded_captions, decode_lengths, alphas
         if scale is not None:
             ce = ce * scale
     return ce + alpha_regulariser(alphas, alpha_c)
+
+
+def weighted_token_loss(logits, targets, weights, count, bf16_grad_only=False):
+    """sum over the scored positions of weights * cross-entropy, divided by ``count`` — the token loss of sequence-level
+    training (scst.self_critical_loss: the weight of a token is its caption's advantage).  ``logits`` (B, T, V) from either
+    decoder's forward; ``targets`` (B, T) int64, -1 at unscored positions; ``weights`` (B, T) fp32 (no gradient flows to
+    them; any sign); ``count`` a host number.  The gradient is formed by the weighted fused kernels
+    (icd_weighted_cross_entropy_bwd / _fwd_grad16) and, from the attention decoder's bf16 tier, handed to the decoder
+    backward as bf16 like ``attention_caption_loss`` does; ``bf16_grad_only`` has the same meaning and conditions there.
+    The result carries ``.row_loss``: the (B*T,) unweighted cross-entropy of every position (0 where the target is -1),
+    i.e. -log p of each scored token, with no gradient."""
+    B, T, V = logits.shape
+    assert targets.shape == (B, T) and weights.shape == (B, T), "targets and weights must be (B, T) like the logits"
+    box = getattr(logits, "_icd_box", None)
+    want_bf16 = bool(getattr(logits, "_icd_bf16_tier", False)) and box is not None
+    w = weights.detach().to(device=logits.device, dtype=torch.float32).reshape(-1).contiguous()
+    return _FusedCE.apply(logits.reshape(B * T, V), targets.reshape(-1).contiguous(), count, want_bf16, bf16_grad_only, box, w)
 
 
 class _MaskedMeanCE(torch.autograd.Function):

@@ -212,12 +212,13 @@ def cross_entropy_fwd(logits, targets):
     return row_loss, lse
 
 
-def cross_entropy_bwd(logits, targets, lse, inv_count, upstream=None, want_bf16=False, want_fp32=True):
+def cross_entropy_bwd(logits, targets, lse, inv_count, upstream=None, want_bf16=False, want_fp32=True, weights=None):
     """-> (d_logits (R,V) fp32 = (softmax - onehot) * inv_count * upstream, d_logits16 (R, up8(V)) bf16 or None);
     ``upstream`` is a 0-dim / 1-element CUDA fp32 tensor read on the device (no host sync).
     want_fp32=False (needs want_bf16): the fp32 gradient is NOT written — the returned fp32 tensor is allocated but
-    hollow (its contents are undefined); only for callers that hand the bf16 copy on (see losses._FusedCE)."""
-    _need_cuda(logits, targets, lse)
+    hollow (its contents are undefined); only for callers that hand the bf16 copy on (see losses._FusedCE).
+    ``weights``: optional (R,) CUDA fp32 per-row factors (icd_weighted_cross_entropy_bwd): row r is also times weights[r]."""
+    _need_cuda(logits, targets, lse, weights)
     R, V = logits.shape
     assert want_fp32 or want_bf16
     d_logits = torch.empty_like(logits)
@@ -225,25 +226,41 @@ def cross_entropy_bwd(logits, targets, lse, inv_count, upstream=None, want_bf16=
     if want_bf16:
         ld16 = (V + 7) // 8 * 8
         d16 = torch.empty(R, ld16, device=logits.device, dtype=torch.bfloat16)
-    check(lib().icd_cross_entropy_bwd(ctypes.c_int64(R), V, ptr(logits), ptr(targets), ptr(lse), ptr(upstream),
-                                      ctypes.c_float(inv_count), ptr(d_logits) if want_fp32 else None, ptr(d16),
-                                      ctypes.c_int64(ld16),
-                                      stream_ptr()), "icd_cross_entropy_bwd")
+    if weights is None:
+        check(lib().icd_cross_entropy_bwd(ctypes.c_int64(R), V, ptr(logits), ptr(targets), ptr(lse), ptr(upstream),
+                                          ctypes.c_float(inv_count), ptr(d_logits) if want_fp32 else None, ptr(d16),
+                                          ctypes.c_int64(ld16),
+                                          stream_ptr()), "icd_cross_entropy_bwd")
+    else:
+        assert weights.dtype == torch.float32 and weights.is_contiguous() and weights.numel() == R
+        check(lib().icd_weighted_cross_entropy_bwd(ctypes.c_int64(R), V, ptr(logits), ptr(targets), ptr(lse), ptr(upstream),
+                                                   ctypes.c_float(inv_count), ptr(weights),
+                                                   ptr(d_logits) if want_fp32 else None, ptr(d16), ctypes.c_int64(ld16),
+                                                   stream_ptr()), "icd_weighted_cross_entropy_bwd")
     return d_logits, d16
 
 
-def cross_entropy_fwd_grad16(logits, targets, inv_count):
+def cross_entropy_fwd_grad16(logits, targets, inv_count, weights=None):
     """Forward and bf16 gradient in one pass over the logits (icd_cross_entropy_fwd_grad16)
-    -> (row_loss (R,), lse (R,), d_logits16 (R, up8(V)) bf16 = (softmax - onehot) * inv_count, NOT yet times the upstream gradient)"""
-    _need_cuda(logits, targets)
+    -> (row_loss (R,), lse (R,), d_logits16 (R, up8(V)) bf16 = (softmax - onehot) * inv_count, NOT yet times the upstream gradient)
+    ``weights``: optional (R,) CUDA fp32 per-row factors of the gradient (icd_weighted_cross_entropy_fwd_grad16); row_loss
+    stays unweighted."""
+    _need_cuda(logits, targets, weights)
     R, V = logits.shape
     ld16 = (V + 7) // 8 * 8
     row_loss = torch.empty(R, device=logits.device, dtype=torch.float32)
     lse = torch.empty(R, device=logits.device, dtype=torch.float32)
     d16 = torch.empty(R, ld16, device=logits.device, dtype=torch.bfloat16)
-    check(lib().icd_cross_entropy_fwd_grad16(ctypes.c_int64(R), V, ptr(logits), ptr(targets), ctypes.c_float(inv_count),
-                                             ptr(row_loss), ptr(lse), ptr(d16), ctypes.c_int64(ld16), stream_ptr()),
-          "icd_cross_entropy_fwd_grad16")
+    if weights is None:
+        check(lib().icd_cross_entropy_fwd_grad16(ctypes.c_int64(R), V, ptr(logits), ptr(targets), ctypes.c_float(inv_count),
+                                                 ptr(row_loss), ptr(lse), ptr(d16), ctypes.c_int64(ld16), stream_ptr()),
+              "icd_cross_entropy_fwd_grad16")
+    else:
+        assert weights.dtype == torch.float32 and weights.is_contiguous() and weights.numel() == R
+        check(lib().icd_weighted_cross_entropy_fwd_grad16(ctypes.c_int64(R), V, ptr(logits), ptr(targets),
+                                                          ctypes.c_float(inv_count), ptr(weights), ptr(row_loss), ptr(lse),
+                                                          ptr(d16), ctypes.c_int64(ld16), stream_ptr()),
+              "icd_weighted_cross_entropy_fwd_grad16")
     return row_loss, lse, d16
 
 

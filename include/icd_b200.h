@@ -562,6 +562,18 @@ ICD_API int icd_cross_entropy_bwd(int64_t R, int V, const float* logits, const i
 ICD_API int icd_cross_entropy_fwd_grad16(int64_t R, int V, const float* logits, const int64_t* targets, float inv_count,
                           float* row_loss, float* lse, void* d_logits16, int64_t ld16, void* stream);
 ICD_API int icd_scale_bf16_by_device_scalar(void* x16, int64_t n, const float* scale, void* stream);
+/* Per-row weighted gradients (sequence-level training: a reward advantage per caption token): the same kernels with the
+ * gradient of row r also multiplied by weights[r] (R fp32 values on the device, any sign, 0 allowed):
+ *   bwd      : d_logits[r,v] = (exp(logits[r,v] - lse[r]) - [v == targets[r]]) * ((inv_count * (*upstream)) * weights[r])
+ *   fwd_grad16: the bf16 gradient is (exp(x - lse) - onehot) * (inv_count * weights[r]); row_loss and lse stay unweighted.
+ * weights == 1 reproduces the unweighted results bit for bit; a row of weight 0 is written as zeros; rows with targets[r] < 0
+ * are zero as before.  Every argument (null weights, ld16, V of the one-pass kernel) is checked before any CUDA call. */
+ICD_API int icd_weighted_cross_entropy_bwd(int64_t R, int V, const float* logits, const int64_t* targets, const float* lse,
+                          const float* upstream, float inv_count, const float* weights, float* d_logits, void* d_logits16,
+                          int64_t ld16, void* stream);
+ICD_API int icd_weighted_cross_entropy_fwd_grad16(int64_t R, int V, const float* logits, const int64_t* targets,
+                          float inv_count, const float* weights, float* row_loss, float* lse, void* d_logits16, int64_t ld16,
+                          void* stream);
 
 /* Doubly stochastic attention regulariser (models/attention.py:413-414): reg = mean_{b,p} (alpha_c - sum_t alphas[b,t,p])^2.
  * forward : resid[b,p] = alpha_c - sum_t alphas[b,t,p] (saved for the backward); reg[0] = the mean (summed in a fixed order:
