@@ -72,6 +72,7 @@ BeamDesc = _make_struct("icd_beam_desc_t")
 BaseBeamDesc = _make_struct("icd_base_beam_desc_t")
 SampleDesc = _make_struct("icd_sample_desc_t")
 BaseSampleDesc = _make_struct("icd_base_sample_desc_t")
+AttIndex = _make_struct("icd_att_index_t")
 
 PREC_FP32 = DEFINES["ICD_PREC_FP32"]
 PREC_BF16 = DEFINES["ICD_PREC_BF16"]
@@ -105,13 +106,16 @@ def lib():
     L.icd_gemm_ws_bytes.restype = ctypes.c_int64
     L.icd_gemm_bf16_splitk_ws_floats.restype = ctypes.c_int64
     L.icd_attention_decoder_ws_bytes.restype = ctypes.c_int64
+    L.icd_attention_decoder_ws_bytes_indexed.restype = ctypes.c_int64
+    L.icd_attention_proj_bwd_ws_floats_indexed.restype = ctypes.c_int64
     L.icd_baseline_decoder_ws_bytes.restype = ctypes.c_int64
     if L.icd_version() != DEFINES["ICD_B200_ABI_VERSION"]:
         raise IcdError("libicd_b200.so ABI %d != header ABI %d — rebuild" %
                        (L.icd_version(), DEFINES["ICD_B200_ABI_VERSION"]))
     for fn, st in (("icd_sizeof_att_desc", AttDesc), ("icd_sizeof_base_desc", BaseDesc),
                    ("icd_sizeof_beam_desc", BeamDesc), ("icd_sizeof_base_beam_desc", BaseBeamDesc),
-                   ("icd_sizeof_sample_desc", SampleDesc), ("icd_sizeof_base_sample_desc", BaseSampleDesc)):
+                   ("icd_sizeof_sample_desc", SampleDesc), ("icd_sizeof_base_sample_desc", BaseSampleDesc),
+                   ("icd_sizeof_att_index", AttIndex)):
         if getattr(L, fn)() != ctypes.sizeof(st):
             raise IcdError("%s: C says %d bytes, ctypes says %d" % (fn, getattr(L, fn)(), ctypes.sizeof(st)))
     _lib = L

@@ -115,4 +115,5 @@ int icd_sizeof_beam_desc(void) { return (int)sizeof(icd_beam_desc_t); }
 int icd_sizeof_base_beam_desc(void) { return (int)sizeof(icd_base_beam_desc_t); }
 int icd_sizeof_sample_desc(void) { return (int)sizeof(icd_sample_desc_t); }
 int icd_sizeof_base_sample_desc(void) { return (int)sizeof(icd_base_sample_desc_t); }
+int icd_sizeof_att_index(void) { return (int)sizeof(icd_att_index_t); }
 }

@@ -639,6 +639,8 @@ __global__ void __launch_bounds__(RING_THREADS, (K <= 5 ? 2 : 1)) att_step_fwd_g
 // ------------------------------------------------------------------------------------------------
 // weighted pixel sum + gate.  grid = (ceil(C/256), rows), block = 256 = 4 pixel groups x 64 float4 lanes.
 // alpha == NULL  => plain mean over pixels (init_hidden_state, models/attention.py:161).
+// out_row_ptr != NULL (captions that share images): CTA row r is image r, and its result is written to the output rows
+// out_rows[out_row_ptr[r] .. out_row_ptr[r+1]) instead of row r (the pixel mean computed once per image, gathered to rows).
 // ------------------------------------------------------------------------------------------------
 constexpr int WS_LANES = 64, WS_GROUPS = 4, WS_UNROLL = 7;
 
@@ -646,7 +648,8 @@ __global__ void __launch_bounds__(256) weighted_pixel_sum_kernel(
         int P, int C, const int* __restrict__ img_index, const float* __restrict__ enc,
         const float* __restrict__ alpha, long long ld_alpha,
         const float* __restrict__ fbeta_pre, long long ld_fb,
-        float* __restrict__ awe_raw, float* __restrict__ gate, float* __restrict__ gated) {
+        float* __restrict__ awe_raw, float* __restrict__ gate, float* __restrict__ gated,
+        const int* __restrict__ out_row_ptr, const int* __restrict__ out_rows) {
     extern __shared__ __align__(16) float sm[];
     float* s_alpha = sm;                                                  // P (padded to mult. of 4)
     float4* s_part = reinterpret_cast<float4*>(sm + ((P + 3) & ~3));      // (WS_GROUPS-1) * WS_LANES float4
@@ -692,14 +695,18 @@ __global__ void __launch_bounds__(256) weighted_pixel_sum_kernel(
             acc.x += o.x; acc.y += o.y; acc.z += o.z; acc.w += o.w;
         }
         if (!alpha) { const float inv = (float)P; acc.x /= inv; acc.y /= inv; acc.z /= inv; acc.w /= inv; }
-        const long long o = (long long)r * C + c;
-        if (awe_raw) *reinterpret_cast<float4*>(awe_raw + o) = acc;
-        if (fbeta_pre) {
-            const float4 f = *reinterpret_cast<const float4*>(fbeta_pre + (long long)r * ld_fb + c);
-            const float4 g = make_float4(sigmoidf_(f.x), sigmoidf_(f.y), sigmoidf_(f.z), sigmoidf_(f.w));
-            if (gate) *reinterpret_cast<float4*>(gate + o) = g;
-            if (gated) *reinterpret_cast<float4*>(gated + o) =
-                    make_float4(g.x * acc.x, g.y * acc.y, g.z * acc.z, g.w * acc.w);
+        const int k0 = out_row_ptr ? out_row_ptr[r] : r, k1 = out_row_ptr ? out_row_ptr[r + 1] : r + 1;
+        for (int k = k0; k < k1; ++k) {
+            const int ro = out_row_ptr ? out_rows[k] : r;
+            const long long o = (long long)ro * C + c;
+            if (awe_raw) *reinterpret_cast<float4*>(awe_raw + o) = acc;
+            if (fbeta_pre) {
+                const float4 f = *reinterpret_cast<const float4*>(fbeta_pre + (long long)ro * ld_fb + c);
+                const float4 g = make_float4(sigmoidf_(f.x), sigmoidf_(f.y), sigmoidf_(f.z), sigmoidf_(f.w));
+                if (gate) *reinterpret_cast<float4*>(gate + o) = g;
+                if (gated) *reinterpret_cast<float4*>(gated + o) =
+                        make_float4(g.x * acc.x, g.y * acc.y, g.z * acc.z, g.w * acc.w);
+            }
         }
     }
 }
@@ -708,7 +715,7 @@ __global__ void __launch_bounds__(256) weighted_pixel_sum_kernel(
 // step backward.  grid = rows, block = 256.  smem: C + 3*P + A + 40 floats + 2*... see launcher.
 // ------------------------------------------------------------------------------------------------
 __global__ void __launch_bounds__(256) att_step_bwd_kernel(
-        int P, int C, int A,
+        int P, int C, int A, const int* __restrict__ img_index,
         const float* __restrict__ enc, const float* __restrict__ att_enc,
         const float* __restrict__ att_dec, long long ld_dec, const float* __restrict__ w_full,
         const float* __restrict__ alpha, long long ld_alpha,
@@ -725,6 +732,7 @@ __global__ void __launch_bounds__(256) att_step_bwd_kernel(
     float* s_red = s_de + ((P + 3) & ~3);     // 40
     float* s_part = s_red + 40;               // A   (second pixel-group partial of d_att_dec)
     const int r = blockIdx.x;
+    const int img = img_index ? img_index[r] : r;
     const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5, nwarp = blockDim.x >> 5;
 
     // (A) gate backward, elementwise over C
@@ -750,7 +758,7 @@ __global__ void __launch_bounds__(256) att_step_bwd_kernel(
 
     // (B) d_alpha[p] = <d_awe, enc[r,p,:]>   warp per pixel row, 8 x 128-bit loads in flight per lane
     {
-        const float* eb = enc + (long long)r * P * C;
+        const float* eb = enc + (long long)img * P * C;
         const int C4 = C >> 2;
         for (int p = warp; p < P; p += nwarp) {
             const float* row = eb + (long long)p * C;
@@ -798,7 +806,7 @@ __global__ void __launch_bounds__(256) att_step_bwd_kernel(
 
     // (D) d_att_dec[a] = w_full[a] * sum_p d_e[p] * [att_enc[p,a] + att_dec[a] > 0]
     {
-        const float* ab = att_enc + (long long)r * P * A;
+        const float* ab = att_enc + (long long)img * P * A;
         const int A4 = A >> 2;
         const int half = blockDim.x >> 1;                 // two pixel groups
         const int grp = threadIdx.x / half, t = threadIdx.x % half;
@@ -947,6 +955,96 @@ __global__ void __launch_bounds__(1024) att_proj_bwd_kernel_wide(int B, int T, i
     att_proj_bwd_body(B, T, P, A, row_len, att_enc, att_dec_all, ld_dec, w_full, d_e, d_att_enc, partial);
 }
 
+// Captions that share images: the same sums per IMAGE i over the (row, step) pairs of its rows,
+//   d_att_enc[i,p,a] = w_full[a] * sum_{r in rows(i)} sum_{t < len_r} d_e[r,t,p] * [att_enc[i,p,a] + att_dec[t,r,a] > 0],
+// formed directly (no per-row (B,P,A) tensor).  grid = (ceil(P/PROJ_IMG_PB), n_img), block = A/4 threads; a thread owns 4
+// channels of the CTA's 4 pixels and keeps their sums in registers while the (row, step) pairs of the image pass through shared
+// memory, PROJ_IMG_KC steps of one row at a time: rows in CSR order (ascending), then steps in order — deterministic.
+// partial[(i*gridDim.x + chunk)*(2A+4)] as above.  smem: PROJ_IMG_KC*(A + PROJ_IMG_PB) + 40 floats.
+constexpr int PROJ_IMG_PB = 4, PROJ_IMG_KC = 32;
+__global__ void __launch_bounds__(1024) att_proj_bwd_img_kernel(int B, int T, int P, int A, const int* __restrict__ row_len,
+                                        const int* __restrict__ row_ptr, const int* __restrict__ rows,
+                                        const float* __restrict__ att_enc, const float* __restrict__ att_dec_all,
+                                        long long ld_dec, const float* __restrict__ w_full,
+                                        const float* __restrict__ d_e, float* __restrict__ d_att_enc,
+                                        float* __restrict__ partial) {
+    extern __shared__ __align__(16) float sm[];
+    const int i = blockIdx.y, p0 = blockIdx.x * PROJ_IMG_PB;
+    const int np = min(PROJ_IMG_PB, P - p0);
+    float* s_dec = sm;                                   // PROJ_IMG_KC * A
+    float* s_de = sm + (size_t)PROJ_IMG_KC * A;          // PROJ_IMG_KC * PROJ_IMG_PB
+    float* s_red = s_de + PROJ_IMG_KC * PROJ_IMG_PB;     // 40
+    const int a = threadIdx.x * 4;
+    float x[4][4], acc[4][4];
+#pragma unroll
+    for (int u = 0; u < 4; ++u)
+#pragma unroll
+        for (int c = 0; c < 4; ++c) { x[u][c] = 0.f; acc[u][c] = 0.f; }
+    if (a < A) {
+#pragma unroll
+        for (int u = 0; u < 4; ++u) {
+            const float4 raw = ld_stream_f4(att_enc + ((long long)i * P + p0 + min(u, np - 1)) * A + a);
+            x[u][0] = raw.x; x[u][1] = raw.y; x[u][2] = raw.z; x[u][3] = raw.w;
+        }
+    }
+    float4 wacc = make_float4(0.f, 0.f, 0.f, 0.f);
+    float de_sum = 0.f;
+    for (int k = row_ptr[i]; k < row_ptr[i + 1]; ++k) {
+        const int b = rows[k], Tb = row_len[b];
+        for (int t0 = 0; t0 < Tb; t0 += PROJ_IMG_KC) {
+            const int nt = min(PROJ_IMG_KC, Tb - t0);
+            __syncthreads();                             // the previous round is consumed
+            for (int j = threadIdx.x; j < nt * (A >> 2); j += blockDim.x) {
+                const int t = j / (A >> 2), a4 = (j % (A >> 2)) * 4;
+                *reinterpret_cast<float4*>(s_dec + (size_t)t * A + a4) =
+                    *reinterpret_cast<const float4*>(att_dec_all + ((long long)(t0 + t) * B + b) * ld_dec + a4);
+            }
+            for (int j = threadIdx.x; j < nt * PROJ_IMG_PB; j += blockDim.x) {
+                const int t = j / PROJ_IMG_PB, pp = j % PROJ_IMG_PB;
+                const float v = (pp < np) ? d_e[((long long)b * T + t0 + t) * P + p0 + pp] : 0.f;
+                s_de[j] = v;
+                de_sum += v;
+            }
+            __syncthreads();
+            if (a < A) {
+                for (int t = 0; t < nt; ++t) {
+                    const float4 de4 = *reinterpret_cast<const float4*>(s_de + t * PROJ_IMG_PB);
+                    const float4 d = *reinterpret_cast<const float4*>(s_dec + (size_t)t * A + a);
+                    const float de[4] = {de4.x, de4.y, de4.z, de4.w};
+                    const float dd[4] = {d.x, d.y, d.z, d.w};
+                    float wl[4] = {0.f, 0.f, 0.f, 0.f};
+#pragma unroll
+                    for (int u = 0; u < 4; ++u) {
+#pragma unroll
+                        for (int c = 0; c < 4; ++c) {
+                            const float sv = x[u][c] + dd[c];
+                            acc[u][c] += (sv > 0.f) ? de[u] : 0.f;
+                            wl[c] = fmaf(de[u], fmaxf(sv, 0.f), wl[c]);
+                        }
+                    }
+                    wacc.x += wl[0]; wacc.y += wl[1]; wacc.z += wl[2]; wacc.w += wl[3];
+                }
+            }
+        }
+    }
+    float4 bacc = make_float4(0.f, 0.f, 0.f, 0.f);
+    if (a < A) {
+        const float4 w = *reinterpret_cast<const float4*>(w_full + a);
+#pragma unroll
+        for (int u = 0; u < 4; ++u) {
+            if (u >= np) break;
+            const long long o = ((long long)i * P + p0 + u) * A + a;
+            const float4 r = make_float4(acc[u][0] * w.x, acc[u][1] * w.y, acc[u][2] * w.z, acc[u][3] * w.w);
+            bacc.x += r.x; bacc.y += r.y; bacc.z += r.z; bacc.w += r.w;
+            *reinterpret_cast<float4*>(d_att_enc + o) = r;
+        }
+    }
+    float* mine = partial + ((long long)i * gridDim.x + blockIdx.x) * (2 * A + 4);
+    if (a < A) { *reinterpret_cast<float4*>(mine + a) = wacc; *reinterpret_cast<float4*>(mine + A + a) = bacc; }
+    const float tot = block_sum(de_sum, s_red);
+    if (threadIdx.x == 0) { mine[2 * A] = tot; mine[2 * A + 1] = 0.f; mine[2 * A + 2] = 0.f; mine[2 * A + 3] = 0.f; }
+}
+
 struct BtPack { int v[ICD_MAX_STEPS]; };
 __global__ void row_len_from_pack_kernel(int B, int T, const BtPack bt, int* __restrict__ row_len) {
     const int b = blockIdx.x * blockDim.x + threadIdx.x;
@@ -960,7 +1058,8 @@ __global__ void row_len_from_pack_kernel(int B, int T, const BtPack bt, int* __r
 
 int icd_weighted_pixel_sum(int rows, int P, int C, const int32_t* img_index, const float* enc,
                            const float* alpha, int64_t ld_alpha, const float* fbeta_pre, int64_t ld_fb,
-                           float* awe_raw, float* gate, float* gated, cudaStream_t s) {
+                           float* awe_raw, float* gate, float* gated, cudaStream_t s,
+                           const int32_t* out_row_ptr, const int32_t* out_rows) {
     if (rows == 0) return 0;
     ICD_CHECK_ARG(C % 4 == 0, "attention: C=%d must be a multiple of 4", C);
     ICD_CHECK_ARG(!fbeta_pre || ld_fb % 4 == 0, "attention: ld_fb must be a multiple of 4");
@@ -968,7 +1067,7 @@ int icd_weighted_pixel_sum(int rows, int P, int C, const int32_t* img_index, con
     dim3 grid((C + WS_LANES * 4 - 1) / (WS_LANES * 4), rows);
     const size_t smem = (((P + 3) & ~3) + (WS_GROUPS - 1) * WS_LANES * 4) * sizeof(float);
     weighted_pixel_sum_kernel<<<grid, 256, smem, s>>>(P, C, img_index, enc, alpha, ld_alpha, fbeta_pre, ld_fb,
-                                                      awe_raw, gate, gated);
+                                                      awe_raw, gate, gated, out_row_ptr, out_rows);
     ICD_LAUNCH_CHECK();
     return 0;
 }
@@ -1012,6 +1111,20 @@ extern "C" int icd_attention_step_bwd(int rows, int P, int C, int A,
                                       float* d_att_dec, int64_t ld_ddec,
                                       float* d_fbeta_pre, int64_t ld_dfb,
                                       float* d_e, int64_t ld_de, float* d_awe_out, void* stream) {
+    return icd_attention_step_bwd_idx(rows, P, C, A, nullptr, enc, att_enc, att_dec, ld_dec, w_full, alpha, ld_alpha, d_alpha_ext,
+                                      ld_dalpha, gate, awe_raw, d_gated, d_att_dec, ld_ddec, d_fbeta_pre, ld_dfb, d_e, ld_de,
+                                      d_awe_out, stream);
+}
+
+int icd_attention_step_bwd_idx(int rows, int P, int C, int A, const int32_t* img_index,
+                                      const float* enc, const float* att_enc,
+                                      const float* att_dec, int64_t ld_dec, const float* w_full,
+                                      const float* alpha, int64_t ld_alpha,
+                                      const float* d_alpha_ext, int64_t ld_dalpha,
+                                      const float* gate, const float* awe_raw, const float* d_gated,
+                                      float* d_att_dec, int64_t ld_ddec,
+                                      float* d_fbeta_pre, int64_t ld_dfb,
+                                      float* d_e, int64_t ld_de, float* d_awe_out, void* stream) {
     cudaStream_t s = icd_stream(stream);
     if (rows == 0) return 0;
     ICD_CHECK_ARG(A % 4 == 0 && C % 4 == 0, "attention_step_bwd: A and C must be multiples of 4");
@@ -1026,7 +1139,7 @@ extern "C" int icd_attention_step_bwd(int rows, int P, int C, int A,
         }
     }
     icd_prof_mark_begin(1, rows, s);
-    att_step_bwd_kernel<<<rows, 256, smem, s>>>(P, C, A, enc, att_enc, att_dec, ld_dec, w_full, alpha, ld_alpha,
+    att_step_bwd_kernel<<<rows, 256, smem, s>>>(P, C, A, (const int*)img_index, enc, att_enc, att_dec, ld_dec, w_full, alpha, ld_alpha,
                                                  d_alpha_ext, ld_dalpha, gate, awe_raw, d_gated,
                                                  d_att_dec, ld_ddec, d_fbeta_pre, ld_dfb, d_e, ld_de, d_awe_out);
     icd_prof_mark_end(1, s);
@@ -1039,6 +1152,46 @@ extern "C" int64_t icd_attention_proj_bwd_ws_floats(int B, int P, int A) {
     // per-CTA partials (d_w_full[A] | d_b_enc[A] | sum d_e + pad) + [B] int row lengths (4-byte words at the end)
     // + A floats for the att_dec part of d_w_full (bf16 tier, icd_attention_proj_bwd_bf16_ex)
     return (int64_t)B * chunks * (2 * A + 4) + B + 8 + 49 * (int64_t)A;      // 49 = 1 + COLDOT_CHUNKS (attention_step_bf16.cu)
+}
+
+extern "C" int64_t icd_attention_proj_bwd_ws_floats_indexed(int B, int n_img, int P, int A) {
+    // per-CTA partials of the per-image pass (its chunks are PROJ_IMG_PB = 4 pixels; the bf16 pass uses 8 and needs fewer)
+    // + [B] row lengths + the att_dec part of d_w_full, as above
+    const int64_t chunks = (P + PROJ_IMG_PB - 1) / PROJ_IMG_PB;
+    return (int64_t)n_img * chunks * (2 * A + 4) + B + 8 + 49 * (int64_t)A;
+}
+
+// the row-length vector of both per-image passes sits behind their partials (n_img * chunks rows of 2A+4 floats)
+int icd_attention_proj_bwd_indexed(int B, int n_img, int T, int P, int A, const int32_t* bt_host, const int32_t* row_ptr,
+                                   const int32_t* rows, const float* att_enc, const float* att_dec_all, int64_t ld_dec,
+                                   const float* w_full, const float* d_e, float* d_att_enc, float* d_w_full, float* d_b_full,
+                                   float* d_b_enc, float* partial, cudaStream_t s) {
+    ICD_CHECK_ARG(T > 0 && T <= ICD_MAX_STEPS, "attention_proj_bwd: T=%d out of range", T);
+    ICD_CHECK_ARG(A % 4 == 0 && A / 4 <= 1024, "attention_proj_bwd: A=%d unsupported", A);
+    ICD_CHECK_ARG(ld_dec % 4 == 0, "attention_proj_bwd: ld_dec must be a multiple of 4");
+    ICD_CHECK_ARG(n_img > 0 && n_img <= 65535, "attention_proj_bwd: n_img=%d out of range", n_img);
+    const int chunks = (P + PROJ_IMG_PB - 1) / PROJ_IMG_PB;
+    const int W = 2 * A + 4;
+    int* row_len = reinterpret_cast<int*>(partial + (int64_t)n_img * chunks * W);
+    BtPack pack;
+    for (int t = 0; t < ICD_MAX_STEPS; ++t) pack.v[t] = t < T ? bt_host[t] : 0;
+    row_len_from_pack_kernel<<<(B + 127) / 128, 128, 0, s>>>(B, T, pack, row_len);
+    ICD_LAUNCH_CHECK();
+    const size_t smem = ((size_t)PROJ_IMG_KC * (A + PROJ_IMG_PB) + 40) * sizeof(float);
+    ICD_CHECK_ARG(smem <= 220 * 1024, "attention_proj_bwd: A too large for shared memory");
+    static size_t configured = 48 * 1024;
+    if (smem > configured) {
+        ICD_CUDA(cudaFuncSetAttribute(att_proj_bwd_img_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+        configured = smem;
+    }
+    const int threads = ((A / 4 + 31) / 32) * 32;
+    att_proj_bwd_img_kernel<<<dim3(chunks, n_img), threads, smem, s>>>(B, T, P, A, row_len, row_ptr, rows, att_enc, att_dec_all,
+                                                                        ld_dec, w_full, d_e, d_att_enc, partial);
+    ICD_LAUNCH_CHECK();
+    ICD_TRY(icd_colsum(partial, W, (int64_t)n_img * chunks, A, nullptr, d_w_full, s));
+    if (d_b_enc) ICD_TRY(icd_colsum(partial + A, W, (int64_t)n_img * chunks, A, nullptr, d_b_enc, s));
+    ICD_TRY(icd_colsum(partial + 2 * A, W, (int64_t)n_img * chunks, 1, nullptr, d_b_full, s));
+    return 0;
 }
 
 extern "C" int icd_attention_proj_bwd(int B, int T, int P, int A, const int32_t* bt_host,
@@ -1160,49 +1313,62 @@ int icd_attention_step_fwd_grouped(int n_img, int k, int P, int C, int A, const 
 //   d_enc[b,p,c] = sum_{t < len_b} alpha[b,t,p] * d_awe[t,b,c]  +  d_mean[b,c] / P          (written, not accumulated)
 // The enc_att part, d_att_enc W_e, is added afterwards by a contraction with beta = 1.
 // grid = (ceil(C/1024), B), block = 256 threads x 4 channels; d_awe of up to 32 steps lives in registers, alphas in smem.
+// row_ptr != NULL (captions that share images): CTA row i is image i and d_enc[i] is the sum of the above over the rows
+// rows[row_ptr[i] .. row_ptr[i+1]), added in that order (an image without rows gets zeros).
 // ------------------------------------------------------------------------------------------------
 namespace {
 constexpr int EG_TCH = 32;
 __global__ void __launch_bounds__(256, 1) enc_grad_kernel(int B, int T, int P, int C, const int* __restrict__ row_len,
+                                                          const int* __restrict__ row_ptr, const int* __restrict__ rows,
                                                           const float* __restrict__ alphas,      // (B,T,P)
                                                           const float* __restrict__ d_awe_all,   // (T,B,C)
                                                           const float* __restrict__ d_mean,      // (B,C) or NULL
                                                           float* __restrict__ d_enc) {           // (B,P,C)
     extern __shared__ __align__(16) float sm[];     // EG_TCH * P alphas of the current step chunk
-    const int b = blockIdx.y;
+    const int img = blockIdx.y;
     const int c = blockIdx.x * 1024 + threadIdx.x * 4;
-    const int Tb = row_len ? row_len[b] : T;
     const float invP = 1.f / (float)P;
-    for (int t0 = 0; t0 < max(Tb, 1); t0 += EG_TCH) {
-        const int nt = min(EG_TCH, Tb - t0);
-        __syncthreads();
-        for (int i = threadIdx.x; i < max(nt, 0) * P; i += blockDim.x)
-            sm[i] = alphas[((long long)b * T + t0 + i / P) * P + (i % P)];
-        __syncthreads();
-        if (c >= C) continue;
-        float4 da[EG_TCH];
+    const int k0 = row_ptr ? row_ptr[img] : img, k1 = row_ptr ? row_ptr[img + 1] : img + 1;
+    if (k0 == k1 && c < C)
+        for (int p = 0; p < P; ++p) *reinterpret_cast<float4*>(d_enc + ((long long)img * P + p) * C + c) = make_float4(0.f, 0.f, 0.f, 0.f);
+    for (int k = k0; k < k1; ++k) {
+        const int b = row_ptr ? rows[k] : img;
+        const int Tb = row_len ? row_len[b] : T;
+        for (int t0 = 0; t0 < max(Tb, 1); t0 += EG_TCH) {
+            const int nt = min(EG_TCH, Tb - t0);
+            __syncthreads();
+            for (int j = threadIdx.x; j < max(nt, 0) * P; j += blockDim.x)
+                sm[j] = alphas[((long long)b * T + t0 + j / P) * P + (j % P)];
+            __syncthreads();
+            if (c >= C) continue;
+            float4 da[EG_TCH];
 #pragma unroll
-        for (int u = 0; u < EG_TCH; ++u)
-            da[u] = (u < nt) ? *reinterpret_cast<const float4*>(d_awe_all + ((long long)(t0 + u) * B + b) * C + c)
-                             : make_float4(0.f, 0.f, 0.f, 0.f);
-        float4 base = make_float4(0.f, 0.f, 0.f, 0.f);
-        if (t0 == 0 && d_mean) {
-            const float4 m = *reinterpret_cast<const float4*>(d_mean + (long long)b * C + c);
-            base = make_float4(m.x * invP, m.y * invP, m.z * invP, m.w * invP);
-        }
-        for (int p = 0; p < P; ++p) {
-            float4 acc = base;
-            float* o = d_enc + ((long long)b * P + p) * C + c;
-            if (t0 > 0) acc = *reinterpret_cast<const float4*>(o);
-#pragma unroll
-            for (int u = 0; u < EG_TCH; ++u) {
-                if (u < nt) {
-                    const float al = sm[u * P + p];
-                    acc.x = fmaf(al, da[u].x, acc.x); acc.y = fmaf(al, da[u].y, acc.y);
-                    acc.z = fmaf(al, da[u].z, acc.z); acc.w = fmaf(al, da[u].w, acc.w);
-                }
+            for (int u = 0; u < EG_TCH; ++u)
+                da[u] = (u < nt) ? *reinterpret_cast<const float4*>(d_awe_all + ((long long)(t0 + u) * B + b) * C + c)
+                                 : make_float4(0.f, 0.f, 0.f, 0.f);
+            float4 base = make_float4(0.f, 0.f, 0.f, 0.f);
+            if (t0 == 0 && d_mean) {
+                const float4 m = *reinterpret_cast<const float4*>(d_mean + (long long)b * C + c);
+                base = make_float4(m.x * invP, m.y * invP, m.z * invP, m.w * invP);
             }
-            *reinterpret_cast<float4*>(o) = acc;
+            for (int p = 0; p < P; ++p) {
+                float4 acc = base;
+                float* o = d_enc + ((long long)img * P + p) * C + c;
+                if (t0 > 0) acc = *reinterpret_cast<const float4*>(o);
+                else if (k > k0) {                                    // a later row of the image: add to the rows before it
+                    const float4 prev = *reinterpret_cast<const float4*>(o);
+                    acc = make_float4(prev.x + base.x, prev.y + base.y, prev.z + base.z, prev.w + base.w);
+                }
+#pragma unroll
+                for (int u = 0; u < EG_TCH; ++u) {
+                    if (u < nt) {
+                        const float al = sm[u * P + p];
+                        acc.x = fmaf(al, da[u].x, acc.x); acc.y = fmaf(al, da[u].y, acc.y);
+                        acc.z = fmaf(al, da[u].z, acc.z); acc.w = fmaf(al, da[u].w, acc.w);
+                    }
+                }
+                *reinterpret_cast<float4*>(o) = acc;
+            }
         }
     }
 }
@@ -1211,8 +1377,15 @@ __global__ void __launch_bounds__(256, 1) enc_grad_kernel(int B, int T, int P, i
 extern "C" int icd_attention_enc_grad(int B, int T, int P, int C, const int32_t* bt_host,
                                       const float* alphas, const float* d_awe_all, const float* d_mean,
                                       float* d_enc, int32_t* row_len_ws, void* stream) {
-    cudaStream_t s = icd_stream(stream);
+    return icd_attention_enc_grad_indexed(B, B, T, P, C, bt_host, nullptr, nullptr, alphas, d_awe_all, d_mean, d_enc, row_len_ws,
+                                          icd_stream(stream));
+}
+
+int icd_attention_enc_grad_indexed(int B, int n_img, int T, int P, int C, const int32_t* bt_host, const int32_t* row_ptr,
+                                   const int32_t* rows, const float* alphas, const float* d_awe_all, const float* d_mean,
+                                   float* d_enc, int32_t* row_len_ws, cudaStream_t s) {
     ICD_CHECK_ARG(B > 0 && T > 0 && T <= ICD_MAX_STEPS && C % 4 == 0 && B <= 65535, "attention_enc_grad: bad dims");
+    ICD_CHECK_ARG(n_img > 0 && n_img <= 65535 && (row_ptr != nullptr || n_img == B), "attention_enc_grad: bad image count");
     ICD_CHECK_ARG(alphas && d_awe_all && d_enc, "attention_enc_grad: null argument");
     int* row_len = nullptr;
     if (bt_host) {
@@ -1230,8 +1403,8 @@ extern "C" int icd_attention_enc_grad(int B, int T, int P, int C, const int32_t*
         ICD_CUDA(cudaFuncSetAttribute(enc_grad_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
         configured = smem;
     }
-    dim3 grid((C + 1023) / 1024, B);
-    enc_grad_kernel<<<grid, 256, smem, s>>>(B, T, P, C, row_len, alphas, d_awe_all, d_mean, d_enc);
+    dim3 grid((C + 1023) / 1024, n_img);
+    enc_grad_kernel<<<grid, 256, smem, s>>>(B, T, P, C, row_len, (const int*)row_ptr, (const int*)rows, alphas, d_awe_all, d_mean, d_enc);
     ICD_LAUNCH_CHECK();
     return 0;
 }

@@ -351,7 +351,7 @@ template <bool DEEP>     // DEEP (launches of at most two CTAs per SM: few rows,
                          // in flight in the two streaming phases — such a launch is bound by its chain of dependent load batches.
                          // Same operations in the same order as the 64-register instantiation: bit-identical (tested).
 __global__ void __launch_bounds__(256, DEEP ? 2 : 4) att_step_bwd_bf16_kernel(
-        int P, int C, int A,
+        int P, int C, int A, const int* __restrict__ img_index,
         const __nv_bfloat16* __restrict__ enc, const __nv_bfloat16* __restrict__ att_enc,
         const float* __restrict__ att_dec, long long ld_dec, const float* __restrict__ w_full,
         const float* __restrict__ alpha, long long ld_alpha,
@@ -391,6 +391,7 @@ __global__ void __launch_bounds__(256, DEEP ? 2 : 4) att_step_bwd_bf16_kernel(
     const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5, nwarp = blockDim.x >> 5;
     pdl_trigger();
     pdl_wait();
+    const int img = img_index ? img_index[r] : r;
 
     // (A) gate backward (elementwise over C)
     {
@@ -439,7 +440,7 @@ __global__ void __launch_bounds__(256, DEEP ? 2 : 4) att_step_bwd_bf16_kernel(
         const int CW = C / nwarp, NB = CW >> 5;
         const int cb0 = warp * CW;
         const int Pp16 = ((P + 15) >> 4) << 4;
-        const __nv_bfloat16* eb = enc + (long long)r * P * C + cb0 + 8 * t;
+        const __nv_bfloat16* eb = enc + (long long)img * P * C + cb0 + 8 * t;
         const __nv_bfloat16* bsrc = (g < 3) ? (s_hl + g * C + cb0 + 8 * t) : s_hl;
         for (int pb = p_lo >> 4; pb < ((p_hi + 15) >> 4); ++pb) {
             const int p0 = pb * 16 + g, p1 = p0 + 8;
@@ -483,7 +484,7 @@ __global__ void __launch_bounds__(256, DEEP ? 2 : 4) att_step_bwd_bf16_kernel(
             s_de[p] = acc;
         }
     } else {
-        const __nv_bfloat16* eb = enc + (long long)r * P * C;
+        const __nv_bfloat16* eb = enc + (long long)img * P * C;
         const int C8 = C >> 3;
         for (int p = p_lo + warp; p < p_hi; p += nwarp) {
             const __nv_bfloat16* row = eb + (long long)p * C;
@@ -546,7 +547,7 @@ __global__ void __launch_bounds__(256, DEEP ? 2 : 4) att_step_bwd_bf16_kernel(
     // (D) d_att_dec[a] = w_full[a] * sum_p d_e[p] * [att_enc[p,a] + att_dec[a] > 0]
     //     thread = (pixel group g of 4, 8-channel column j); loops over column chunks of 64 * 8 channels
     {
-        const __nv_bfloat16* ab = att_enc + (long long)r * P * A;
+        const __nv_bfloat16* ab = att_enc + (long long)img * P * A;
         const int A8 = A >> 3;
         const int grp = threadIdx.x >> 6, t = threadIdx.x & 63;
         for (int j0 = 0; j0 < A8; j0 += 64) {
@@ -830,13 +831,150 @@ __global__ void __launch_bounds__(1024) att_proj_bwd_bf16_kernel_wide(int B, int
     att_proj_bwd_bf16_body(B, T, P, A, row_len, att_enc, att_dec_all, ld_dec, w_full, d_e, d_att_enc, d_att_enc16, partial, split_wfull);
 }
 
+// Captions that share images: the same pass per IMAGE i over the (row, step) pairs of its rows (rows in CSR order, then steps):
+//   d_att_enc[i,p,a] = w_full[a] * sum_{r in rows(i)} sum_{t < len_r} d_e[r,t,p] * [att_enc[i,p,a] + att_dec[t,r,a] > 0]
+// grid = (ceil(P/PROJ_IMG16_PB), n_img), block = 2 x A/4 threads: each half owns 4 of the CTA's 8 pixels, a thread 4 channels,
+// and the 16 masked sums stay in registers while the pairs pass through shared memory PROJ_IMG16_KC steps of one row at a
+// time — no per-row (B,P,A) tensor, a fixed summation order.  The split form of d_w_full and its fallback are those above.
+// ------------------------------------------------------------------------------------------------
+constexpr int PROJ_IMG16_PB = 8, PROJ_IMG16_KC = 32;
+__global__ void __launch_bounds__(1024) att_proj_bwd_img_bf16_kernel(int B, int T, int P, int A, const int* __restrict__ row_len,
+                                         const int* __restrict__ row_ptr, const int* __restrict__ rows,
+                                         const __nv_bfloat16* __restrict__ att_enc,
+                                         const float* __restrict__ att_dec_all, long long ld_dec,
+                                         const float* __restrict__ w_full, const float* __restrict__ d_e,
+                                         __nv_bfloat16* __restrict__ d_att_enc16, float* __restrict__ partial, int split_wfull) {
+    pdl_trigger();
+    pdl_wait();
+    extern __shared__ __align__(16) float sm[];
+    const int i = blockIdx.y, p0 = blockIdx.x * PROJ_IMG16_PB;
+    const int np = min(PROJ_IMG16_PB, P - p0);
+    float* s_dec = sm;                                        // PROJ_IMG16_KC * A
+    float* s_de = sm + (size_t)PROJ_IMG16_KC * A;             // PROJ_IMG16_KC * PROJ_IMG16_PB
+    float* s_red = s_de + PROJ_IMG16_KC * PROJ_IMG16_PB;      // 40
+    bool fast = false;
+    if (split_wfull) {
+        int bad = 0;
+        for (int a4 = threadIdx.x * 4; a4 < A; a4 += blockDim.x * 4) {
+            const float4 w = *reinterpret_cast<const float4*>(w_full + a4);
+            bad |= (fabsf(w.x) < PROJ_W_MIN) | (fabsf(w.y) < PROJ_W_MIN) | (fabsf(w.z) < PROJ_W_MIN) | (fabsf(w.w) < PROJ_W_MIN);
+        }
+        fast = __syncthreads_or(bad) == 0;
+    }
+    const float sgn = fast ? -1.f : 1.f;
+    const int th = blockDim.x >> 1, half = threadIdx.x / th;
+    const int a = (threadIdx.x - half * th) * 4, pq = half * 4;
+    float x[4][4], acc[4][4];
+#pragma unroll
+    for (int u = 0; u < 4; ++u)
+#pragma unroll
+        for (int c = 0; c < 4; ++c) { x[u][c] = 0.f; acc[u][c] = 0.f; }
+    if (a < A) {
+#pragma unroll
+        for (int u = 0; u < 4; ++u) {
+            const uint2 raw = ld_stream_u2(att_enc + ((long long)i * P + p0 + min(pq + u, np - 1)) * A + a);
+            x[u][0] = __uint_as_float(raw.x << 16); x[u][1] = __uint_as_float(raw.x & 0xffff0000u);
+            x[u][2] = __uint_as_float(raw.y << 16); x[u][3] = __uint_as_float(raw.y & 0xffff0000u);
+        }
+    }
+    float4 wacc = make_float4(0.f, 0.f, 0.f, 0.f);
+    float de_sum = 0.f;
+    for (int k = row_ptr[i]; k < row_ptr[i + 1]; ++k) {
+        const int b = rows[k], Tb = row_len[b];
+        for (int t0 = 0; t0 < Tb; t0 += PROJ_IMG16_KC) {
+            const int nt = min(PROJ_IMG16_KC, Tb - t0);
+            __syncthreads();                                  // the previous round is consumed
+            for (int j = threadIdx.x; j < nt * (A >> 2); j += blockDim.x) {
+                const int t = j / (A >> 2), a4 = (j % (A >> 2)) * 4;
+                const float4 v = *reinterpret_cast<const float4*>(att_dec_all + ((long long)(t0 + t) * B + b) * ld_dec + a4);
+                *reinterpret_cast<float4*>(s_dec + (size_t)t * A + a4) = make_float4(sgn * v.x, sgn * v.y, sgn * v.z, sgn * v.w);
+            }
+            for (int j = threadIdx.x; j < nt * PROJ_IMG16_PB; j += blockDim.x) {
+                const int t = j / PROJ_IMG16_PB, pp = j % PROJ_IMG16_PB;
+                const float v = (pp < np) ? d_e[((long long)b * T + t0 + t) * P + p0 + pp] : 0.f;
+                s_de[j] = v;
+                de_sum += v;
+            }
+            __syncthreads();
+            if (a >= A) continue;
+            if (fast) {
+                for (int t = 0; t < nt; ++t) {
+                    const float4 de4 = *reinterpret_cast<const float4*>(s_de + t * PROJ_IMG16_PB + pq);
+                    const float4 d = *reinterpret_cast<const float4*>(s_dec + (size_t)t * A + a);     // -att_dec[t]
+                    const float de[4] = {de4.x, de4.y, de4.z, de4.w};
+                    const float nd[4] = {d.x, d.y, d.z, d.w};
+#pragma unroll
+                    for (int u = 0; u < 4; ++u)
+#pragma unroll
+                        for (int c = 0; c < 4; ++c) acc[u][c] = fmaf(gt_mask(x[u][c], nd[c]), de[u], acc[u][c]);
+                }
+            } else {
+                for (int t = 0; t < nt; ++t) {
+                    const float4 de4 = *reinterpret_cast<const float4*>(s_de + t * PROJ_IMG16_PB + pq);
+                    const float4 d = *reinterpret_cast<const float4*>(s_dec + (size_t)t * A + a);
+                    const float de[4] = {de4.x, de4.y, de4.z, de4.w};
+                    const float dd[4] = {d.x, d.y, d.z, d.w};
+                    float wl[4] = {0.f, 0.f, 0.f, 0.f};
+#pragma unroll
+                    for (int u = 0; u < 4; ++u) {
+#pragma unroll
+                        for (int c = 0; c < 4; ++c) {
+                            const float sv = x[u][c] + dd[c];
+                            acc[u][c] += (sv > 0.f) ? de[u] : 0.f;
+                            wl[c] = fmaf(de[u], fmaxf(sv, 0.f), wl[c]);
+                        }
+                    }
+                    wacc.x += wl[0]; wacc.y += wl[1]; wacc.z += wl[2]; wacc.w += wl[3];
+                }
+            }
+        }
+    }
+    float4 bacc = make_float4(0.f, 0.f, 0.f, 0.f);
+    if (a < A) {
+        if (fast) {
+            float wl[4] = {0.f, 0.f, 0.f, 0.f};
+#pragma unroll
+            for (int u = 0; u < 4; ++u)
+#pragma unroll
+                for (int c = 0; c < 4; ++c) wl[c] = fmaf(x[u][c], acc[u][c], wl[c]);    // pixels past np carry S = 0
+            wacc = make_float4(wl[0], wl[1], wl[2], wl[3]);
+        }
+        const float4 w = *reinterpret_cast<const float4*>(w_full + a);
+#pragma unroll
+        for (int u = 0; u < 4; ++u) {
+            if (pq + u >= np) break;
+            const long long o = ((long long)i * P + p0 + pq + u) * A + a;
+            const float4 r = make_float4(acc[u][0] * w.x, acc[u][1] * w.y, acc[u][2] * w.z, acc[u][3] * w.w);
+            bacc.x += r.x; bacc.y += r.y; bacc.z += r.z; bacc.w += r.w;
+            *reinterpret_cast<uint2*>(d_att_enc16 + o) = make_uint2(pack2(r.x, r.y), pack2(r.z, r.w));
+        }
+    }
+    float* mine = partial + ((long long)i * gridDim.x + blockIdx.x) * (2 * A + 4);
+    __syncthreads();                                          // everyone is done with s_dec: reuse it to add the halves
+    if (half == 1 && a < A) { *reinterpret_cast<float4*>(s_dec + a) = wacc; *reinterpret_cast<float4*>(s_dec + A + a) = bacc; }
+    __syncthreads();
+    if (half == 0 && a < A) {
+        const float4 w1 = *reinterpret_cast<const float4*>(s_dec + a), b1 = *reinterpret_cast<const float4*>(s_dec + A + a);
+        *reinterpret_cast<float4*>(mine + a) = make_float4(wacc.x + w1.x, wacc.y + w1.y, wacc.z + w1.z, wacc.w + w1.w);
+        *reinterpret_cast<float4*>(mine + A + a) = make_float4(bacc.x + b1.x, bacc.y + b1.y, bacc.z + b1.z, bacc.w + b1.w);
+    }
+    const float tot = block_sum(de_sum, s_red);
+    if (threadIdx.x == 0) { mine[2 * A] = tot; mine[2 * A + 1] = 0.f; mine[2 * A + 2] = 0.f; mine[2 * A + 3] = 0.f; }
+}
+
 // ------------------------------------------------------------------------------------------------
 // fp32 features -> bf16 features + pixel mean in ONE pass over encoder_out (models/attention.py:161 mean(dim=1)).
 // grid = (ceil(C/256), B), block = 256 = 4 pixel groups x 64 float4 lanes.
 // ------------------------------------------------------------------------------------------------
+// row_ptr != NULL (captions that share images): CTA row b is image b, its mean goes to rows[row_ptr[b] .. row_ptr[b+1]).
+__device__ __forceinline__ void mean_rows(int b, const int* row_ptr, int& k0, int& k1) {
+    k0 = row_ptr ? row_ptr[b] : b;
+    k1 = row_ptr ? row_ptr[b + 1] : b + 1;
+}
 __global__ void __launch_bounds__(256) convert_features_kernel(int P, int C, const float* __restrict__ enc,
                                                                __nv_bfloat16* __restrict__ enc16,
-                                                               float* __restrict__ mean, __nv_bfloat16* __restrict__ mean16) {
+                                                               float* __restrict__ mean, __nv_bfloat16* __restrict__ mean16,
+                                                               const int* __restrict__ row_ptr, const int* __restrict__ rows) {
     pdl_trigger();
     pdl_wait();
     __shared__ float4 s_part[3 * 64];
@@ -871,9 +1009,13 @@ __global__ void __launch_bounds__(256) convert_features_kernel(int P, int C, con
         for (int g = 0; g < 3; ++g) { const float4 o = s_part[g * 64 + lane]; acc.x += o.x; acc.y += o.y; acc.z += o.z; acc.w += o.w; }
         const float inv = (float)P;
         acc.x /= inv; acc.y /= inv; acc.z /= inv; acc.w /= inv;
-        const long long o = (long long)b * C + c;
-        if (mean) *reinterpret_cast<float4*>(mean + o) = acc;
-        if (mean16) *reinterpret_cast<uint2*>(mean16 + o) = make_uint2(pack2(acc.x, acc.y), pack2(acc.z, acc.w));
+        int k0, k1;
+        mean_rows(b, row_ptr, k0, k1);
+        for (int k = k0; k < k1; ++k) {
+            const long long o = (long long)(row_ptr ? rows[k] : b) * C + c;
+            if (mean) *reinterpret_cast<float4*>(mean + o) = acc;
+            if (mean16) *reinterpret_cast<uint2*>(mean16 + o) = make_uint2(pack2(acc.x, acc.y), pack2(acc.z, acc.w));
+        }
     }
 }
 
@@ -891,7 +1033,8 @@ __global__ void row_len_from_pack_kernel16(int B, int T, const BtPack bt, int* _
 // pixel mean of bf16-stored features (models/attention.py:161) when the caller hands the features over in bf16.
 // grid = (ceil(C/512), B), block = 256 = 4 pixel groups x 64 lanes of 8 channels (16 B).
 __global__ void __launch_bounds__(256) feature_mean_bf16_kernel(int P, int C, const __nv_bfloat16* __restrict__ enc16,
-                                                                float* __restrict__ mean, __nv_bfloat16* __restrict__ mean16) {
+                                                                float* __restrict__ mean, __nv_bfloat16* __restrict__ mean16,
+                                                                const int* __restrict__ row_ptr, const int* __restrict__ rows) {
     pdl_trigger();
     pdl_wait();
     __shared__ float s_part[3 * 64 * 8];
@@ -936,14 +1079,18 @@ __global__ void __launch_bounds__(256) feature_mean_bf16_kernel(int P, int C, co
             acc[i] += s_part[(0 * 64 + lane) * 8 + i] + s_part[(1 * 64 + lane) * 8 + i] + s_part[(2 * 64 + lane) * 8 + i];
             acc[i] /= inv;
         }
-        const long long o = (long long)b * C + c;
-        if (mean) {
-            *reinterpret_cast<float4*>(mean + o) = make_float4(acc[0], acc[1], acc[2], acc[3]);
-            *reinterpret_cast<float4*>(mean + o + 4) = make_float4(acc[4], acc[5], acc[6], acc[7]);
+        int k0, k1;
+        mean_rows(b, row_ptr, k0, k1);
+        for (int k = k0; k < k1; ++k) {
+            const long long o = (long long)(row_ptr ? rows[k] : b) * C + c;
+            if (mean) {
+                *reinterpret_cast<float4*>(mean + o) = make_float4(acc[0], acc[1], acc[2], acc[3]);
+                *reinterpret_cast<float4*>(mean + o + 4) = make_float4(acc[4], acc[5], acc[6], acc[7]);
+            }
+            if (mean16)
+                *reinterpret_cast<uint4*>(mean16 + o) = make_uint4(pack2(acc[0], acc[1]), pack2(acc[2], acc[3]),
+                                                                   pack2(acc[4], acc[5]), pack2(acc[6], acc[7]));
         }
-        if (mean16)
-            *reinterpret_cast<uint4*>(mean16 + o) = make_uint4(pack2(acc[0], acc[1]), pack2(acc[2], acc[3]),
-                                                               pack2(acc[4], acc[5]), pack2(acc[6], acc[7]));
     }
 }
 
@@ -1067,6 +1214,21 @@ extern "C" int icd_attention_step_bwd_bf16(int rows, int P, int C, int A,
                                            float* d_fbeta_pre, int64_t ld_dfb,
                                            float* d_e, int64_t ld_de,
                                            void* dz16, int64_t ld_dz16, float* d_awe_out, void* stream) {
+    return icd_attention_step_bwd_bf16_idx(rows, P, C, A, nullptr, enc16, att_enc16, att_dec, ld_dec, w_full, alpha, ld_alpha,
+                                           d_alpha_ext, ld_dalpha, gate, awe_raw, d_gated, d_att_dec, ld_ddec, d_fbeta_pre, ld_dfb,
+                                           d_e, ld_de, dz16, ld_dz16, d_awe_out, stream);
+}
+
+int icd_attention_step_bwd_bf16_idx(int rows, int P, int C, int A, const int32_t* img_index,
+                                    const void* enc16, const void* att_enc16,
+                                    const float* att_dec, int64_t ld_dec, const float* w_full,
+                                    const float* alpha, int64_t ld_alpha,
+                                    const float* d_alpha_ext, int64_t ld_dalpha,
+                                    const float* gate, const float* awe_raw, const float* d_gated,
+                                    float* d_att_dec, int64_t ld_ddec,
+                                    float* d_fbeta_pre, int64_t ld_dfb,
+                                    float* d_e, int64_t ld_de,
+                                    void* dz16, int64_t ld_dz16, float* d_awe_out, void* stream) {
     cudaStream_t s = icd_stream(stream);
     if (rows == 0) return 0;
     ICD_CHECK_ARG(A % 8 == 0 && C % 8 == 0, "attention_step_bwd_bf16: A and C must be multiples of 8");
@@ -1085,7 +1247,7 @@ extern "C" int icd_attention_step_bwd_bf16(int rows, int P, int C, int A,
     const AttLaunchPlan plan = att_bwd16_plan(rows, P, smem);
     const int n_split = plan.shared_rows;
     icd_prof_mark_begin(1, rows, s);
-#define ICD_BWD16_ARGS P, C, A, reinterpret_cast<const __nv_bfloat16*>(enc16), reinterpret_cast<const __nv_bfloat16*>(att_enc16),           \
+#define ICD_BWD16_ARGS P, C, A, (const int*)img_index, reinterpret_cast<const __nv_bfloat16*>(enc16), reinterpret_cast<const __nv_bfloat16*>(att_enc16),           \
                        att_dec, (long long)ld_dec, w_full, alpha, (long long)ld_alpha, d_alpha_ext, (long long)ld_dalpha,                   \
                        gate, awe_raw, d_gated, d_att_dec, (long long)ld_ddec, d_fbeta_pre, (long long)ld_dfb,                               \
                        d_e, (long long)ld_de, reinterpret_cast<__nv_bfloat16*>(dz16), (long long)ld_dz16, d_awe_out, use_mma
@@ -1094,14 +1256,14 @@ extern "C" int icd_attention_step_bwd_bf16(int rows, int P, int C, int A,
                                         ICD_BWD16_ARGS, 0));
     else if (n_split > 0)
         ICD_CUDA(icd_launch_pdl_cluster(ICD_PDL_ATT_BWD, att_step_bwd_bf16_kernel<false>, dim3(rows + n_split), dim3(256), smem, s, 2u, P, C, A,
-                            reinterpret_cast<const __nv_bfloat16*>(enc16), reinterpret_cast<const __nv_bfloat16*>(att_enc16),
+                            (const int*)img_index, reinterpret_cast<const __nv_bfloat16*>(enc16), reinterpret_cast<const __nv_bfloat16*>(att_enc16),
                             att_dec, (long long)ld_dec, w_full, alpha, (long long)ld_alpha, d_alpha_ext, (long long)ld_dalpha,
                             gate, awe_raw, d_gated, d_att_dec, (long long)ld_ddec, d_fbeta_pre, (long long)ld_dfb,
                             d_e, (long long)ld_de, reinterpret_cast<__nv_bfloat16*>(dz16), (long long)ld_dz16, d_awe_out,
                             use_mma, rows - n_split));
     else
         ICD_CUDA(icd_launch_pdl(ICD_PDL_ATT_BWD, att_step_bwd_bf16_kernel<false>, dim3(rows), dim3(256), smem, s, P, C, A,
-                            reinterpret_cast<const __nv_bfloat16*>(enc16), reinterpret_cast<const __nv_bfloat16*>(att_enc16),
+                            (const int*)img_index, reinterpret_cast<const __nv_bfloat16*>(enc16), reinterpret_cast<const __nv_bfloat16*>(att_enc16),
                             att_dec, (long long)ld_dec, w_full, alpha, (long long)ld_alpha, d_alpha_ext, (long long)ld_dalpha,
                             gate, awe_raw, d_gated, d_att_dec, (long long)ld_ddec, d_fbeta_pre, (long long)ld_dfb,
                             d_e, (long long)ld_de, reinterpret_cast<__nv_bfloat16*>(dz16), (long long)ld_dz16, d_awe_out,
@@ -1173,20 +1335,73 @@ extern "C" int icd_attention_proj_bwd_bf16_ex(int B, int T, int P, int A, const 
     return 0;
 }
 
-int icd_convert_features_bf16(int B, int P, int C, const float* enc, void* enc16, float* mean, void* mean16, cudaStream_t s) {
+// per-image pass (see att_proj_bwd_img_bf16_kernel); partial: icd_attention_proj_bwd_ws_floats_indexed floats, whose layout
+// (per-image partials, then B row lengths, then the (1 + COLDOT_CHUNKS) * A floats of the split d_w_full) is that of the
+// per-row pass with n_img * ceil(P / PROJ_IMG16_PB) partial rows
+int icd_attention_proj_bwd_bf16_indexed(int B, int n_img, int T, int P, int A, const int32_t* bt_host, const int32_t* row_ptr,
+                                        const int32_t* rows, const void* att_enc16, const float* att_dec_all, int64_t ld_dec,
+                                        const float* w_full, const float* d_e, void* d_att_enc16, float* d_w_full,
+                                        float* d_b_full, float* d_b_enc, float* partial, const float* d_att_dec_all,
+                                        int64_t ld_ddec, cudaStream_t s) {
+    ICD_CHECK_ARG(T > 0 && T <= ICD_MAX_STEPS, "attention_proj_bwd_bf16: T=%d out of range", T);
+    ICD_CHECK_ARG(A % 4 == 0 && A / 4 <= 512, "attention_proj_bwd_bf16: A=%d unsupported", A);
+    ICD_CHECK_ARG(ld_dec % 4 == 0, "attention_proj_bwd_bf16: ld_dec must be a multiple of 4");
+    ICD_CHECK_ARG(n_img > 0 && n_img <= 65535, "attention_proj_bwd_bf16: n_img=%d out of range", n_img);
+    const int chunks = (P + PROJ_IMG16_PB - 1) / PROJ_IMG16_PB;
+    const int W = 2 * A + 4;
+    const int64_t nparts = (int64_t)n_img * chunks;
+    int* row_len = reinterpret_cast<int*>(partial + nparts * W);
+    BtPack pack;
+    for (int t = 0; t < ICD_MAX_STEPS; ++t) pack.v[t] = t < T ? bt_host[t] : 0;
+    ICD_CUDA(icd_launch_pdl(ICD_PDL_POINTWISE, row_len_from_pack_kernel16, dim3((unsigned)((B + 127) / 128)), dim3(128), (size_t)0, s, B, T, pack, row_len));
+    ICD_LAUNCH_CHECK();
+    const size_t smem = ((size_t)PROJ_IMG16_KC * (A + PROJ_IMG16_PB) + 40) * sizeof(float);
+    ICD_CHECK_ARG(smem <= 220 * 1024, "attention_proj_bwd_bf16: A too large for shared memory");
+    static size_t configured = 48 * 1024;
+    if (smem > configured) {
+        ICD_CUDA(cudaFuncSetAttribute(att_proj_bwd_img_bf16_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+        configured = smem;
+    }
+    const int threads = 2 * (((A / 4 + 31) / 32) * 32);
+    ICD_CUDA(icd_launch_pdl(ICD_PDL_POINTWISE, att_proj_bwd_img_bf16_kernel, dim3(chunks, n_img), dim3((unsigned)threads), smem, s,
+                            B, T, P, A, (const int*)row_len, (const int*)row_ptr, (const int*)rows,
+                            reinterpret_cast<const __nv_bfloat16*>(att_enc16), att_dec_all, (long long)ld_dec, w_full, d_e,
+                            reinterpret_cast<__nv_bfloat16*>(d_att_enc16), partial, d_att_dec_all ? 1 : 0));
+    ICD_LAUNCH_CHECK();
+    ICD_TRY(icd_colsum(partial, W, nparts, A, nullptr, d_w_full, s));
+    if (d_att_dec_all) {
+        float* t2 = partial + nparts * W + B + 8;
+        float* t2_parts = t2 + A;
+        ICD_CUDA(icd_launch_pdl(ICD_PDL_POINTWISE, coldot_kernel, dim3((A + 31) / 32, COLDOT_CHUNKS), dim3(32, 32), (size_t)0, s, att_dec_all,
+                                (long long)ld_dec, d_att_dec_all, (long long)ld_ddec, (long long)T * B, A, t2_parts));
+        ICD_LAUNCH_CHECK();
+        ICD_TRY(icd_colsum(t2_parts, A, COLDOT_CHUNKS, A, nullptr, t2, s));
+        ICD_CUDA(icd_launch_pdl(ICD_PDL_POINTWISE, proj_wfull_finish_kernel, dim3(1), dim3(256), (size_t)0, s, A, w_full, (const float*)t2, d_w_full));
+        ICD_LAUNCH_CHECK();
+    }
+    if (d_b_enc) ICD_TRY(icd_colsum(partial + A, W, nparts, A, nullptr, d_b_enc, s));
+    ICD_TRY(icd_colsum(partial + 2 * A, W, nparts, 1, nullptr, d_b_full, s));
+    return 0;
+}
+
+int icd_convert_features_bf16(int B, int P, int C, const float* enc, void* enc16, float* mean, void* mean16, cudaStream_t s,
+                              const int32_t* row_ptr, const int32_t* rows) {
     ICD_CHECK_ARG(C % 4 == 0 && B <= 65535, "convert_features: C=%d must be a multiple of 4, B <= 65535", C);
     dim3 grid((C + 255) / 256, B);
     ICD_CUDA(icd_launch_pdl(ICD_PDL_POINTWISE, convert_features_kernel, grid, dim3(256), (size_t)0, s, P, C, enc,
-                            reinterpret_cast<__nv_bfloat16*>(enc16), mean, reinterpret_cast<__nv_bfloat16*>(mean16)));
+                            reinterpret_cast<__nv_bfloat16*>(enc16), mean, reinterpret_cast<__nv_bfloat16*>(mean16),
+                            (const int*)row_ptr, (const int*)rows));
     ICD_LAUNCH_CHECK();
     return 0;
 }
 
-int icd_feature_mean_bf16(int B, int P, int C, const void* enc16, float* mean, void* mean16, cudaStream_t s) {
+int icd_feature_mean_bf16(int B, int P, int C, const void* enc16, float* mean, void* mean16, cudaStream_t s,
+                          const int32_t* row_ptr, const int32_t* rows) {
     ICD_CHECK_ARG(C % 8 == 0 && B <= 65535, "feature_mean_bf16: C=%d must be a multiple of 8, B <= 65535", C);
     dim3 grid((C + 511) / 512, B);
     ICD_CUDA(icd_launch_pdl(ICD_PDL_POINTWISE, feature_mean_bf16_kernel, grid, dim3(256), (size_t)0, s, P, C,
-                            reinterpret_cast<const __nv_bfloat16*>(enc16), mean, reinterpret_cast<__nv_bfloat16*>(mean16)));
+                            reinterpret_cast<const __nv_bfloat16*>(enc16), mean, reinterpret_cast<__nv_bfloat16*>(mean16),
+                            (const int*)row_ptr, (const int*)rows));
     ICD_LAUNCH_CHECK();
     return 0;
 }

@@ -172,7 +172,32 @@ int icd_lstm_pointwise_bwd(int rows, int D, const float* dh_in, const float* d_h
                            const float* dh_parts = nullptr, int n_parts = 0, int parts_rows = 0);   // deferred split-K planes of dh
 int icd_weighted_pixel_sum(int rows, int P, int C, const int32_t* img_index, const float* enc,
                            const float* alpha, int64_t ld_alpha, const float* fbeta_pre, int64_t ld_fb,
-                           float* awe_raw, float* gate, float* gated, cudaStream_t s);
+                           float* awe_raw, float* gate, float* gated, cudaStream_t s,
+                           const int32_t* out_row_ptr = nullptr, const int32_t* out_rows = nullptr);
+// ---- captions that share images (icd_att_index_t): the step backward with an image index, and the per-image reductions ----
+int icd_attention_step_bwd_idx(int rows, int P, int C, int A, const int32_t* img_index, const float* enc, const float* att_enc,
+                               const float* att_dec, int64_t ld_dec, const float* w_full, const float* alpha, int64_t ld_alpha,
+                               const float* d_alpha_ext, int64_t ld_dalpha, const float* gate, const float* awe_raw,
+                               const float* d_gated, float* d_att_dec, int64_t ld_ddec, float* d_fbeta_pre, int64_t ld_dfb,
+                               float* d_e, int64_t ld_de, float* d_awe_out, void* stream);
+int icd_attention_step_bwd_bf16_idx(int rows, int P, int C, int A, const int32_t* img_index, const void* enc16,
+                                    const void* att_enc16, const float* att_dec, int64_t ld_dec, const float* w_full,
+                                    const float* alpha, int64_t ld_alpha, const float* d_alpha_ext, int64_t ld_dalpha,
+                                    const float* gate, const float* awe_raw, const float* d_gated, float* d_att_dec,
+                                    int64_t ld_ddec, float* d_fbeta_pre, int64_t ld_dfb, float* d_e, int64_t ld_de,
+                                    void* dz16, int64_t ld_dz16, float* d_awe_out, void* stream);
+int icd_attention_proj_bwd_indexed(int B, int n_img, int T, int P, int A, const int32_t* bt_host, const int32_t* row_ptr,
+                                   const int32_t* rows, const float* att_enc, const float* att_dec_all, int64_t ld_dec,
+                                   const float* w_full, const float* d_e, float* d_att_enc, float* d_w_full, float* d_b_full,
+                                   float* d_b_enc, float* partial, cudaStream_t s);
+int icd_attention_proj_bwd_bf16_indexed(int B, int n_img, int T, int P, int A, const int32_t* bt_host, const int32_t* row_ptr,
+                                        const int32_t* rows, const void* att_enc16, const float* att_dec_all, int64_t ld_dec,
+                                        const float* w_full, const float* d_e, void* d_att_enc16, float* d_w_full,
+                                        float* d_b_full, float* d_b_enc, float* partial, const float* d_att_dec_all,
+                                        int64_t ld_ddec, cudaStream_t s);
+int icd_attention_enc_grad_indexed(int B, int n_img, int T, int P, int C, const int32_t* bt_host, const int32_t* row_ptr,
+                                   const int32_t* rows, const float* alphas, const float* d_awe_all, const float* d_mean,
+                                   float* d_enc, int32_t* row_len_ws, cudaStream_t s);
 int icd_attention_step_fwd_grouped(int n_img, int k, int P, int C, int A, const int* k_live, const float* enc,
                                    const float* att_enc, const float* att_dec, int64_t ld_dec, const float* w_full,
                                    const float* b_full, const float* fbeta_pre, int64_t ld_fb, float* alpha,

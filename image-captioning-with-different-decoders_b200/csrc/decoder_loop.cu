@@ -39,6 +39,15 @@ int check_common(const icd_att_desc_t* d) {
 
 }  // namespace
 
+// captions that share images (icd_att_index_t): the index is checked here, its device contents are the caller's
+int icd_check_att_index(const icd_att_desc_t* d, const icd_att_index_t* ix) {
+    if (!ix) return 0;
+    ICD_CHECK_ARG(ix->n_img > 0 && ix->n_img <= 65535, "attention_decoder: n_img=%d out of range (1..65535)", ix->n_img);
+    ICD_CHECK_ARG(ix->img_index && ix->img_row_ptr && ix->img_rows, "attention_decoder: the image index needs img_index, img_row_ptr and img_rows");
+    ICD_CHECK_ARG(d->d_enc == nullptr || d->d_awe_all != nullptr, "attention_decoder: d_enc needs the d_awe_all scratch buffer");
+    return 0;
+}
+
 extern "C" int icd_init_hidden_state(int B, int P, int C, int D, int precision, const float* enc,
                                      const float* h_lin_w, const float* h_lin_b,
                                      const float* c_lin_w, const float* c_lin_b,
@@ -54,9 +63,9 @@ extern "C" int icd_init_hidden_state(int B, int P, int C, int D, int precision, 
     return 0;
 }
 
-int64_t icd_att_tc_ws_bytes(const icd_att_desc_t* d);                         // decoder_loop_bf16.cu
-int icd_attention_decoder_fwd_bf16(const icd_att_desc_t* d, cudaStream_t s);
-int icd_attention_decoder_bwd_bf16(const icd_att_desc_t* d, cudaStream_t s);
+int64_t icd_att_tc_ws_bytes(const icd_att_desc_t* d, int n_img);             // decoder_loop_bf16.cu
+int icd_attention_decoder_fwd_bf16(const icd_att_desc_t* d, const icd_att_index_t* ix, cudaStream_t s);
+int icd_attention_decoder_bwd_bf16(const icd_att_desc_t* d, const icd_att_index_t* ix, cudaStream_t s);
 
 // fp32-grade tier: the splits of the two weight matrices every step of the time loop reads ([W_dec; W_fbeta; W_hh] and
 // W_ih[:, E:], K-major in the forward loop, MN-major in the BPTT) are made once per call and kept at the tail of tc_ws
@@ -67,25 +76,31 @@ static int64_t x3_cache_bytes(const icd_att_desc_t* d) {
     return icd_x3_split_bytes(NZ, d->D) + icd_x3_split_bytes(4 * (int64_t)d->D, d->C) + 512;
 }
 
-extern "C" int64_t icd_attention_decoder_ws_bytes(const icd_att_desc_t* d) {
+static int64_t ws_bytes(const icd_att_desc_t* d, const icd_att_index_t* ix) {
     if (!d) return 0;
-    if (d->precision == ICD_PREC_BF16) return icd_att_tc_ws_bytes(d);
+    const int64_t n_img = ix ? ix->n_img : d->B;        // the rows of the per-image contractions are n_img * P pixel rows
+    if (d->precision == ICD_PREC_BF16) return icd_att_tc_ws_bytes(d, (int)n_img);
     if (d->precision != ICD_PREC_FP32X3) return 0;
     // fp32-grade tensor-core tier: every contraction splits its two operands on the fly (gemm_tc.cu); size for the largest
     const int64_t B = d->B, T = d->T, P = d->P, C = d->C, A = d->A, D = d->D, E = d->E, V = d->V, NZ = A + C + 4 * D, TB = T * B;
+    const int64_t NP = n_img * P;
     const int64_t shapes[][3] = {
-        {B * P, A, C}, {B, D, C}, {TB, 4 * D, E}, {B, NZ, D}, {B, 4 * D, C}, {B * T, V, D},
+        {NP, A, C}, {B, D, C}, {TB, 4 * D, E}, {B, NZ, D}, {B, 4 * D, C}, {B * T, V, D},
         {B * T, D, V}, {V, D, B * T}, {B, C, 4 * D}, {B, D, NZ}, {D, C, B}, {NZ, D, TB}, {4 * D, E, TB}, {4 * D, C, TB},
-        {TB, E, 4 * D}, {A, C, B * P}, {B, C, D}, {B * P, C, A}};
+        {TB, E, 4 * D}, {A, C, NP}, {B, C, D}, {NP, C, A}};
     int64_t need = 0;
     for (const auto& sh : shapes) need = std::max(need, icd_gemm_ws_bytes((int)sh[0], (int)sh[1], (int)sh[2], ICD_PREC_FP32X3));
     return need + x3_cache_bytes(d);
 }
 
-extern "C" int icd_attention_decoder_fwd(const icd_att_desc_t* d, void* stream) {
+extern "C" int64_t icd_attention_decoder_ws_bytes(const icd_att_desc_t* d) { return ws_bytes(d, nullptr); }
+extern "C" int64_t icd_attention_decoder_ws_bytes_indexed(const icd_att_desc_t* d, const icd_att_index_t* ix) { return ws_bytes(d, ix); }
+
+static int decoder_fwd(const icd_att_desc_t* d, const icd_att_index_t* ix, void* stream) {
     ICD_TRY(check_common(d));
+    ICD_TRY(icd_check_att_index(d, ix));
     cudaStream_t s = icd_stream(stream);
-    if (d->precision == ICD_PREC_BF16) return icd_attention_decoder_fwd_bf16(d, s);
+    if (d->precision == ICD_PREC_BF16) return icd_attention_decoder_fwd_bf16(d, ix, s);
     ICD_CHECK_ARG(d->precision == ICD_PREC_FP32 || d->precision == ICD_PREC_FP32X3, "attention_decoder: unknown precision %d", d->precision);
     ICD_CHECK_ARG(d->enc != nullptr, "attention_decoder(fp32): enc is required (bf16-stored features need ICD_PREC_BF16)");
     IcdSimpleWsScope ws_scope(d->tc_ws, d->tc_ws_bytes, x3_cache_bytes(d));   // ICD_PREC_FP32X3: operand splits live in the caller's arena
@@ -95,6 +110,8 @@ extern "C" int icd_attention_decoder_fwd(const icd_att_desc_t* d, void* stream) 
     const int NZ = A + C + 4 * D;
     const int prec = d->precision;
     const long long BD = (long long)B * D;
+    const int n_img = ix ? ix->n_img : B;
+    const int32_t* img_index = ix ? ix->img_index : nullptr;
 
     BtPack pack;
     for (int t = 0; t < ICD_MAX_STEPS; ++t) pack.v[t] = t < T ? d->bt_host[t] : 0;
@@ -120,11 +137,19 @@ extern "C" int icd_attention_decoder_fwd(const icd_att_desc_t* d, void* stream) 
     ICD_CUDA(cudaMemsetAsync(d->b_cat + A + C, 0, sizeof(float) * 4 * D, s));
 
     // K1: att_enc = enc_att(encoder_out), once per batch (:54)
-    ICD_TRY(icd_gemm_simple(prec, d->enc, C, 1, d->enc_att_w, C, 1, d->att_enc, A, B * P, A, C,
+    ICD_TRY(icd_gemm_simple(prec, d->enc, C, 1, d->enc_att_w, C, 1, d->att_enc, A, n_img * P, A, C,
                             d->enc_att_b, nullptr, nullptr, 0, nullptr, 0, nullptr, 0.f, s));
-    // K7: init_hidden_state (:250)
-    ICD_TRY(icd_init_hidden_state(B, P, C, D, prec, d->enc, d->h_lin_w, d->h_lin_b, d->c_lin_w, d->c_lin_b,
-                                  d->mean_enc, d->h_all, d->c_all, s));
+    // K7: init_hidden_state (:250); with an image index the pixel mean is formed once per image and written to its rows
+    if (ix) {
+        ICD_TRY(icd_weighted_pixel_sum(n_img, P, C, nullptr, d->enc, nullptr, 0, nullptr, 0, d->mean_enc, nullptr, nullptr, s,
+                                       ix->img_row_ptr, ix->img_rows));
+        ICD_TRY(icd_gemm_simple(prec, d->mean_enc, C, 1, d->h_lin_w, C, 1, d->h_all, D, B, D, C, d->h_lin_b, nullptr,
+                                nullptr, 0, nullptr, 0, nullptr, 0.f, s));
+        ICD_TRY(icd_gemm_simple(prec, d->mean_enc, C, 1, d->c_lin_w, C, 1, d->c_all, D, B, D, C, d->c_lin_b, nullptr,
+                                nullptr, 0, nullptr, 0, nullptr, 0.f, s));
+    } else
+        ICD_TRY(icd_init_hidden_state(B, P, C, D, prec, d->enc, d->h_lin_w, d->h_lin_b, d->c_lin_w, d->c_lin_b,
+                                      d->mean_enc, d->h_all, d->c_all, s));
     // K5: embedding lookup (:247) + hoisted input contraction
     // emb_w == NULL: emb_x (T,B,E) was filled by the caller with pre-computed embeddings (the reference's use_bert branch,
     // models/attention.py:242-244: (B,L,768) BERT vectors instead of the table lookup); they carry no gradient
@@ -142,7 +167,7 @@ extern "C" int icd_attention_decoder_fwd(const icd_att_desc_t* d, void* stream) 
         ICD_TRY(icd_gemm_simple(prec, h_prev, D, 1, d->w_cat, D, 1, zt, NZ, bt, NZ, D, d->b_cat, nullptr,
                                 nullptr, 0, nullptr, 0, nullptr, 0.f, s));
         // K3: attention + gate (:267-271); alpha goes straight into attention_weights[:bt, t, :] (:281)
-        ICD_TRY(icd_attention_step_fwd(bt, P, C, A, nullptr, d->enc, d->att_enc, zt, NZ,
+        ICD_TRY(icd_attention_step_fwd(bt, P, C, A, img_index, d->enc, d->att_enc, zt, NZ,
                                        d->full_att_w, d->full_att_b, zt + A, NZ,
                                        d->alphas + (size_t)t * P, (int64_t)T * P,
                                        d->awe_raw + (size_t)t * B * C, d->gate + (size_t)t * B * C,
@@ -163,10 +188,16 @@ extern "C" int icd_attention_decoder_fwd(const icd_att_desc_t* d, void* stream) 
     return 0;
 }
 
-extern "C" int icd_attention_decoder_bwd(const icd_att_desc_t* d, void* stream) {
+extern "C" int icd_attention_decoder_fwd(const icd_att_desc_t* d, void* stream) { return decoder_fwd(d, nullptr, stream); }
+extern "C" int icd_attention_decoder_fwd_indexed(const icd_att_desc_t* d, const icd_att_index_t* ix, void* stream) {
+    return decoder_fwd(d, ix, stream);
+}
+
+static int decoder_bwd(const icd_att_desc_t* d, const icd_att_index_t* ix, void* stream) {
     ICD_TRY(check_common(d));
+    ICD_TRY(icd_check_att_index(d, ix));
     cudaStream_t s = icd_stream(stream);
-    if (d->precision == ICD_PREC_BF16) return icd_attention_decoder_bwd_bf16(d, s);
+    if (d->precision == ICD_PREC_BF16) return icd_attention_decoder_bwd_bf16(d, ix, s);
     IcdSimpleWsScope ws_scope(d->tc_ws, d->tc_ws_bytes, x3_cache_bytes(d));
     icd_x3_cache_mark(d->w_cat);
     icd_x3_cache_mark(d->w_ih + d->E);
@@ -175,6 +206,8 @@ extern "C" int icd_attention_decoder_bwd(const icd_att_desc_t* d, void* stream) 
     const int prec = d->precision;
     const long long BD = (long long)B * D;
     const int TB = T * B;
+    const int n_img = ix ? ix->n_img : B;
+    const int32_t* img_index = ix ? ix->img_index : nullptr;
 
     ICD_CUDA(cudaMemsetAsync(d->dz, 0, sizeof(float) * (size_t)TB * NZ, s));
     ICD_CUDA(cudaMemsetAsync(d->d_e, 0, sizeof(float) * (size_t)B * T * P, s));
@@ -205,7 +238,7 @@ extern "C" int icd_attention_decoder_bwd(const icd_att_desc_t* d, void* stream) 
         ICD_TRY(icd_gemm_simple(prec, dzt + A + C, NZ, 1, d->w_ih + E, 1, E + C, d->d_gated, C, bt, C, 4 * D,
                                 nullptr, nullptr, nullptr, 0, nullptr, 0, nullptr, 0.f, s));
         // attention + gate adjoint -> dz[:, 0:A] (d att_dec), dz[:, A:A+C] (d fbeta_pre), d_e saved
-        ICD_TRY(icd_attention_step_bwd(bt, P, C, A, d->enc, d->att_enc, zt, NZ, d->full_att_w,
+        ICD_TRY(icd_attention_step_bwd_idx(bt, P, C, A, img_index, d->enc, d->att_enc, zt, NZ, d->full_att_w,
                                        d->alphas + (size_t)t * P, (int64_t)T * P,
                                        d->d_alphas ? d->d_alphas + (size_t)t * P : nullptr, (int64_t)T * P,
                                        d->gate + (size_t)t * B * C, d->awe_raw + (size_t)t * B * C, d->d_gated,
@@ -246,10 +279,15 @@ extern "C" int icd_attention_decoder_bwd(const icd_att_desc_t* d, void* stream) 
     }
     if (d->ev_rec_ready) ICD_CUDA(cudaEventRecord(reinterpret_cast<cudaEvent_t>(d->ev_rec_ready), s));
     // attention projections: d_att_enc for all steps at once, full_att grads, then enc_att grads (:54)
-    ICD_TRY(icd_attention_proj_bwd(B, T, P, A, d->bt_host, d->att_enc, d->z, NZ, d->full_att_w, d->d_e,
-                                   d->d_att_enc, d->d_full_att_w, d->d_full_att_b, d->d_enc_att_b, d->proj_partial,
-                                   stream));
-    ICD_TRY(icd_gemm_simple(prec, d->d_att_enc, 1, A, d->enc, 1, C, d->d_enc_att_w, C, A, C, B * P,
+    if (ix)          // per image: d_att_enc (n_img,P,A) summed over each image's (row, step) pairs
+        ICD_TRY(icd_attention_proj_bwd_indexed(B, n_img, T, P, A, d->bt_host, ix->img_row_ptr, ix->img_rows, d->att_enc, d->z, NZ,
+                                               d->full_att_w, d->d_e, d->d_att_enc, d->d_full_att_w, d->d_full_att_b,
+                                               d->d_enc_att_b, d->proj_partial, s));
+    else
+        ICD_TRY(icd_attention_proj_bwd(B, T, P, A, d->bt_host, d->att_enc, d->z, NZ, d->full_att_w, d->d_e,
+                                       d->d_att_enc, d->d_full_att_w, d->d_full_att_b, d->d_enc_att_b, d->proj_partial,
+                                       stream));
+    ICD_TRY(icd_gemm_simple(prec, d->d_att_enc, 1, A, d->enc, 1, C, d->d_enc_att_w, C, A, C, n_img * P,
                             nullptr, nullptr, nullptr, 0, nullptr, 0, nullptr, 0.f, s, ICD_GEMM_ALLOW_SPLITK));
     // ---- optional: gradient w.r.t. the encoder features (--fine_tune_encoder) ----
     if (d->d_enc) {
@@ -260,10 +298,17 @@ extern "C" int icd_attention_decoder_bwd(const icd_att_desc_t* d, void* stream) 
         ICD_TRY(icd_gemm_simple(prec, d->dc, D, 1, d->c_lin_w, 1, C, d->d_mean, C, B, C, D,
                                 nullptr, nullptr, nullptr, 0, nullptr, 0, nullptr, 1.f, s));
         int32_t* row_len_ws = reinterpret_cast<int32_t*>(d->proj_partial);       // free again after the projection pass
-        ICD_TRY(icd_attention_enc_grad(B, T, P, C, d->bt_host, d->alphas, d->d_awe_all, d->d_mean, d->d_enc, row_len_ws, stream));
+        ICD_TRY(icd_attention_enc_grad_indexed(B, n_img, T, P, C, d->bt_host, ix ? ix->img_row_ptr : nullptr,
+                                               ix ? ix->img_rows : nullptr, d->alphas, d->d_awe_all, d->d_mean, d->d_enc,
+                                               row_len_ws, s));
         // + d_att_enc W_e  (:54)
-        ICD_TRY(icd_gemm_simple(prec, d->d_att_enc, A, 1, d->enc_att_w, 1, C, d->d_enc, C, B * P, C, A,
+        ICD_TRY(icd_gemm_simple(prec, d->d_att_enc, A, 1, d->enc_att_w, 1, C, d->d_enc, C, n_img * P, C, A,
                                 nullptr, nullptr, nullptr, 0, nullptr, 0, nullptr, 1.f, s));
     }
     return 0;
+}
+
+extern "C" int icd_attention_decoder_bwd(const icd_att_desc_t* d, void* stream) { return decoder_bwd(d, nullptr, stream); }
+extern "C" int icd_attention_decoder_bwd_indexed(const icd_att_desc_t* d, const icd_att_index_t* ix, void* stream) {
+    return decoder_bwd(d, ix, stream);
 }

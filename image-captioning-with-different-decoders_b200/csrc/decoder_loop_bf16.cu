@@ -52,19 +52,20 @@ struct Bufs {
     int64_t ldE, ldV;
 };
 
-void carve(const icd_att_desc_t* d, Arena& a, Bufs& b) {
+// n_img: images of the features (= B, or icd_att_index_t.n_img when captions share images): enc, att_enc and d_att_enc are per image
+void carve(const icd_att_desc_t* d, int64_t n_img, Arena& a, Bufs& b) {
     const int64_t B = d->B, T = d->T, P = d->P, C = d->C, A = d->A, D = d->D, E = d->E, V = d->V;
     const int64_t NZ = A + C + 4 * D, TB = T * B;
     b.ldE = up8(E); b.ldV = up8(V);
     b.We = a.take(A, C); b.Wcat = a.take(NZ, D); b.WihE = a.take(4 * D, b.ldE); b.WihC = a.take(4 * D, C);
     b.Wh = a.take(D, C); b.Wc = a.take(D, C); b.Wfc = a.take(V, D);
     b.WihCp = a.take(4 * D, C);
-    b.enc = d->enc16 ? const_cast<void*>(d->enc16) : a.take(B * P, C);      // caller-provided bf16 features are used in place
-    b.att_enc = a.take(B * P, A); b.mean = a.take(B, C); b.embx = a.take(TB, b.ldE);
+    b.enc = d->enc16 ? const_cast<void*>(d->enc16) : a.take(n_img * P, C);      // caller-provided bf16 features are used in place
+    b.att_enc = a.take(n_img * P, A); b.mean = a.take(B, C); b.embx = a.take(TB, b.ldE);
     b.h = a.take(TB + B, D);
     b.gated = a.take(TB, C); b.hdrop = a.take(B * T, D);
     b.dY = a.take(B * T, b.ldV); b.dz = a.take(TB, NZ); b.dh = a.take(B, D); b.dc = a.take(B, D);
-    b.dae = a.take(B * P, A);
+    b.dae = a.take(n_img * P, A);
     // split-K workspace: the largest request among the contractions that may split
     const int shapes[][3] = {
         {(int)B, (int)D, (int)C},            // h_lin / c_lin
@@ -77,7 +78,7 @@ void carve(const icd_att_desc_t* d, Arena& a, Bufs& b) {
         {(int)(4 * D), (int)E, (int)TB},     // d W_ih (embedding part)
         {(int)(4 * D), (int)C, (int)TB},     // d W_ih (awe part)
         {(int)TB, (int)E, (int)(4 * D)},     // d emb_x
-        {(int)A, (int)C, (int)(B * P)},      // d enc_att.weight
+        {(int)A, (int)C, (int)(n_img * P)},  // d enc_att.weight
         {(int)V, (int)D, (int)(B * T)},      // d fc.weight
         {(int)(B * T), (int)D, (int)V},      // d hdrop
     };
@@ -88,11 +89,11 @@ void carve(const icd_att_desc_t* d, Arena& a, Bufs& b) {
     b.colsum_ws = reinterpret_cast<float*>(a.take_bytes(icd_colsum_bf16_ws_floats(B * T, (int)V) * 4));
 }
 
-int check16(const icd_att_desc_t* d, Arena& a, Bufs& b) {
+int check16(const icd_att_desc_t* d, int n_img, Arena& a, Bufs& b) {
     ICD_CHECK_ARG(d->A % 8 == 0 && d->C % 8 == 0 && d->D % 8 == 0 && d->E % 4 == 0,
                   "attention_decoder(bf16): A, C, D must be multiples of 8 and E of 4 (A=%d C=%d D=%d E=%d)", d->A, d->C, d->D, d->E);
     a.base = reinterpret_cast<char*>(d->tc_ws); a.cap = d->tc_ws_bytes; a.off = 0; a.ok = true;
-    carve(d, a, b);
+    carve(d, n_img, a, b);
     ICD_CHECK_ARG(d->tc_ws != nullptr && a.ok, "attention_decoder(bf16): tc_ws too small (%lld bytes given, %lld needed)",
                   (long long)d->tc_ws_bytes, (long long)a.off);
     return 0;
@@ -108,19 +109,24 @@ inline char* at16(void* p, int64_t elem_off) { return reinterpret_cast<char*>(p)
 
 }  // namespace
 
-int icd_convert_features_bf16(int B, int P, int C, const float* enc, void* enc16, float* mean, void* mean16, cudaStream_t s);
-int icd_feature_mean_bf16(int B, int P, int C, const void* enc16, float* mean, void* mean16, cudaStream_t s);
+// B images -> pixel means; row_ptr / rows (optional): the mean of image b is written to rows[row_ptr[b] .. row_ptr[b+1])
+int icd_convert_features_bf16(int B, int P, int C, const float* enc, void* enc16, float* mean, void* mean16, cudaStream_t s,
+                              const int32_t* row_ptr, const int32_t* rows);
+int icd_feature_mean_bf16(int B, int P, int C, const void* enc16, float* mean, void* mean16, cudaStream_t s,
+                          const int32_t* row_ptr, const int32_t* rows);
 
-int64_t icd_att_tc_ws_bytes(const icd_att_desc_t* d) {
+int64_t icd_att_tc_ws_bytes(const icd_att_desc_t* d, int n_img) {
     Arena a; a.base = nullptr; a.cap = 0; a.off = 0; a.ok = true;
     Bufs b;
-    carve(d, a, b);
+    carve(d, n_img, a, b);
     return a.off;
 }
 
-int icd_attention_decoder_fwd_bf16(const icd_att_desc_t* d, cudaStream_t s) {
+int icd_attention_decoder_fwd_bf16(const icd_att_desc_t* d, const icd_att_index_t* ix, cudaStream_t s) {
+    const int n_img = ix ? ix->n_img : d->B;
+    const int32_t* img_index = ix ? ix->img_index : nullptr;
     Arena ar; Bufs u;
-    ICD_TRY(check16(d, ar, u));
+    ICD_TRY(check16(d, n_img, ar, u));
     const int B = d->B, T = d->T, P = d->P, C = d->C, A = d->A, D = d->D, E = d->E, V = d->V;
     const int NZ = A + C + 4 * D, TB = T * B;
     const long long BD = (long long)B * D;
@@ -166,14 +172,17 @@ int icd_attention_decoder_fwd_bf16(const icd_att_desc_t* d, cudaStream_t s) {
     }
     if (fused_cell) ICD_TRY(icd_convert_bf16_gateperm(d->w_ih + E, E + C, D, C, u.WihCp, C, s));
     // ---- features: fp32 -> bf16 and the pixel mean (:161) in one pass over encoder_out ----
-    if (d->enc16) ICD_TRY(icd_feature_mean_bf16(B, P, C, d->enc16, d->mean_enc, u.mean, s));
+    //    (captions that share images: once per image, the mean written to each of the image's rows)
+    const int32_t* mrow_ptr = ix ? ix->img_row_ptr : nullptr;
+    const int32_t* mrows = ix ? ix->img_rows : nullptr;
+    if (d->enc16) ICD_TRY(icd_feature_mean_bf16(n_img, P, C, d->enc16, d->mean_enc, u.mean, s, mrow_ptr, mrows));
     else {
         ICD_CHECK_ARG(d->enc != nullptr, "attention_decoder(bf16): neither enc nor enc16 given");
-        ICD_TRY(icd_convert_features_bf16(B, P, C, d->enc, u.enc, d->mean_enc, u.mean, s));
+        ICD_TRY(icd_convert_features_bf16(n_img, P, C, d->enc, u.enc, d->mean_enc, u.mean, s, mrow_ptr, mrows));
     }
 
     // K1: att_enc = enc_att(encoder_out), once per batch (models/attention.py:54); stored bf16 only
-    MMX(u.enc, C, 0, u.We, C, 0, nullptr, 0, B * P, A, C, d->enc_att_b, nullptr, nullptr, 0, nullptr, 0, nullptr, u.att_enc, A);
+    MMX(u.enc, C, 0, u.We, C, 0, nullptr, 0, n_img * P, A, C, d->enc_att_b, nullptr, nullptr, 0, nullptr, 0, nullptr, u.att_enc, A);
     // K7: init_hidden_state (:162-163); h_0 also emitted as bf16 (operand of the first step)
     MMX(u.mean, C, 0, u.Wh, C, 0, d->h_all, D, B, D, C, d->h_lin_b, nullptr, nullptr, 0, nullptr, 0, nullptr, u.h, D);
     MMX(u.mean, C, 0, u.Wc, C, 0, d->c_all, D, B, D, C, d->c_lin_b, nullptr, nullptr, 0, nullptr, 0, nullptr, nullptr, 0);
@@ -193,7 +202,7 @@ int icd_attention_decoder_fwd_bf16(const icd_att_desc_t* d, cudaStream_t s) {
         char* g16 = at16(u.gated, (int64_t)t * B * C);
         icd_gemm_next_feeds_attention();       // the attention-step grid is staged behind K2 and placed when K2's last CTA exits
         MMX(h16, D, 0, u.Wcat, D, 0, zt, NZ, bt, NZ, D, d->b_cat, nullptr, nullptr, 0, nullptr, 0, nullptr, nullptr, 0);   // K2
-        ICD_TRY(icd_attention_step_fwd_bf16(bt, P, C, A, nullptr, u.enc, u.att_enc, zt, NZ, d->full_att_w, d->full_att_b,
+        ICD_TRY(icd_attention_step_fwd_bf16(bt, P, C, A, img_index, u.enc, u.att_enc, zt, NZ, d->full_att_w, d->full_att_b,
                                             zt + A, NZ, d->alphas + (size_t)t * P, (int64_t)T * P,
                                             d->awe_raw + (size_t)t * B * C, d->gate + (size_t)t * B * C,
                                             d->gated + (size_t)t * B * C, g16, (void*)s));                         // K3
@@ -218,11 +227,13 @@ int icd_attention_decoder_fwd_bf16(const icd_att_desc_t* d, cudaStream_t s) {
     return 0;
 }
 
-int icd_attention_decoder_bwd_bf16(const icd_att_desc_t* d, cudaStream_t s) {
+int icd_attention_decoder_bwd_bf16(const icd_att_desc_t* d, const icd_att_index_t* ix, cudaStream_t s) {
+    const int n_img = ix ? ix->n_img : d->B;
+    const int32_t* img_index = ix ? ix->img_index : nullptr;
     Arena ar; Bufs u;
-    ICD_TRY(check16(d, ar, u));
+    ICD_TRY(check16(d, n_img, ar, u));
     const int B = d->B, T = d->T, P = d->P, C = d->C, A = d->A, D = d->D, E = d->E, V = d->V;
-    const int NZ = A + C + 4 * D, TB = T * B, BT = B * T, BP = B * P;
+    const int NZ = A + C + 4 * D, TB = T * B, BT = B * T, BP = n_img * P;      // BP: pixel rows of the per-image tensors
     const long long BD = (long long)B * D;
     const float* NF = nullptr;
 
@@ -262,7 +273,7 @@ int icd_attention_decoder_bwd_bf16(const icd_att_desc_t* d, cudaStream_t s) {
         // d_gated = dG W_ih[:, E:]           (W_ih[:, E:] stored [4D, C] = MN-major B, N = C, K = 4D)
         icd_gemm_next_feeds_attention();
         MMX(at16(dz16, A + C), NZ, 0, u.WihC, C, 1, d->d_gated, C, bt, C, 4 * D, NF, NF, NF, 0, NF, 0, nullptr, nullptr, 0);
-        ICD_TRY(icd_attention_step_bwd_bf16(bt, P, C, A, u.enc, u.att_enc, zt, NZ, d->full_att_w,
+        ICD_TRY(icd_attention_step_bwd_bf16_idx(bt, P, C, A, img_index, u.enc, u.att_enc, zt, NZ, d->full_att_w,
                                             d->alphas + (size_t)t * P, (int64_t)T * P,
                                             d->d_alphas ? d->d_alphas + (size_t)t * P : nullptr, (int64_t)T * P,
                                             d->gate + (size_t)t * B * C, d->awe_raw + (size_t)t * B * C, d->d_gated,
@@ -300,9 +311,14 @@ int icd_attention_decoder_bwd_bf16(const icd_att_desc_t* d, cudaStream_t s) {
     if (d->ev_rec_ready) ICD_CUDA(cudaEventRecord(reinterpret_cast<cudaEvent_t>(d->ev_rec_ready), s)); // recurrent gradients final
     // attention projections: d_att_enc for all steps at once (bf16 only: it is just the A operand of the next
     // contraction), full_att grads and the enc_att bias grad from the same pass, then the enc_att weight grad (:54)
-    ICD_TRY(icd_attention_proj_bwd_bf16_ex(B, T, P, A, d->bt_host, u.att_enc, d->z, NZ, d->full_att_w, d->d_e,
-                                           nullptr, u.dae, d->d_full_att_w, d->d_full_att_b, d->d_enc_att_b,
-                                           d->proj_partial, d->dz, NZ, (void*)s));
+    if (ix)          // per image: d_att_enc (n_img,P,A) summed over each image's (row, step) pairs
+        ICD_TRY(icd_attention_proj_bwd_bf16_indexed(B, n_img, T, P, A, d->bt_host, ix->img_row_ptr, ix->img_rows, u.att_enc, d->z, NZ,
+                                                    d->full_att_w, d->d_e, u.dae, d->d_full_att_w, d->d_full_att_b,
+                                                    d->d_enc_att_b, d->proj_partial, d->dz, NZ, s));
+    else
+        ICD_TRY(icd_attention_proj_bwd_bf16_ex(B, T, P, A, d->bt_host, u.att_enc, d->z, NZ, d->full_att_w, d->d_e,
+                                               nullptr, u.dae, d->d_full_att_w, d->d_full_att_b, d->d_enc_att_b,
+                                               d->proj_partial, d->dz, NZ, (void*)s));
     MMX(u.dae, A, 1, u.enc, C, 1, d->d_enc_att_w, C, A, C, BP, NF, NF, NF, 0, NF, 0, nullptr, nullptr, 0);
     // ---- optional: gradient w.r.t. the encoder features (--fine_tune_encoder) ----
     if (d->d_enc) {
@@ -312,7 +328,9 @@ int icd_attention_decoder_bwd_bf16(const icd_att_desc_t* d, cudaStream_t s) {
         ICD_TRY(icd_gemm_bf16_ex(u.dc, D, 0, u.Wc, C, 1, d->d_mean, C, B, C, D, NF, NF, NF, 0, NF, 0, nullptr, 1.f, s,
                                  nullptr, 0, u.splitk, u.splitk_floats));
         int32_t* row_len_ws = reinterpret_cast<int32_t*>(d->proj_partial);       // free again after the projection pass
-        ICD_TRY(icd_attention_enc_grad(B, T, P, C, d->bt_host, d->alphas, d->d_awe_all, d->d_mean, d->d_enc, row_len_ws, (void*)s));
+        ICD_TRY(icd_attention_enc_grad_indexed(B, n_img, T, P, C, d->bt_host, ix ? ix->img_row_ptr : nullptr,
+                                               ix ? ix->img_rows : nullptr, d->alphas, d->d_awe_all, d->d_mean, d->d_enc,
+                                               row_len_ws, s));
         // + d_att_enc W_e (:54): W_e stored [A, C] = MN-major B (N = C, K = A)
         ICD_TRY(icd_gemm_bf16_ex(u.dae, A, 0, u.We, C, 1, d->d_enc, C, BP, C, A, NF, NF, NF, 0, NF, 0, nullptr, 1.f, s,
                                  nullptr, 0, nullptr, 0));

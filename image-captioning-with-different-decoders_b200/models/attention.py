@@ -12,6 +12,9 @@ word-piece merging) needs ``pytorch_pretrained_bert`` and downloaded weights, ne
 ``captions -> (B, L, embed_size)`` in as ``decoder.bert_embedder``, or pass ``embeddings=`` to ``forward``.
 ``encoder_out.requires_grad`` (``--fine_tune_encoder``, train.py:39) is honoured: the backward also returns the gradient
 w.r.t. the encoder features (attention-weighted sum, ``enc_att`` projection and initial-state mean paths).
+``forward(..., image_index=idx)``: captions that share images (several references per image, self-critical samples) — caption
+row r attends over ``encoder_out[idx[r]]``, with the result of ``forward(encoder_out[idx], ...)`` and without replicating the
+features; the per-image work (``enc_att``, the pixel mean, the feature gradient) runs once per image.
 """
 import ctypes
 
@@ -174,13 +177,23 @@ class AttentionDecoder(nn.Module):
         with torch.no_grad():
             return self.bert_embedder(encoded_captions)
 
-    def forward(self, encoder_out, encoded_captions, caption_lengths, embeddings=None):
+    def forward(self, encoder_out, encoded_captions, caption_lengths, embeddings=None, image_index=None):
         """(:218-284) -> (predictions (B,T,V), encoded_captions, decode_lengths, attention_weights (B,T,P)).
         ``embeddings`` (extension): pre-computed (B, L, embed_size) caption embeddings used instead of the table lookup —
-        what the reference's ``use_bert`` branch feeds the loop (:242-244, :273)."""
-        batch_size = encoder_out.size(0)
+        what the reference's ``use_bert`` branch feeds the loop (:242-244, :273).
+        ``image_index`` (extension): a 1-D integer tensor (CPU or CUDA) of B values in [0, n_img) — caption row r attends over
+        image ``image_index[r]`` of ``encoder_out`` (n_img, ..., C).  The result is that of ``forward(encoder_out[image_index],
+        ...)``; the gradient w.r.t. ``encoder_out`` is (n_img, ...), each image's rows summed.  A CPU tensor reaches the
+        device in one asynchronous copy from pinned memory (the host does not wait for the GPU); a CUDA tensor is first read
+        back to the host for validation, which waits for the GPU.  Bad input raises ValueError before any work is queued."""
+        index = None
+        if image_index is not None:
+            index = ImageIndex(image_index, encoded_captions.size(0), encoder_out.size(0))
+            batch_size = index.B
+        else:
+            batch_size = encoder_out.size(0)
         encoder_dim = encoder_out.size(-1)
-        enc = encoder_out.reshape(batch_size, -1, encoder_dim)                         # :230
+        enc = encoder_out.reshape(encoder_out.size(0), -1, encoder_dim)                # :230
         decode_lengths = [caption_length - 1 for caption_length in caption_lengths]    # :236
         T = max(decode_lengths)
         dl_np = np.asarray(decode_lengths, dtype=np.int64)
@@ -210,8 +223,54 @@ class AttentionDecoder(nn.Module):
             self.h_lin.weight, self.h_lin.bias, self.c_lin.weight, self.c_lin.bias,
             self.f_beta.weight, self.f_beta.bias, self.fc.weight, self.fc.bias,
             bt, mask, (1.0 / (1.0 - p)) if mask is not None else 1.0, self.precision,
-            getattr(self, "_icd_grad_sink", None))
+            getattr(self, "_icd_grad_sink", None), index)
         return predictions, encoded_captions, decode_lengths, alphas
+
+
+def build_image_index(image_index, batch_size, n_img):
+    """Host side of ``forward(..., image_index=)``: validate the index and form its per-image row lists.
+    -> (img_index (B,), row_ptr (n_img+1,), rows (B,)) int32 numpy arrays: the rows of image i are rows[row_ptr[i]:row_ptr[i+1]],
+    ascending (the order in which every per-image gradient sum adds them).  Raises ValueError on a tensor that is not 1-D, not
+    of an integer dtype, not of length ``batch_size``, or with a value outside [0, n_img)."""
+    if not isinstance(image_index, torch.Tensor):
+        raise ValueError("image_index must be a torch tensor, got %s" % type(image_index).__name__)
+    if image_index.dim() != 1:
+        raise ValueError("image_index must be 1-D, got shape %s" % (tuple(image_index.shape),))
+    if image_index.dtype.is_floating_point or image_index.dtype.is_complex or image_index.dtype == torch.bool:
+        raise ValueError("image_index must have an integer dtype, got %s" % image_index.dtype)
+    if image_index.shape[0] != batch_size:
+        raise ValueError("image_index has %d entries for %d caption rows" % (image_index.shape[0], batch_size))
+    if not 1 <= n_img <= 65535:
+        raise ValueError("image_index: encoder_out holds %d images (1 .. 65535 supported)" % n_img)
+    idx = image_index.detach().cpu().numpy().astype(np.int64)
+    if idx.size and (idx.min() < 0 or idx.max() >= n_img):
+        raise ValueError("image_index values must lie in [0, %d), got [%d, %d]" % (n_img, idx.min(), idx.max()))
+    row_ptr = np.zeros(n_img + 1, dtype=np.int64)
+    np.cumsum(np.bincount(idx, minlength=n_img), out=row_ptr[1:])
+    rows = np.argsort(idx, kind="stable")
+    return idx.astype(np.int32), row_ptr.astype(np.int32), rows.astype(np.int32)
+
+
+class ImageIndex:
+    """A validated image index (``build_image_index``); ``device(dev)`` copies it to the GPU in one transfer and returns the
+    C descriptor (icd_att_index_t) with the tensor that owns its memory."""
+
+    def __init__(self, image_index, batch_size, n_img):
+        self.img_index, self.row_ptr, self.rows = build_image_index(image_index, batch_size, n_img)
+        self.B, self.n_img = batch_size, n_img
+
+    def device(self, dev):
+        """-> (descriptor, device tensor that owns its memory, host staging tensor).  For a CUDA device the copy is one
+        asynchronous transfer from pinned memory: the host does not wait for the device.  The staging tensor must outlive
+        the copy."""
+        host = torch.from_numpy(np.concatenate([self.img_index, self.row_ptr, self.rows]))
+        if dev.type == "cuda":
+            host = host.pin_memory()
+        packed = host.to(dev, non_blocking=True)
+        B, n = self.B, self.n_img
+        ix = _lib.AttIndex()
+        fill(ix, n_img=n, img_index=packed[:B], img_row_ptr=packed[B:B + n + 1], img_rows=packed[B + n + 1:])
+        return ix, packed, host
 
 
 _W_NAMES = ["enc_att_w", "enc_att_b", "dec_att_w", "dec_att_b", "full_att_w", "full_att_b",
@@ -233,7 +292,7 @@ class _AttentionDecoderFn(torch.autograd.Function):
     @staticmethod
     def forward(ctx, enc, captions, emb_w, *rest):
         weights = rest[:18]
-        bt, mask, drop_scale, precision, sink = rest[18:]
+        bt, mask, drop_scale, precision, sink, index = rest[18:]
         _lib.remember_versions(ctx, list(zip(_W_NAMES, weights)) + [("embedding.weight", emb_w), ("encoder_out", enc)])
         ctx.sink = sink                  # DataParallelClipAdam in overlap mode: gradients go straight into its flat buffer
         if not enc.is_cuda:
@@ -250,7 +309,11 @@ class _AttentionDecoderFn(torch.autograd.Function):
             enc = enc.contiguous().float()
         captions = captions.contiguous()
         assert captions.dtype == torch.int64
-        B, P, C = (enc16 if enc is None else enc).shape
+        n_img, P, C = (enc16 if enc is None else enc).shape
+        B = index.B if index is not None else n_img
+        ix = None
+        if index is not None:                               # (n_img, P, *) per-image tensors, (B, *) per-row ones
+            ix, ix_mem, ix_host = index.device(dev)
         T = len(bt)
         L = captions.shape[1]
         A = weights[0].shape[0]
@@ -270,7 +333,7 @@ class _AttentionDecoderFn(torch.autograd.Function):
         f32 = dict(device=dev, dtype=torch.float32)
         bufs = dict(
             predictions=torch.empty(B, T, V, **f32), alphas=torch.empty(B, T, P, **f32),
-            att_enc=torch.empty(B, P, A, **f32), mean_enc=torch.empty(B, C, **f32),
+            att_enc=torch.empty(n_img, P, A, **f32), mean_enc=torch.empty(B, C, **f32),
             emb_x=(pre if pre is not None else torch.empty(T, B, E, **f32)), xg=torch.empty(T, B, 4 * D, **f32),
             w_cat=torch.empty(NZ, D, **f32), b_cat=torch.empty(NZ, **f32), z=torch.empty(T, B, NZ, **f32),
             awe_raw=torch.empty(T, B, C, **f32), gate=torch.empty(T, B, C, **f32), gated=torch.empty(T, B, C, **f32),
@@ -284,16 +347,26 @@ class _AttentionDecoderFn(torch.autograd.Function):
              emb_w=emb_c, **dict(zip(_W_NAMES, weights)), **bufs)
         for t in range(T):
             d.bt_host[t] = bt[t]
-        need = int(lib().icd_attention_decoder_ws_bytes(ctypes.byref(d)))
+        if ix is None:
+            need = int(lib().icd_attention_decoder_ws_bytes(ctypes.byref(d)))
+        else:
+            need = int(lib().icd_attention_decoder_ws_bytes_indexed(ctypes.byref(d), ctypes.byref(ix)))
+            bufs["ix_mem"], bufs["ix_host"] = ix_mem, ix_host
         tc_ws = torch.empty(need, device=dev, dtype=torch.uint8) if need else None
         fill(d, tc_ws=tc_ws, tc_ws_bytes=need)
         bufs["tc_ws"] = tc_ws
-        check(lib().icd_attention_decoder_fwd(ctypes.byref(d), stream_ptr()), "icd_attention_decoder_fwd")
+        if ix is None:
+            check(lib().icd_attention_decoder_fwd(ctypes.byref(d), stream_ptr()), "icd_attention_decoder_fwd")
+        else:
+            check(lib().icd_attention_decoder_fwd_indexed(ctypes.byref(d), ctypes.byref(ix), stream_ptr()),
+                  "icd_attention_decoder_fwd_indexed")
         predictions, alphas = bufs.pop("predictions"), bufs.pop("alphas")
         # the returned tensors get this node as grad_fn: keeping them in ctx would create a reference cycle (and
         # leak ~3 GB of activations per step until the cyclic GC runs) — keep a detached alias of alphas instead
         bufs["alphas_saved"] = alphas.detach()
         ctx.desc = d
+        ctx.ix = ix
+        ctx.n_img = n_img
         ctx.keep = (enc if enc is not None else enc16, captions, emb_c, weights, mask, bufs)   # keeps buffers alive
         ctx.dims = (B, T, L, P, C, A, D, E, V, NZ, emb_is_f64)
         ctx.row_valid = bufs["row_valid"]
@@ -307,6 +380,7 @@ class _AttentionDecoderFn(torch.autograd.Function):
     @staticmethod
     def backward(ctx, d_pred, d_alphas):
         B, T, L, P, C, A, D, E, V, NZ, emb_is_f64 = ctx.dims
+        n_img, ix = ctx.n_img, ctx.ix
         if ctx.keep is None:
             raise RuntimeError("icd_b200: AttentionDecoder backward called a second time; its saved activations were "
                                "released after the first backward (like autograd's saved tensors without retain_graph)")
@@ -366,22 +440,28 @@ class _AttentionDecoderFn(torch.autograd.Function):
         scratch = dict(
             d_hdrop=torch.empty(B, T, D, **f32), dz=torch.empty(T, B, NZ, **f32), d_e=torch.empty(B, T, P, **f32),
             dh=torch.empty(B, D, **f32), dc=torch.empty(B, D, **f32), d_gated=torch.empty(B, C, **f32),
-            d_att_enc=(torch.empty(B, P, A, **f32) if ctx.precision != "bf16" else None),
+            d_att_enc=(torch.empty(n_img, P, A, **f32) if ctx.precision != "bf16" else None),
             d_emb_x=(torch.empty(T, B, E, **f32) if want_emb else None),
-            d_enc=(torch.empty(B, P, C, **f32) if want_enc else None),
+            d_enc=(torch.empty(n_img, P, C, **f32) if want_enc else None),
             d_awe_all=(torch.empty(T, B, C, **f32) if want_enc else None),
             d_mean=(torch.empty(B, C, **f32) if want_enc else None),
-            proj_partial=torch.empty(int(lib().icd_attention_proj_bwd_ws_floats(B, P, A)), **f32))
+            proj_partial=torch.empty(int(lib().icd_attention_proj_bwd_ws_floats(B, P, A) if ix is None else
+                                         lib().icd_attention_proj_bwd_ws_floats_indexed(B, n_img, P, A)), **f32))
         d = ctx.desc
         fill(d, d_predictions=d_pred, d_predictions16=d_pred16,
              ld_dpred16=(d_pred16.stride(0) if d_pred16 is not None else 0), d_alphas=d_alphas, **g, **scratch)
         d.ev_fc_ready, d.ev_rec_ready = ev_fc, ev_rec
-        check(lib().icd_attention_decoder_bwd(ctypes.byref(d), stream_ptr()), "icd_attention_decoder_bwd")
+        if ix is None:
+            check(lib().icd_attention_decoder_bwd(ctypes.byref(d), stream_ptr()), "icd_attention_decoder_bwd")
+        else:
+            check(lib().icd_attention_decoder_bwd_indexed(ctypes.byref(d), ctypes.byref(ix), stream_ptr()),
+                  "icd_attention_decoder_bwd_indexed")
         # release the ~GBs of saved activations now (stream-ordered: the caching allocator only hands them to later
         # work on this stream), not when the last reference to the loss tensor dies — otherwise two steps' worth of
         # activations coexist whenever the caller keeps `loss` across iterations
         ctx.keep = None
         ctx.desc = None
+        ctx.ix = None
         dwc, dbc = g["d_w_cat"], g["d_b_cat"]
         d_b_lstm = dbc[A + C:]
         if sink is not None:
@@ -402,4 +482,4 @@ class _AttentionDecoderFn(torch.autograd.Function):
             d_enc = d_enc.to(ctx.in_dtype)
         if sink is not None:
             sink.backward_issued(sunk)
-        return (d_enc, None, g["d_emb_w"], *grads, None, None, None, None, None)
+        return (d_enc, None, g["d_emb_w"], *grads, None, None, None, None, None, None)

@@ -5,7 +5,8 @@ One call of ``self_critical_loss`` (the definition is restated on the CPU in tes
 2. forms the advantage ``A = r - b`` against a baseline ``b``: the reward of the greedy caption ("greedy", the self-critical
    baseline) or the mean reward of the image's other samples ("mean", leave-one-out);
 3. packs the samples as one training batch, rows sorted by length (``pack_samples``), and runs the decoder's training forward
-   on them in eval mode (the sampled distribution has no dropout);
+   on them in eval mode (the sampled distribution has no dropout); the attention decoder reads each image's features once
+   for its m rows (``forward(..., image_index=)``), the baseline decoder gets its (E,) feature replicated per row;
 4. returns ``(1/N) sum A_row * CE(logits, next token)`` over the N scored tokens — ``-(1/N) sum A * logp`` — formed by the
    weighted fused cross-entropy kernels (``losses.weighted_token_loss``).
 The scored positions are exactly the sampler's steps 1 .. len-1, ``<end>`` included when it was drawn.  In the fp32 and
@@ -26,10 +27,11 @@ class PackedSamples:
     """The n x m samples of ``sample_captions`` as R = n*m training rows, sorted by a stable descending sort of the length
     (ties keep the flat index i*m + j), as the attention forward needs (it runs the first ``batch_size_t`` rows)."""
 
-    def __init__(self, captions, lengths, img_idx, perm, n, m):
+    def __init__(self, captions, lengths, img_idx, perm, n, m, img_idx_host=None):
         self.captions = captions      # (R, Lmax) int64, 0 beyond the length
         self.lengths = lengths        # list of R ints
         self.img_idx = img_idx        # (R,) int64: image of each row
+        self.img_idx_host = img_idx_host   # the same on the CPU (the attention forward's image_index: no device round trip)
         self.perm = perm              # (R,) int64: flat index i*m + j of each row
         self.n, self.m = n, m
 
@@ -57,7 +59,7 @@ def pack_samples(samples):
     rows = seq.reshape(n * m, -1)[perm, :Lmax].long()
     keep = torch.arange(Lmax, device=dev)[None, :] < torch.tensor(lengths, device=dev)[:, None]
     captions = torch.where(keep, rows, torch.zeros_like(rows))
-    return PackedSamples(captions, lengths, perm // m, perm, n, m)
+    return PackedSamples(captions, lengths, perm // m, perm, n, m, torch.from_numpy(order // m))
 
 
 def scored_targets(captions, lengths, baseline_decoder, row_valid=None):
@@ -136,11 +138,10 @@ def self_critical_loss(decoder, features, reward_fn, n_samples, start_id, end_id
     was_training = decoder.training
     decoder.eval()
     try:
-        x = features[pk.img_idx]
         if base:
-            logits = decoder(x, pk.captions)
+            logits = decoder(features[pk.img_idx], pk.captions)
         else:
-            logits = decoder(x, pk.captions, lengths)[0]
+            logits = decoder(features, pk.captions, lengths, image_index=pk.img_idx_host)[0]
         tgt = scored_targets(pk.captions, lengths, base, getattr(logits, "_icd_row_valid", None))
         w = pk.pack(adv)[:, None].expand(R, logits.shape[1]).contiguous()
         loss = weighted_token_loss(logits, tgt, w, n_tokens, bf16_grad_only=bf16_grad_only)

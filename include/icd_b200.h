@@ -317,6 +317,33 @@ ICD_API int64_t icd_attention_decoder_ws_bytes(const icd_att_desc_t* d);
 ICD_API int icd_attention_decoder_fwd(const icd_att_desc_t* d, void* stream);
 ICD_API int icd_attention_decoder_bwd(const icd_att_desc_t* d, void* stream);
 
+/* ------------------------------------------------------------------------------------------------
+ * Captions that share images (several reference captions per image, self-critical samples): the teacher-forced forward and
+ * backward above with caption row r attending over image img_index[r] of n_img images.  The result is by definition that of
+ * the plain calls on the replicated features enc[img_index]; the features are never replicated.
+ * In an indexed call these fields of icd_att_desc_t hold ONE ENTRY PER IMAGE (n_img leading rows instead of B):
+ *   enc / enc16 (n_img,P,C), att_enc (n_img,P,A), d_enc (n_img,P,C) (the sum over each image's rows), d_att_enc (n_img,P,A).
+ * Every other field stays per row (B), mean_enc included: it is computed once per image and written to each of its rows, so
+ * the h_lin / c_lin contractions and their gradients do not change.
+ * img_row_ptr / img_rows: the rows of image i are img_rows[img_row_ptr[i] .. img_row_ptr[i+1]), ascending — every per-image
+ * sum (d_att_enc, d enc_att.*, d_enc) adds its rows in that order, then steps in order: the result is deterministic.
+ * The device-side index is not validated (values must lie in [0, n_img) and agree with the CSR); the host wrappers check it.
+ * A NULL index makes the _indexed entry points identical to the plain ones.
+ * ---------------------------------------------------------------------------------------------- */
+typedef struct {
+    int32_t n_img;                /* images (>= 1); an image may have no rows */
+    const int32_t* img_index;     /* (B)         device: image of each caption row      */
+    const int32_t* img_row_ptr;   /* (n_img + 1) device: CSR offsets, [0] = 0, [n_img] = B */
+    const int32_t* img_rows;      /* (B)         device: rows of each image, ascending    */
+} icd_att_index_t;
+
+ICD_API int icd_sizeof_att_index(void);
+ICD_API int64_t icd_attention_decoder_ws_bytes_indexed(const icd_att_desc_t* d, const icd_att_index_t* ix);
+ICD_API int icd_attention_decoder_fwd_indexed(const icd_att_desc_t* d, const icd_att_index_t* ix, void* stream);
+ICD_API int icd_attention_decoder_bwd_indexed(const icd_att_desc_t* d, const icd_att_index_t* ix, void* stream);
+/* floats of desc->proj_partial an indexed backward needs (B caption rows, n_img images) */
+ICD_API int64_t icd_attention_proj_bwd_ws_floats_indexed(int B, int n_img, int P, int A);
+
 /* init_hidden_state (models/attention.py:151-164): mean over pixels, h_lin, c_lin.  h, c: (B,D).
  * Stand-alone entry point (caption generation): precision must be ICD_PREC_FP32 — the tensor-core tiers need a
  * workspace and are reached through icd_attention_decoder_fwd / icd_beam_search. */
